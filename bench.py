@@ -225,6 +225,23 @@ def rel_mse(img, ref, eps=1e-2):
     return float(np.mean((a - b) ** 2 / (b * b + eps)))
 
 
+DUMP_PIXELS = 1 << 20  # 2 x 16 MB of frame samples + 8 MB of indices: under 64 MB at any frame size
+
+
+def dump_frame(out_dir: str, hdr, ldr):
+    """Writes the HDR and LDR frames (RGBA float32) as out_dir/{hdr,ldr}.npy, each (n, 4), at the pixels listed in
+    out_dir/pixel_index.npy (float64, row-major pixel numbers): every pixel when the frame has at most DUMP_PIXELS of
+    them, otherwise the same seeded sample of DUMP_PIXELS pixels in every run of the same frame size."""
+    import numpy as np
+    n = hdr.shape[0] * hdr.shape[1]
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "hdr.npy"), hdr.reshape(n, 4)[idx])
+    np.save(os.path.join(out_dir, "ldr.npy"), ldr.reshape(n, 4)[idx])
+    log(f"[bench] wrote the frame of the last timed step ({len(idx)} of {n} pixels) to {out_dir}")
+
+
 def workload_record(Y, name: str, local: int, trav: int, spp: int, steps: int) -> dict:
     """A BASELINE.json configs[2] / configs[3] shape on one GPU: full MIS+NEE paths, `steps` waves of `spp` samples of the
     1080p frame after 3 warm-up waves, device-timed, with the surface-shading kernel's share and roofline.  `wave32`: the
@@ -416,6 +433,11 @@ def run_ours(args):
     clocks = ClockSampler(local if rank == 0 else -1)
     S_weak = spp * world  # weak scaling: the wave grows with the GPU count, every GPU keeps W*H*spp camera paths per step
     weak = timed_waves(S_weak, args.steps, n_warm)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # the frame as it stands after the last timed wave (the padding steps below render more waves), read on the root
+        # as yr_read does (combined tile shards); written once the clock window has closed
+        dumped = ctx.resolve_combined() if dist and not buckets else ctx.resolve()[:2]
     # keep the GPU under the same load until a few clock samples exist (not timed); the number of
     # extra steps is agreed across ranks so nothing can hang
     el = weak["w1"] - weak["w0"]
@@ -425,6 +447,8 @@ def run_ours(args):
         weak["step"](weak["total_waves"] - 1)
     sync_all()
     clk = clocks.stop(weak["w0"], time.time())
+    if dumped:
+        dump_frame(args.dump_outputs, *dumped)
     s0, s1 = weak["s0"], weak["s1"]
 
     frames_direct = bool(dist and not buckets and ctx.comm_frames_direct())
@@ -505,7 +529,7 @@ def run_ours(args):
         e2e_step()
     sync_all()
     e0 = time.time()
-    n_e2e = max(2, min(args.steps, 10))
+    n_e2e = args.steps
     for _ in range(n_e2e):
         e2e_step()
     sync_all()
@@ -571,7 +595,7 @@ def run_ours(args):
             workloads = {}
             for name in ("sponza", "mclaren"):
                 try:
-                    workloads[name] = workload_record(Y, name, local, trav, spp, max(3, min(args.steps, 8)))
+                    workloads[name] = workload_record(Y, name, local, trav, spp, args.steps)
                 except Exception as ex:  # noqa: BLE001
                     workloads[name] = {"error": str(ex)}
         dev_ms = weak["dev_ms"]
@@ -643,7 +667,7 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of the headline, e2e and workload records (cpu_baseline: 2 reference renders)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="soup", choices=sorted(WORKLOADS))
@@ -658,7 +682,11 @@ def main():
                          "reference = the reference-order BVH2 walk (bit-identical frames)")
     ap.add_argument("--width", type=int, default=1920)
     ap.add_argument("--height", type=int, default=1080, help="3840 x 2160 for the BASELINE.json configs[4] shape")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame they produced as DIR/<name>.npy (see dump_frame)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global W, H, METRIC
     W, H = args.width, args.height
     if (W, H) != (1920, 1080):

@@ -6,6 +6,8 @@ anything under oracle/.  Nothing here reads /root/reference at run time.
 """
 from __future__ import annotations
 
+import hashlib
+import json
 import os
 import struct
 import subprocess
@@ -115,6 +117,17 @@ def oracle_render(scene: str, w: int, h: int, spp: int, cam: dict, binary=ORACLE
     hdr = np.frombuffer(raw, np.float32, n, off).reshape(hh, ww, 4).copy()
     ldr = np.frombuffer(raw, np.float32, n, off + 4 * n).reshape(hh, ww, 4).copy()
     return dict(hdr=hdr, ldr=ldr, rays=rays, ms=ms, threads=threads, build_ms=build_ms)
+
+
+def oracle_texload(image: bytes, tex_type: int, channels) -> np.ndarray:
+    """The reference's loadTexture<C> on an encoded image: (h, w, C) uint8."""
+    with tempfile.TemporaryDirectory() as d:
+        fin, fout = os.path.join(d, "image"), os.path.join(d, "out.bin")
+        open(fin, "wb").write(image)
+        run_oracle("texload", fin, tex_type, len(channels), ",".join(map(str, channels)), fout)
+        raw = open(fout, "rb").read()
+    w, h, c = struct.unpack_from("<III", raw, 0)
+    return np.frombuffer(raw, np.uint8, w * h * c, 12).reshape(h, w, c)
 
 
 def oracle_bvh(scene: str, kind: str = "sah"):
@@ -274,3 +287,28 @@ def bits_equal(a: np.ndarray, b: np.ndarray) -> np.ndarray:
     """Bitwise float equality; any NaN equals any NaN (payloads are not part of the contract)."""
     a, b = np.ascontiguousarray(a, np.float32), np.ascontiguousarray(b, np.float32)
     return (a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))
+
+
+# ------------------------------------------------------------------------------------------
+# the reference's outputs recorded as digests (tests/golden/reference_digests.json, record_digests.py next to it):
+# equal digests are the bitwise equality bits_equal() checks, without storing full frames
+# ------------------------------------------------------------------------------------------
+REFERENCE_DIGESTS = os.path.join(GOLDEN, "reference_digests.json")
+_recorded = None
+
+
+def digest(a) -> str:
+    """SHA-256 of an array's shape, dtype and bytes, every float NaN replaced by one NaN (bits_equal's rule)."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), a.dtype.type(np.nan), a).astype(a.dtype)
+    return hashlib.sha256(f"{a.shape}{a.dtype.str}".encode() + a.tobytes()).hexdigest()
+
+
+def recorded(key: str):
+    """The reference's recorded output for one test input: a digest or a dict of digests and counts."""
+    global _recorded
+    if _recorded is None:
+        with open(REFERENCE_DIGESTS) as f:
+            _recorded = json.load(f)
+    return _recorded[key]

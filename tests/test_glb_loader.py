@@ -2,10 +2,10 @@
 
 The reference's loader cannot be built here (fastgltf is not vendored), so the reader is pinned by
 (i) texture decode + conversion against the reference's own loadTexture (stb_image + glibc pow, through
-`oracle_ref texload`), (ii) an independently constructed expected scene (.ysc bytes) for a GLB that
-exercises every branch of gltf.cpp, and (iii) rendering the loaded scene against the oracle."""
+`oracle_ref texload`; recorded in tests/golden/reference_digests.json), (ii) an independently constructed expected
+scene (.ysc bytes) for a GLB that exercises every branch of gltf.cpp, and (iii) rendering the loaded scene against the
+reference's recorded frame."""
 import os
-import struct
 
 import numpy as np
 import pytest
@@ -16,17 +16,19 @@ from yart_b200 import scenes as S
 from yart_b200.glbwriter import GlbBuilder, png_encode
 
 pytestmark = pytest.mark.usefixtures("hostsim_lib")
-needs_oracle = pytest.mark.skipif(not H.have_oracle(), reason="oracle/_ref/oracle_ref not built")
 f32 = np.float32
+TEXLOAD_CASES = ((S.SRGB, [0, 1, 2, 3]), (S.NONCOLOR, [1, 2]), (S.NONCOLOR, [0]), (S.SRGB, [0, 1, 2]), (S.LINEAR, [2, 1, 0]))
 
 
-def oracle_texload(png: bytes, tex_type: int, channels, tmp_path) -> np.ndarray:
-    pin, pout = tmp_path / "t.png", tmp_path / "t.bin"
-    pin.write_bytes(png)
-    H.run_oracle("texload", pin, tex_type, len(channels), ",".join(map(str, channels)), pout)
-    raw = pout.read_bytes()
-    w, h, c = struct.unpack_from("<III", raw, 0)
-    return np.frombuffer(raw, np.uint8, w * h * c, 12).reshape(h, w, c)
+def texload_key(name: str, tex_type: int, channels) -> str:
+    return f"texload_{name}_{tex_type}_{''.join(map(str, channels))}"
+
+
+def reference_texload(name: str, png: bytes, tex_type: int, channels) -> np.ndarray:
+    """loadTexture's result for the named test image: the product's decode, checked against the reference's."""
+    got = Y.decode_texture(png, tex_type, channels)
+    assert H.digest(got) == H.recorded(texload_key(name, tex_type, channels)), (name, tex_type, channels)
+    return got
 
 
 def sample_images():
@@ -41,9 +43,7 @@ def sample_images():
     }
 
 
-@needs_oracle
-@pytest.mark.parametrize("name", ["rgba", "rgb", "grey", "grey_alpha", "smooth_rgb", "palette", "rgb16"])
-def test_png_decode_and_conversion_match_reference_loadTexture(name, tmp_path):
+def sample_png(name: str) -> bytes:
     rng = np.random.default_rng(5)
     if name == "palette":
         pal = rng.integers(0, 256, (37, 3), dtype=np.uint8)
@@ -52,11 +52,14 @@ def test_png_decode_and_conversion_match_reference_loadTexture(name, tmp_path):
         png = png_encode(rng.integers(0, 65536, (7, 9, 3)).astype(np.uint16), bit_depth=16)
     else:
         png = png_encode(sample_images()[name])
-    for tex_type, channels in ((S.SRGB, [0, 1, 2, 3]), (S.NONCOLOR, [1, 2]), (S.NONCOLOR, [0]), (S.SRGB, [0, 1, 2]),
-                               (S.LINEAR, [2, 1, 0])):
-        want = oracle_texload(png, tex_type, channels, tmp_path)
-        got = Y.decode_texture(png, tex_type, channels)
-        assert got.shape == want.shape and np.array_equal(got, want), (name, tex_type, channels)
+    return png
+
+
+@pytest.mark.parametrize("name", ["rgba", "rgb", "grey", "grey_alpha", "smooth_rgb", "palette", "rgb16"])
+def test_png_decode_and_conversion_match_reference_loadTexture(name):
+    png = sample_png(name)
+    for tex_type, channels in TEXLOAD_CASES:
+        reference_texload(name, png, tex_type, channels)
 
 
 def test_png_errors():
@@ -102,7 +105,7 @@ def quat(axis, deg):
     return [float(f32(x)) for x in (*(a * np.sin(h)), np.cos(h))]
 
 
-def build_case(tmp_path, with_oracle_textures=True):
+def build_case(tmp_path, check_textures=True):
     """A GLB touching every branch of gltf.cpp, plus the scene it must load as."""
     imgs = sample_images()
     g = GlbBuilder()
@@ -158,10 +161,12 @@ def build_case(tmp_path, with_oracle_textures=True):
     glb.write_bytes(g.tobytes())
 
     # ---- the scene gltf::load would build, constructed independently -------------------------------
-    texload = (lambda png, t, ch: oracle_texload(png, t, ch, tmp_path)) if with_oracle_textures else Y.decode_texture
+    texload = reference_texload if check_textures else (lambda _, png, t, ch: Y.decode_texture(png, t, ch))
     e = S.Scene()
-    e.textures = [S.Texture(texload(png_base, S.SRGB, [0, 1, 2, 3]), S.SRGB), S.Texture(texload(png_mr, S.NONCOLOR, [1, 2]), S.NONCOLOR),
-                  S.Texture(texload(png_nrm, S.NONCOLOR, [0, 1, 2]), S.NONCOLOR), S.Texture(texload(png_em, S.SRGB, [0, 1, 2]), S.SRGB)]
+    e.textures = [S.Texture(texload("rgba", png_base, S.SRGB, [0, 1, 2, 3]), S.SRGB),
+                  S.Texture(texload("rgb", png_mr, S.NONCOLOR, [1, 2]), S.NONCOLOR),
+                  S.Texture(texload("smooth_rgb", png_nrm, S.NONCOLOR, [0, 1, 2]), S.NONCOLOR),
+                  S.Texture(texload("rgb", png_em, S.SRGB, [0, 1, 2]), S.SRGB)]
     e.materials = [
         S.Material(base=(f32(0.9), f32(0.8), f32(0.7)), base_tex=0, mr_tex=1, normal_tex=2, roughness=0.6, metallic=0.2,
                    clearcoat_roughness=0.03, normal_scale=0.7, thin=1),
@@ -196,7 +201,6 @@ def build_case(tmp_path, with_oracle_textures=True):
     return str(glb), e
 
 
-@needs_oracle
 def test_glb_loads_as_the_expected_scene(tmp_path):
     glb, expected = build_case(tmp_path)
     want, got = tmp_path / "want.ysc", tmp_path / "got.ysc"
@@ -205,25 +209,35 @@ def test_glb_loads_as_the_expected_scene(tmp_path):
     assert got.read_bytes() == want.read_bytes()
 
 
-@needs_oracle
-def test_glb_scene_renders_bit_exactly_like_the_reference(tmp_path):
-    glb, _ = build_case(tmp_path)
-    env = S.sky_hdr(16, 16, 5, 50.0)
-    ysc = tmp_path / "scene.ysc"
-    Y.glb_to_ysc(glb, str(ysc), env=env, env_radius=80.0)
-    cam = dict(pos=(0.5, 4.0, 14.0), target=(0.0, 2.5, 0.0), focal=35.0, fnum=0.0, exposure=0.0)
-    ref = H.oracle_render(str(ysc), 64, 40, 8, cam, first=8, max=8, tonemap="agx", ppm=str(tmp_path / "ref.ppm"))
-    sc = Y.Scene(glb, env=env, env_radius=80.0)  # straight from the GLB
+GLB_CAM = dict(pos=(0.5, 4.0, 14.0), target=(0.0, 2.5, 0.0), focal=35.0, fnum=0.0, exposure=0.0)
+
+
+def glb_env():
+    return S.sky_hdr(16, 16, 5, 50.0)
+
+
+def render_glb_case(tmp_path):
+    """The GLB case straight from the file, with a sky, 64x40 at 8 spp: (render data, hdr, ldr, PPM bytes)."""
+    glb, _ = build_case(tmp_path, check_textures=False)
+    cam = GLB_CAM
+    sc = Y.Scene(glb, env=glb_env(), env_radius=80.0)
     assert sc.flat.nLights == 5 and sc.flat.nArea == 4 and sc.flat.nMeshes == 3
     c = Y.make_camera(64, 40, 35.0, 0.0, cam["pos"], cam["target"])
     r = Y.Renderer(64, 40, c, sc, samples=8, first_wave_samples=8, max_wave_samples=8)
     d = r.render_sync()
     hdr, ldr, _ = r.read()
-    assert d["total_rays"] == ref["rays"]
-    assert H.bits_equal(hdr, ref["hdr"]).all() and H.bits_equal(ldr, ref["ldr"]).all()
-    # output::writePPM parity (ppm.cpp:6-21)
     r.write_ppm(str(tmp_path / "ours.ppm"))
-    assert (tmp_path / "ours.ppm").read_bytes() == (tmp_path / "ref.ppm").read_bytes()
+    r.close()
+    return d, hdr, ldr, (tmp_path / "ours.ppm").read_bytes()
+
+
+def test_glb_scene_renders_bit_exactly_like_the_reference(tmp_path):
+    d, hdr, ldr, ppm = render_glb_case(tmp_path)
+    ref = H.recorded("glb_scene_64x40_8spp")
+    assert d["total_rays"] == ref["rays"]
+    assert H.digest(hdr) == ref["hdr"] and H.digest(ldr) == ref["ldr"]
+    # output::writePPM parity (ppm.cpp:6-21)
+    assert H.digest(np.frombuffer(ppm, np.uint8)) == ref["ppm"]
 
 
 def test_glb_errors(tmp_path):
@@ -231,7 +245,7 @@ def test_glb_errors(tmp_path):
     p.write_bytes(b"nope" + b"\0" * 32)
     with pytest.raises(Y.YartError, match="not a glTF file"):
         Y.Scene(str(p))
-    glb, _ = build_case(tmp_path, with_oracle_textures=False)
+    glb, _ = build_case(tmp_path, check_textures=False)
     raw = open(glb, "rb").read()
     p.write_bytes(raw[: len(raw) - 100])
     with pytest.raises(Y.YartError, match="truncated"):

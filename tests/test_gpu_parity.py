@@ -227,69 +227,25 @@ def _render_ctx(sc, cam, w, h, spp, waves, max_depth=30, tonemap=Y.TONEMAP_AGX, 
     return hdr, ldr, st
 
 
-needs_oracle = pytest.mark.skipif(not H.have_oracle(), reason="oracle/_ref/oracle_ref not present on this box")
+C1 = dict(scene="cornell", kw={}, w=512, h=512, spp=16, max_depth=30)
+C2 = dict(scene="soup", kw=dict(n_tris=1_000_000), w=1920, h=1080, spp=1, max_depth=1)
+C3 = dict(scene="sponza", kw=dict(n_tris=260_000, tex_res=256, env_res=512), w=1920, h=1080, spp=1, max_depth=30)
+C4 = dict(scene="mclaren", kw=dict(n_tris=2_000_000, env_res=512), w=1920, h=1080, spp=1, max_depth=30)
+C5 = dict(scene="two_quads", kw={}, w=3840, h=2160, spp=30, waves=[15, 15], max_depth=2)
 
 
-@needs_oracle
-def test_c1_cornell_512_16spp_matches_reference_run_here():
-    """configs[0] exactly: Cornell box, 512x512, 16 spp MIS+NEE, against the reference run on this box."""
-    sp, cam = H.scene_file("cornell"), H.scene_camera("cornell")
-    ref = H.oracle_render(sp, 512, 512, 16, cam, first=16, max=16, tonemap="agx")
-    hdr, ldr, st = _render_ctx(Y.Scene(sp), cam, 512, 512, 16, [16])
-    assert H.rel_mse(hdr, ref["hdr"]) < 1e-3 and H.rel_mse(ldr, ref["ldr"]) < 1e-3  # the north-star bar
-    assert st.raysReference == ref["rays"]
-    assert H.bits_equal(hdr, ref["hdr"]).all() and H.bits_equal(ldr, ref["ldr"]).all()
+def render_config(cfg, traversal=None):
+    """A BASELINE.json configuration rendered with the reference-order walk (or `traversal`): (scene, hdr, ldr, stats)."""
+    sc = Y.Scene(H.scene_file(cfg["scene"], **cfg["kw"]))
+    cam = H.scene_camera(cfg["scene"], **cfg["kw"])
+    hdr, ldr, st = _render_ctx(sc, cam, cfg["w"], cfg["h"], cfg["spp"], cfg.get("waves", [cfg["spp"]]), max_depth=cfg["max_depth"],
+                               traversal=traversal)
+    return sc, hdr, ldr, st
 
 
-@needs_oracle
-def test_c3_sponza_shape_1080p_matches_reference_run_here():
-    """configs[2] shape at full resolution and triangle count (260 K tris, textured PBR + normal maps +
-    alpha cut-outs, env light only), 1 spp so the CPU reference finishes in seconds."""
-    kw = dict(n_tris=260_000, tex_res=256, env_res=512)
-    from yart_b200 import scenes
-    sp, cam = H.scene_file("sponza", **kw), scenes.sponza(n_tris=100, tex_res=4, env_res=4).camera
-    ref = H.oracle_render(sp, 1920, 1080, 1, cam, first=1, max=1, tonemap="agx")
-    sc = Y.Scene(sp)
-    assert 200_000 < sc.n_tris < 300_000
-    hdr, ldr, st = _render_ctx(sc, cam, 1920, 1080, 1, [1])
-    _check_frame_against_oracle("C3", ref, hdr, ldr, st)
-
-
-def _check_frame_against_oracle(tag, ref, hdr, ldr, st, exact=True):
-    """North-star bars first (relMSE < 1e-3 on the HDR frame and after AgX, ray counts), then — for the
-    reference-order traversal — bitwise equality of both frames."""
-    rh, rl = H.rel_mse(hdr, ref["hdr"]), H.rel_mse(ldr, ref["ldr"])
-    assert rh < 1e-3 and rl < 1e-3, f"{tag}: relMSE hdr {rh} ldr {rl}"
-    if exact:
-        assert st.raysReference == ref["rays"], f"{tag}: rays {st.raysReference} vs {ref['rays']}"
-        bad = ~H.bits_equal(hdr, ref["hdr"])
-        assert not bad.any(), f"{tag}: HDR differs in {bad.sum()} words, first pixels {np.argwhere(bad.any(-1))[:8].tolist()}"
-        bad = ~H.bits_equal(ldr, ref["ldr"])
-        assert not bad.any(), f"{tag}: LDR differs in {bad.sum()} words, first pixels {np.argwhere(bad.any(-1))[:8].tolist()}"
-    else:
-        # the wide walk: same triangles, same triangle arithmetic, different box culling — pixels differ only where a
-        # path met a last-bit tie or a box-boundary hit (wide_bvh.cuh)
-        assert abs(int(st.raysReference) - int(ref["rays"])) <= 1e-4 * ref["rays"], f"{tag}: rays {st.raysReference} vs {ref['rays']}"
-        same = H.bits_equal(hdr, ref["hdr"]).all(-1).mean()
-        print(f"{tag} wide: relMSE hdr {rh:.3g} ldr {rl:.3g}, {same:.7f} of the pixels bit-identical, rays {st.raysReference} vs {ref['rays']}")
-        assert same > 0.999, f"{tag}: only {same} of the pixels are bit-identical to the reference"
-
-
-@needs_oracle
-def test_c2_soup_1m_tris_1080p_matches_reference_run_here():
-    """configs[1] EXACTLY as bench.py times it (1 M-triangle soup, 1920x1080, primary + shadow rays, maxDepth 1),
-    1 spp, against the reference run on this box: frames and ray count, then hit records of 400 K of the frame's
-    primary rays against RayIntegrator::testNode."""
-    sp, cam = H.scene_file("soup", n_tris=1_000_000), H.scene_camera("soup")
-    ref = H.oracle_render(sp, 1920, 1080, 1, cam, first=1, max=1, tonemap="agx", maxdepth=1)
-    sc = Y.Scene(sp)
-    assert sc.n_tris == 1_000_002  # the soup + the two triangles of the light quad
-    hdr, ldr, st = _render_ctx(sc, cam, 1920, 1080, 1, [1], max_depth=1)
-    _check_frame_against_oracle("C2", ref, hdr, ldr, st)
-    hdr, ldr, st = _render_ctx(sc, cam, 1920, 1080, 1, [1], max_depth=1, traversal=Y.TRAVERSAL_WIDE)  # what bench.py times
-    _check_frame_against_oracle("C2", ref, hdr, ldr, st, exact=False)
-    # ray level: the same frame's primary rays, every 20th, closest hit + any hit, both walks
-    W, Hh = 1920, 1080
+def c2_primary_rays(sc):
+    """Every 20th primary ray of the C2 frame, as the library generates them."""
+    W, Hh, cam = C2["w"], C2["h"], H.scene_camera("soup")
     ctx = Y.Context(max_depth=1, traversal=Y.TRAVERSAL_AUTO)
     ctx.upload_scene(sc)
     ctx.set_camera(Y.make_camera(W, Hh, cam["focal"], cam["fnum"], cam["pos"], cam["target"]))
@@ -300,8 +256,66 @@ def test_c2_soup_1m_tris_1080p_matches_reference_run_here():
     rays = np.empty((n, 8), np.float32)
     ctx.d2h(rays, rays_dev)
     ctx.device_free(rays_dev)
-    sel = rays[::20].copy()
-    want = H.oracle_trace(sp, sel, "closest")
+    return ctx, rays[::20].copy()
+
+
+def hit_digests(hits):
+    """What the reference's hit records pin: hit or miss, and the distance and triangle of every hit."""
+    m = hits["didHit"] == 1
+    return {"did_hit": H.digest(hits["didHit"]), "t": H.digest(hits["t"][m]), "prim": H.digest(hits["prim"][m])}
+
+
+def _check_frame_recorded(tag, key, hdr, ldr, st):
+    """The reference-order walk's frames and ray count against the reference's (recorded), bit for bit."""
+    ref = H.recorded(key)
+    assert st.raysReference == ref["rays"], f"{tag}: rays {st.raysReference} vs {ref['rays']}"
+    assert H.digest(hdr) == ref["hdr"], f"{tag}: HDR differs from the reference's"
+    assert H.digest(ldr) == ref["ldr"], f"{tag}: LDR differs from the reference's"
+
+
+def test_c1_cornell_512_16spp_matches_reference_run_here():
+    """configs[0] exactly: Cornell box, 512x512, 16 spp MIS+NEE, against the reference's frame."""
+    _, hdr, ldr, st = render_config(C1)
+    _check_frame_recorded("C1", "c1_cornell_512_16spp", hdr, ldr, st)
+
+
+def test_c3_sponza_shape_1080p_matches_reference_run_here():
+    """configs[2] shape at full resolution and triangle count (260 K tris, textured PBR + normal maps +
+    alpha cut-outs, env light only), 1 spp."""
+    sc, hdr, ldr, st = render_config(C3)
+    assert 200_000 < sc.n_tris < 300_000
+    _check_frame_recorded("C3", "c3_sponza_1080p_1spp", hdr, ldr, st)
+
+
+def _check_wide_frame(tag, ref, hdr, ldr, st):
+    """The wide walk's frame against the reference's: the north-star bars (relMSE < 1e-3 on the HDR frame and after
+    AgX, ray counts), and pixels differing only where a path met a last-bit tie or a box-boundary hit — same
+    triangles, same triangle arithmetic, different box culling (wide_bvh.cuh)."""
+    rh, rl = H.rel_mse(hdr, ref["hdr"]), H.rel_mse(ldr, ref["ldr"])
+    assert rh < 1e-3 and rl < 1e-3, f"{tag}: relMSE hdr {rh} ldr {rl}"
+    assert abs(int(st.raysReference) - int(ref["rays"])) <= 1e-4 * ref["rays"], f"{tag}: rays {st.raysReference} vs {ref['rays']}"
+    same = H.bits_equal(hdr, ref["hdr"]).all(-1).mean()
+    print(f"{tag} wide: relMSE hdr {rh:.3g} ldr {rl:.3g}, {same:.7f} of the pixels bit-identical, rays {st.raysReference} vs {ref['rays']}")
+    assert same > 0.999, f"{tag}: only {same} of the pixels are bit-identical to the reference"
+
+
+def test_c2_soup_1m_tris_1080p_matches_reference_run_here():
+    """configs[1] EXACTLY as bench.py times it (1 M-triangle soup, 1920x1080, primary + shadow rays, maxDepth 1),
+    1 spp, against the reference's frame and ray count, then hit records of 100 K of the frame's primary rays against
+    RayIntegrator::testNode.  The reference-order walk reproduces the reference bit for bit (checked against the
+    recorded digests first), so its frame and hits then stand for the reference's in the checks of the wide walk."""
+    sc, hdr, ldr, st = render_config(C2)
+    assert sc.n_tris == 1_000_002  # the soup + the two triangles of the light quad
+    _check_frame_recorded("C2", "c2_soup_1080p_1spp", hdr, ldr, st)
+    ref = dict(hdr=hdr, ldr=ldr, rays=int(st.raysReference))
+    _, hdr, ldr, st = render_config(C2, traversal=Y.TRAVERSAL_WIDE)  # what bench.py times
+    _check_wide_frame("C2", ref, hdr, ldr, st)
+    # ray level: the same frame's primary rays, every 20th, closest hit + any hit, both walks
+    ctx, sel = c2_primary_rays(sc)
+    rec = H.recorded("c2_soup_hits")
+    assert H.digest(sel) == rec["rays"], "C2: the primary rays differ from those the reference traced"
+    want, _ = ctx.trace(sel, Y.TRACE_CLOSEST | Y.TRACE_REFERENCE_ORDER)
+    assert hit_digests(want) == rec["closest"], "C2: closest hits of the reference-order walk differ from the reference's"
     m = want["didHit"] == 1
     for walk in (Y.TRACE_REFERENCE_ORDER, Y.TRACE_WIDE):
         got, _ = ctx.trace(sel, Y.TRACE_CLOSEST | walk)
@@ -311,29 +325,26 @@ def test_c2_soup_1m_tris_1080p_matches_reference_run_here():
         ties = m & (got["prim"] != want["prim"])
         assert ties.sum() == 0 if walk == Y.TRACE_REFERENCE_ORDER else ties.sum() <= 4, f"C2: {ties.sum()} hit ids differ"
     sel[:, 7] = np.where(m, want["t"] * 0.5, 1e30)
-    want_any = H.oracle_trace(sp, sel, "any")
+    want_any, _ = ctx.trace(sel, Y.TRACE_ANY | Y.TRACE_REFERENCE_ORDER)
+    assert H.digest(want_any["didHit"]) == rec["any"], "C2: any-hit results of the reference-order walk differ from the reference's"
     for walk in (Y.TRACE_REFERENCE_ORDER, Y.TRACE_WIDE):
         got_any, _ = ctx.trace(sel, Y.TRACE_ANY | walk)
         assert np.array_equal(got_any["didHit"], want_any["didHit"])
     ctx.close()
 
 
-@needs_oracle
 def test_c4_mclaren_shape_2m_tris_1080p_matches_reference_run_here():
     """configs[3] shape at full size (≈ 2 M tris, clearcoat / chrome / thin + solid glass with volume, emissive
-    lamps + env), 1920x1080, full MIS+NEE paths, 1 spp, against the reference run on this box; plus determinism
-    and tile shards summing to the full frame."""
-    from yart_b200 import scenes
-    kw = dict(n_tris=2_000_000, env_res=512)
-    sp, cam = H.scene_file("mclaren", **kw), scenes.mclaren(n_tris=100, env_res=4).camera
-    sc = Y.Scene(sp)
+    lamps + env), 1920x1080, full MIS+NEE paths, 1 spp, against the reference's frame (the reference-order walk's
+    frame stands for it once it matches the recorded digests); plus determinism and tile shards summing to the full
+    frame."""
+    sc, *a = render_config(C4)
     assert sc.n_tris > 1_800_000
-    ref = H.oracle_render(sp, 1920, 1080, 1, cam, first=1, max=1, tonemap="agx")
-    w, h = 1920, 1080
-    a = _render_ctx(sc, cam, w, h, 1, [1])
-    _check_frame_against_oracle("C4", ref, *a)
+    _check_frame_recorded("C4", "c4_mclaren_1080p_1spp", *a)
+    ref = dict(hdr=a[0], ldr=a[1], rays=int(a[2].raysReference))
+    cam, w, h = H.scene_camera("mclaren", **C4["kw"]), C4["w"], C4["h"]
     wide = _render_ctx(sc, cam, w, h, 1, [1], traversal=Y.TRAVERSAL_WIDE)
-    _check_frame_against_oracle("C4", ref, *wide, exact=False)
+    _check_wide_frame("C4", ref, *wide)
     b = _render_ctx(sc, cam, w, h, 1, [1])
     assert H.bits_equal(a[0], b[0]).all() and a[2].raysReference == b[2].raysReference
     assert np.isfinite(a[0]).all() and a[0][..., :3].mean() > 0.01
@@ -342,17 +353,15 @@ def test_c4_mclaren_shape_2m_tris_1080p_matches_reference_run_here():
     assert parts[0][2].raysReference + parts[1][2].raysReference == a[2].raysReference
 
 
-@needs_oracle
 def test_c5_4k_gmon_waves_match_reference_run_here():
     """configs[4] shape: 3840x2160, progressive GMoN waves (15 + 15 samples: m = 3 buckets per wave, blended with
-    finishTile's weights), against the reference run on this box (a two-quad scene so the CPU finishes in seconds)."""
-    sp, cam = H.scene_file("two_quads"), H.scene_camera("two_quads")
-    w, h = 3840, 2160
-    ref = H.oracle_render(sp, w, h, 30, cam, first=15, max=15, tonemap="agx", maxdepth=2)
-    hdr, ldr, st = _render_ctx(Y.Scene(sp), cam, w, h, 30, [15, 15], max_depth=2)
-    _check_frame_against_oracle("C5", ref, hdr, ldr, st)
-    hdr, ldr, st = _render_ctx(Y.Scene(sp), cam, w, h, 30, [15, 15], max_depth=2, traversal=Y.TRAVERSAL_WIDE)
-    _check_frame_against_oracle("C5", ref, hdr, ldr, st, exact=False)
+    finishTile's weights), against the reference's frame (a two-quad scene so the CPU reference finishes in seconds);
+    the reference-order walk's frame stands for it in the check of the wide walk once it matches the recorded digests."""
+    _, hdr, ldr, st = render_config(C5)
+    _check_frame_recorded("C5", "c5_two_quads_4k_30spp", hdr, ldr, st)
+    ref = dict(hdr=hdr, ldr=ldr, rays=int(st.raysReference))
+    _, hdr, ldr, st = render_config(C5, traversal=Y.TRAVERSAL_WIDE)
+    _check_wide_frame("C5", ref, hdr, ldr, st)
 
 
 def test_c5_4k_progressive_gmon_sharded_equals_unsharded():

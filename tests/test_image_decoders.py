@@ -41,6 +41,13 @@ def test_radiance_floats_equal_stbi_loadf(path):
     assert got.shape == want.shape and np.array_equal(got.view(np.uint32), want.view(np.uint32))
 
 
+@pytest.mark.parametrize("path", LDR[::3], ids=os.path.basename)
+def test_srgb_channel_conversion_equals_the_reference(path):
+    """The sRGB → gamma-2 channel conversion of loadTexture, against the reference's (tests/golden/reference_digests.json)."""
+    got = Y.decode_texture(open(path, "rb").read(), S.SRGB, [1, 2])
+    assert H.digest(got) == H.recorded(f"texload_{os.path.basename(path)}_{S.SRGB}_12")
+
+
 @pytest.mark.skipif(not H.have_oracle(), reason="oracle/_ref/oracle_ref not present")
 @pytest.mark.parametrize("path", LDR[::3], ids=os.path.basename)
 def test_recorded_expectations_are_the_reference_run_now(path, tmp_path):

@@ -136,3 +136,18 @@ def test_survey_appendix_c_function_vectors():
     s = np.array([[i % 5, 0.5 * (i % 3), 100.0 if i == 7 else 1.0] for i in range(16)], np.float32)
     out = H.oracle_kat("gmon", struct.pack("<II", 16, 1) + s.tobytes())
     assert np.array_equal(out[:3], np.array([1.88888884, 0.5, 7.5999999], np.float32))
+
+
+@needs_oracle
+def test_recorded_digests_are_the_reference_run_now(hostsim_lib):
+    """tests/golden/reference_digests.json, which the parity tests compare with, is what the reference computes today
+    for their inputs (tests/golden/record_digests.py)."""
+    import json
+    import sys
+    sys.path.insert(0, H.GOLDEN)
+    import record_digests
+    with open(H.REFERENCE_DIGESTS) as f:
+        want = json.load(f)
+    got = record_digests.reference_outputs()
+    assert sorted(got) == sorted(want)
+    assert [k for k in sorted(want) if got[k] != want[k]] == []
