@@ -23,8 +23,8 @@ def case_settings(seed):
                 tile=16 if seed % 2 else 64)
 
 
-def render_case(seed, integrator="mis", scrambler="fastowen", sampler="sobol"):
-    """Renders random scene `seed` with the active library: (render data, hdr, ldr)."""
+def render_case(seed, integrator="mis", scrambler="fastowen", sampler="sobol", traversal=None):
+    """Renders random scene `seed` with the active library (and `traversal`, if given): (render data, hdr, ldr)."""
     k = case_settings(seed)
     cam, w, h = k["cam"], k["w"], k["h"]
     s = Y.Scene(k["path"])
@@ -33,7 +33,8 @@ def render_case(seed, integrator="mis", scrambler="fastowen", sampler="sobol"):
                    background=k["bg"], tonemap=TM[k["tonemap"]], tile_size=k["tile"],
                    integrator=Y.INTEGRATOR_NAIVE if integrator == "naive" else Y.INTEGRATOR_MIS,
                    scrambler={"fastowen": Y.SCRAMBLER_FAST_OWEN, "owen": Y.SCRAMBLER_OWEN, "binary": Y.SCRAMBLER_BINARY_PERMUTE}[scrambler],
-                   sampler={"sobol": Y.SAMPLER_SOBOL, "naive": Y.SAMPLER_NAIVE, "stratified": Y.SAMPLER_STRATIFIED}[sampler])
+                   sampler={"sobol": Y.SAMPLER_SOBOL, "naive": Y.SAMPLER_NAIVE, "stratified": Y.SAMPLER_STRATIFIED}[sampler],
+                   traversal=traversal)
     d = r.render_sync()
     hdr, ldr, _ = r.read()
     r.close()

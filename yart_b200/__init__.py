@@ -45,11 +45,15 @@ class YartError(RuntimeError):
 
 def _check(rc, what, detail=b""):
     if rc != 0:
-        names = {-1: "INVALID", -2: "CUDA", -3: "NO_SCENE", -4: "NO_DEVICE", -5: "STATE", -6: "IO",
-                 -7: "UNSUPPORTED (this build folds the variant away: load capi.SAMPLERS_LIB for the RNG samplers)",
+        names = {-1: "INVALID", -2: "CUDA", -3: "NO_SCENE", -4: "NO_DEVICE", -5: "STATE", -6: "IO", -7: "UNSUPPORTED",
                  -8: "ABORTED"}
         msg = detail.decode() if isinstance(detail, bytes) else str(detail)
         raise YartError(f"{what} failed: YC_ERR_{names.get(rc, rc)} {msg}")
+
+
+_NO_DEVICE = b"(no usable CUDA device: yart_b200 has no CPU fallback)"
+# yc_create returns UNSUPPORTED only for a sampler variant that the default library folds away
+_SAMPLERS_HINT = b"(this build folds the sampler variants away: load capi.SAMPLERS_LIB for the RNG samplers)"
 
 
 def _f3(v):
@@ -187,8 +191,8 @@ class Context:
         opts.traceRefillMin, opts.traceInnerMin = refill_min, inner_min  # traversal scheduling knobs (0 = default)
         opts.tailThreshold = 0xffffffff if tail_threshold < 0 else tail_threshold  # tail kernel hand-over (-1 = never)
         opts.sharedStackEntries = sh_stack_entries  # shared traversal-stack entries in use (0 = default; small = spill-path test)
-        _check(lib().yc_create(device, C.byref(opts), C.byref(self._h)), "yc_create",
-               b"(no usable CUDA device: yart_b200 has no CPU fallback)")
+        rc = lib().yc_create(device, C.byref(opts), C.byref(self._h))
+        _check(rc, "yc_create", _SAMPLERS_HINT if rc == capi.YC_ERR_UNSUPPORTED else _NO_DEVICE)
         self.frame = None
 
     def close(self):
@@ -390,7 +394,7 @@ class Renderer:
             what = "yr_create_dist"
         else:
             rc, what = lib().yr_create(C.byref(s), sh, C.byref(camera), C.byref(self._h)), "yr_create"
-        _check(rc, what, b"(no usable CUDA device: yart_b200 has no CPU fallback)")
+        _check(rc, what, _NO_DEVICE if rc == capi.YC_ERR_NO_DEVICE else b"")
 
     def close(self):
         if self._h:

@@ -834,9 +834,16 @@ extern "C" int yc_upload_scene(yc_ctx* ctx, const YcScene* s) {
     std::vector<WideNode> wn;
     std::vector<WideMesh> wm(s->nMeshes);
     int depth = 0;
-    for (uint32_t mi = 0; mi < s->nMeshes; mi++)
-      depth = std::max(depth, collapseToWide(s->bvhNodes + s->meshes[mi].nodeOffset, s->meshes[mi], wn, wm[mi]));
-    if (3 * depth <= kMaxStack) {
+    bool quantised = true;  // every mesh's boxes fit the quantised grid (quantiseWideNode)
+    for (uint32_t mi = 0; mi < s->nMeshes; mi++) {
+      const int dm = collapseToWide(s->bvhNodes + s->meshes[mi].nodeOffset, s->meshes[mi], wn, wm[mi]);
+      quantised = quantised && dm >= 0;
+      depth = std::max(depth, dm);
+    }
+    if (!quantised) {
+      if (ctx->opts.traversal == YC_TRAVERSAL_WIDE)
+        return fail(ctx, YC_ERR_UNSUPPORTED, "YC_TRAVERSAL_WIDE: a mesh's extent does not fit the wide nodes' quantised grid");
+    } else if (3 * depth <= kMaxStack) {
       const WideNode* dw = nullptr;
       if (wn.empty()) wn.emplace_back();
       YC_TRY(devUpload(ctx, wn.data(), wn.size(), &dw));

@@ -14,17 +14,38 @@
 //       qlo.x qhi.x qlo.y qhi.y qlo.z qhi.z   one byte per child: plane = P + q * Q, rounded OUTWARDS            24 B
 //                              (floor / ceil with a 1/128-quantum guard), so a quantised box contains the child's box
 //       ref[4]                 YcBvhNode::ref encoding, kWideEmpty = unused slot                                   16 B
-//   Per visit a lane forms, per axis,  Sd = S / d  and  Bd = (p' - o) / d  (one FMUL + one FFMA), and per child plane one
-//   PRMT that drops the byte into mantissa bits 8..15 of 1.0f (v = 1 + q / 32768, exact) and one FFMA  t = v * Sd + Bd
-//   = (P + q * Q - o) / d;  near / far planes are picked per axis on the packed words with the ray's sign masks
-//   (6 bit-selects per visit, not 24).
+//   Per visit a lane forms, per axis,  Sd = S / d  and  Bn, Bf = (p' - o) / d  moved down / up by the origin term below
+//   (one FMUL + three FFMA), and per child plane one PRMT that drops the byte into mantissa bits 8..15 of 1.0f
+//   (v = 1 + q / 32768, exact) and one FFMA  t = v * Sd + B = (P + q * Q - o) / d;  near / far planes are picked per
+//   axis on the packed words with the ray's sign masks (6 bit-selects per visit, not 24).
+//
+// Error bound of the box test (u = 2^-24; per axis, w = 1 / d exactly, X = a plane, o the ray origin; every float
+// operation rounds to nearest, so each contributes a relative error of at most u):
+//   idir = w (1 + e1),  odir = -o idir (1 + e2),  Sd = S idir (1 + e3),  Bd = (p' idir + odir) (1 + e4),
+//   t = (v Sd + Bd) (1 + e5).  With X = p' + v S exactly this is
+//     t = (1 + e1)(1 + e5) [ (X - o) w  +  v S w e3  +  (p' - o) w e4  -  o w e2 (1 + e4) ],
+//   and since |p' - o| <= |X - o| + v S:
+//     |t - (X - o) w|  <=  2.02 u v S |w|  +  3 u |X| |w|  +  4 u |o| |w|   (to first order in u).
+//   * 2.02 u v S |w| <= Q |w| / 253 (v < 1.008, S = 2^15 Q): held by the 1/128-quantum guard of the outward rounding.
+//   * the |X| term is held by growing every child box by kWideSlack |corner| before quantising (host, exact in double;
+//     float-corner boxes in slabWideBox: at run time).
+//   * the |o| term is held per ray: odn = odir - kWideSlack |odir| feeds the near planes, odir + >= kWideSlack |odir|
+//     (farOffset) the far ones; that fused add is one more rounding inside B, covered by the same terms.
+// kWideSlack = 16 u also covers what testTriangle's own float arithmetic does to an accepted hit: s = o - p0 and its
+// cross and dot products round relative to each component of s, which moves the tested ray by up to ~6 u |o - p0| per
+// axis, that is 6 u (|o| + |X|) |w| in t.  So the computed [near, far] of a box contains the t of every hit that
+// testTriangle accepts inside it (tests/test_wide_bvh_robustness.py checks this against a float64 brute force at far
+// origins and tiny nodes), except where det is so small that the triangle test's t itself is off by more than the
+// slack (rays grazing a triangle's plane: relative t error ~ u / sin of the angle).  Planes whose S would not be a
+// finite float (extents beyond ~1.3e36) or non-finite boxes are refused: the scene then has no wide layout.
 //
 // What differs from the reference-order BVH2 walk (traverse.cuh), and why results still match:
-//   * box culling only.  The set of triangles tested is a superset / reordering of the reference's, every
+//   * box culling only.  The set of triangles tested is a superset / reordering of the reference's (bound above), every
 //     triangle test is the reference's arithmetic (testTriangle, -fmad=false), and the closest hit is the
 //     minimum over accepted tests.  Hit ids / t / u / v are therefore identical except where two triangles tie
 //     in t to the last bit, or where a hit sits on the boundary of a box that the reference's own slab test
-//     (`bmin * idir + odir`, two roundings, not conservative) culls.  tests/ count those.
+//     (`bmin * idir + odir`, two roundings, not conservative) culls: there the wide walk finds the hit and the
+//     reference misses it.  tests/ count those.
 //   * a zero direction component is clamped to ±1e-20 for the BOX test only (Aila-Laine), so a ray with
 //     d.x == 0 and o.x == 0 no longer has NaN slabs on that axis and no longer walks every box that overlaps
 //     it in y and z (14 K boxes for one ray of the C2 camera, profiles/README.md "Pathological rays").
@@ -46,6 +67,8 @@
 namespace yb {
 
 constexpr uint32_t kWideEmpty = 0xfffffffdu;  // unused child slot (has the leaf bit; never equals a real leaf ref)
+constexpr float kWideSlack = 0x1p-20f;  // 16 float ulps of 1: the relative widening of the bound in the header
+constexpr int kWideMaxExp = 112;        // largest quantum exponent: S = 2^(e + 15) stays a finite float
 
 struct WideNode {
   float pS[3];      // p' = P - S per axis (rounded down)
@@ -69,37 +92,43 @@ struct WideDraft {
   WideChildBox c[4];
   int n;
 };
-inline void quantiseWideNode(const WideDraft& d, WideNode& node) {
+// Quantises one wide node's child boxes; false when an axis cannot be put on a grid with a finite float S and p'
+// (extents beyond ~1.3e36, or non-finite boxes): the scene then has no wide layout.
+inline bool quantiseWideNode(const WideDraft& d, WideNode& node) {
   const WideChildBox* c = d.c;
   const int n = d.n;
   node = WideNode{};
   // Quantisation grid per axis: quantum Q = 2^e, S = 2^15 Q, p' = the float at or below (low corner - S), grid
   // origin P = p' + S (<= the low corner; P, q * Q and their sums are exact in double).  e is the smallest exponent
-  // for which the planes fit in a byte with the guard below.
+  // for which the planes fit in a byte with the guard below.  The boxes quantised are the children's boxes grown by
+  // kWideSlack of their corners' magnitudes (the position term of the bound in the header).
   for (int a = 0; a < 3; a++) {
+    double cl[4], ch[4];
     double lo = INFINITY, hi = -INFINITY;
-    for (int k = 0; k < n; k++) lo = std::min(lo, double(c[k].lo[a])), hi = std::max(hi, double(c[k].hi[a]));
+    for (int k = 0; k < n; k++) {
+      cl[k] = double(c[k].lo[a]) - double(kWideSlack) * std::fabs(double(c[k].lo[a]));
+      ch[k] = double(c[k].hi[a]) + double(kWideSlack) * std::fabs(double(c[k].hi[a]));
+      lo = std::min(lo, cl[k]), hi = std::max(hi, ch[k]);
+    }
+    if (!std::isfinite(lo) || !std::isfinite(hi)) return false;
     int e = -100;
-    if (hi - lo > 0.0 && std::isfinite(hi - lo)) std::frexp((hi - lo) / 254.0, &e);
-    e = std::max(-100, std::min(100, e));
+    if (hi - lo > 0.0) std::frexp((hi - lo) / 254.0, &e);
+    e = std::max(-100, e);
     for (;; e++) {
+      if (e > kWideMaxExp) return false;
       const double Q = std::ldexp(1.0, e), S = std::ldexp(1.0, e + 15);
       float pS = float(lo - S - Q / 64);  // the origin sits 1/64 quantum below the low corner: a guard for q = 0 too
       if (double(pS) > lo - S - Q / 64) pS = std::nextafterf(pS, -INFINITY);
+      if (!std::isfinite(pS)) return false;
       const double P = double(pS) + S;
-      // outward rounding with a 1/128-quantum guard: the device forms t = v * (S / d) + (p' - o) / d in float, whose
-      // rounding (at the magnitude of S / d) is worth up to ~1/512 of a quantum
-      bool fits = e >= 100;
+      // outward rounding with a 1/128-quantum guard: it holds the S-proportional rounding of the device's plane
+      // distances (header: at most Q / 253)
+      bool fits = true;
       uint32_t ql[4], qh[4];
-      if (!fits) {
-        fits = true;
-        for (int k = 0; k < n && fits; k++) {
-          const double l = std::floor((double(c[k].lo[a]) - P) / Q - 1.0 / 128), h = std::ceil((double(c[k].hi[a]) - P) / Q + 1.0 / 128);
-          fits = l >= 0.0 && h <= 255.0;
-          ql[k] = uint32_t(std::max(0.0, l)), qh[k] = uint32_t(std::max(0.0, std::min(255.0, h)));
-        }
-      } else {
-        for (int k = 0; k < n; k++) ql[k] = 0u, qh[k] = 255u;
+      for (int k = 0; k < n && fits; k++) {
+        const double l = std::floor((cl[k] - P) / Q - 1.0 / 128), h = std::ceil((ch[k] - P) / Q + 1.0 / 128);
+        fits = l >= 0.0 && h <= 255.0;
+        ql[k] = uint32_t(std::max(0.0, l)), qh[k] = uint32_t(std::max(0.0, std::min(255.0, h)));
       }
       if (!fits) continue;
       node.pS[a] = pS, node.S[a] = float(S);
@@ -112,6 +141,7 @@ inline void quantiseWideNode(const WideDraft& d, WideNode& node) {
     }
   }
   for (int k = 0; k < 4; k++) node.ref[k] = k < n ? c[k].ref : kWideEmpty;
+  return true;
 }
 
 // One step of the collapse: the wide node that the BVH2 inner node `ref2` opens into (greedy by surface area, the
@@ -185,6 +215,7 @@ inline int collapseSubtree(const YcBvhNode* bvh2, uint32_t ref2, int depth0, std
   return maxDepth;
 }
 
+// Returns the deepest level, or -1 when a node's boxes cannot be quantised (quantiseWideNode).
 inline int collapseToWide(const YcBvhNode* bvh2, const YcMesh& m, std::vector<WideNode>& out, WideMesh& wm) {
   wm.nodeOffset = uint32_t(out.size());
   wm.rootRef = m.rootRef;
@@ -223,8 +254,10 @@ inline int collapseToWide(const YcBvhNode* bvh2, const YcMesh& m, std::vector<Wi
   const auto tq = std::chrono::high_resolution_clock::now();
   const size_t base = out.size();
   out.resize(base + count);
+  std::atomic<bool> quantised{true};
   auto emitTop = [&](size_t lo, size_t hi) {
-    for (size_t i = lo; i < hi; i++) quantiseWideNode(top[i], out[base + i]);
+    for (size_t i = lo; i < hi; i++)
+      if (!quantiseWideNode(top[i], out[base + i])) quantised = false;
   };
   auto emitPart = [&](size_t p) {
     // local index 0 is the part's root, which lives in the top's slot; local index j >= 1 lives at partBase + j - 1
@@ -233,7 +266,7 @@ inline int collapseToWide(const YcBvhNode* bvh2, const YcMesh& m, std::vector<Wi
       WideDraft d = part[j];
       for (int k = 0; k < d.n; k++)
         if (!(d.c[k].ref & YC_REF_LEAF)) d.c[k].ref = uint32_t(partBase[p] + d.c[k].ref - 1);
-      quantiseWideNode(d, out[base + (j == 0 ? size_t(pending[p].draft) : partBase[p] + j - 1)]);
+      if (!quantiseWideNode(d, out[base + (j == 0 ? size_t(pending[p].draft) : partBase[p] + j - 1)])) quantised = false;
     }
   };
   if (threads == 1) {
@@ -248,7 +281,7 @@ inline int collapseToWide(const YcBvhNode* bvh2, const YcMesh& m, std::vector<Wi
       for (size_t i; (i = next.fetch_add(1)) < parts.size() + 1;) {
         if (i == parts.size()) {
           for (size_t t = 0; t < top.size(); t++)
-            if (!isPendingRoot[t]) quantiseWideNode(top[t], out[base + t]);
+            if (!isPendingRoot[t] && !quantiseWideNode(top[t], out[base + t])) quantised = false;
         } else {
           emitPart(i);
         }
@@ -262,23 +295,29 @@ inline int collapseToWide(const YcBvhNode* bvh2, const YcMesh& m, std::vector<Wi
     fprintf(stderr, "yart_b200 wide collapse: %zu nodes, walk %.1f ms, quantisation %.1f ms\n", count,
             std::chrono::duration<double, std::milli>(tq - tw).count(),
             std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - tq).count());
-  return maxDepth;
+  return quantised ? maxDepth : -1;
 }
 
 // ---- device ------------------------------------------------------------------------------------------
 // Per-ray constants of the wide slab test.
 struct WideRay {
-  V3 idir, odir;          // 1 / d (zero components clamped to ±1e-20) and -o * idir
+  V3 idir;                // 1 / d (zero components clamped to ±1e-20)
+  V3 odn;                 // -o * idir moved down by kWideSlack |o * idir| (near planes; farOffset: far planes)
   uint32_t mx, my, mz;    // all ones where d < 0 on that axis (the near plane of a box is its hi plane), else 0
   YB_DEV void set(V3 o, V3 d) {
     const float eps = 1e-20f;
     const float dx = fabsf(d.x) > eps ? d.x : copysignf(eps, d.x), dy = fabsf(d.y) > eps ? d.y : copysignf(eps, d.y),
                 dz = fabsf(d.z) > eps ? d.z : copysignf(eps, d.z);
     idir = V3(1.0f / dx, 1.0f / dy, 1.0f / dz);
-    odir = V3(-o.x * idir.x, -o.y * idir.y, -o.z * idir.z);
+    const V3 odir(-o.x * idir.x, -o.y * idir.y, -o.z * idir.z);
+    odn = V3(fmaf(fabsf(odir.x), -kWideSlack, odir.x), fmaf(fabsf(odir.y), -kWideSlack, odir.y), fmaf(fabsf(odir.z), -kWideSlack, odir.z));
     mx = dx < 0.0f ? 0xffffffffu : 0u, my = dy < 0.0f ? 0xffffffffu : 0u, mz = dz < 0.0f ? 0xffffffffu : 0u;
   }
 };
+
+// -o * idir moved up by at least kWideSlack |o * idir|, formed from odn where it is needed (one FFMA per axis, no
+// register held for the whole walk): 3 kWideSlack |odn| >= 2 kWideSlack |o * idir| + the two roundings.
+YB_DEV float farOffset(float odn) { return fmaf(fabsf(odn), 3.0f * kWideSlack, odn); }
 
 #ifdef YB_HOSTSIM
 YB_DEV float fmaExact(float a, float b, float c) { return fmaf(a, b, c); }
@@ -287,15 +326,18 @@ YB_DEV float fmaExact(float a, float b, float c) { return __fmaf_rn(a, b, c); }
 #endif
 
 // A box given by its float corners (scene-graph node boxes, mesh root boxes): entry distance in `tn`, true when the
-// slab interval [max(tn, tMin), min(tf, tmx)] is not empty.  fmaxf / fminf drop NaN operands, like the reference's
-// NaN-tolerant rmin / rmax.
+// slab interval [max(tn, tMin), min(tf, tmx)] is not empty.  The corners move outwards by kWideSlack of their
+// magnitude first (the position term of the header's bound; quantised child planes carry it from the host).
+// fmaxf / fminf drop NaN operands, like the reference's NaN-tolerant rmin / rmax.
 YB_DEV bool slabWideBox(const WideRay& w, V3 lo, V3 hi, float tmn, float tmx, float& tn) {
+  lo = V3(fmaf(fabsf(lo.x), -kWideSlack, lo.x), fmaf(fabsf(lo.y), -kWideSlack, lo.y), fmaf(fabsf(lo.z), -kWideSlack, lo.z));
+  hi = V3(fmaf(fabsf(hi.x), kWideSlack, hi.x), fmaf(fabsf(hi.y), kWideSlack, hi.y), fmaf(fabsf(hi.z), kWideSlack, hi.z));
   const V3 nearP(w.mx ? hi.x : lo.x, w.my ? hi.y : lo.y, w.mz ? hi.z : lo.z);
   const V3 farP(w.mx ? lo.x : hi.x, w.my ? lo.y : hi.y, w.mz ? lo.z : hi.z);
-  const float tnx = fmaExact(nearP.x, w.idir.x, w.odir.x), tny = fmaExact(nearP.y, w.idir.y, w.odir.y),
-              tnz = fmaExact(nearP.z, w.idir.z, w.odir.z);
-  const float tfx = fmaExact(farP.x, w.idir.x, w.odir.x), tfy = fmaExact(farP.y, w.idir.y, w.odir.y),
-              tfz = fmaExact(farP.z, w.idir.z, w.odir.z);
+  const float tnx = fmaExact(nearP.x, w.idir.x, w.odn.x), tny = fmaExact(nearP.y, w.idir.y, w.odn.y),
+              tnz = fmaExact(nearP.z, w.idir.z, w.odn.z);
+  const float tfx = fmaExact(farP.x, w.idir.x, farOffset(w.odn.x)), tfy = fmaExact(farP.y, w.idir.y, farOffset(w.odn.y)),
+              tfz = fmaExact(farP.z, w.idir.z, farOffset(w.odn.z));
   tn = fmaxf(fmaxf(tnx, tny), fmaxf(tnz, tmn));
   const float tf = fminf(fminf(tfx, tfy), fminf(tfz, tmx));
   return tn <= tf;
@@ -321,11 +363,12 @@ struct WideSlabs {
 };
 template <int K>
 YB_DEV void slabWideChild(WideSlabs& r, uint32_t one, uint32_t nx, uint32_t ny, uint32_t nz, uint32_t fx, uint32_t fy, uint32_t fz,
-                          float Sx, float Sy, float Sz, float Bx, float By, float Bz, float tmn, float tmx, bool live) {
-  const float tnx = fmaExact(planeUnit<K>(nx, one), Sx, Bx), tny = fmaExact(planeUnit<K>(ny, one), Sy, By),
-              tnz = fmaExact(planeUnit<K>(nz, one), Sz, Bz);
-  const float tfx = fmaExact(planeUnit<K>(fx, one), Sx, Bx), tfy = fmaExact(planeUnit<K>(fy, one), Sy, By),
-              tfz = fmaExact(planeUnit<K>(fz, one), Sz, Bz);
+                          float Sx, float Sy, float Sz, float Bnx, float Bny, float Bnz, float Bfx, float Bfy, float Bfz, float tmn,
+                          float tmx, bool live) {
+  const float tnx = fmaExact(planeUnit<K>(nx, one), Sx, Bnx), tny = fmaExact(planeUnit<K>(ny, one), Sy, Bny),
+              tnz = fmaExact(planeUnit<K>(nz, one), Sz, Bnz);
+  const float tfx = fmaExact(planeUnit<K>(fx, one), Sx, Bfx), tfy = fmaExact(planeUnit<K>(fy, one), Sy, Bfy),
+              tfz = fmaExact(planeUnit<K>(fz, one), Sz, Bfz);
   r.tn[K] = fmaxf(fmaxf(tnx, tny), fmaxf(tnz, tmn));
   const float tf = fminf(fminf(tfx, tfy), fminf(tfz, tmx));
   r.hit[K] = live && r.tn[K] <= tf;
@@ -334,16 +377,18 @@ YB_DEV void slabWideChild(WideSlabs& r, uint32_t one, uint32_t nx, uint32_t ny, 
 YB_DEV WideSlabs slabWide4(const WideRay& w, uint32_t one, float px, float py, float pz, float sx, float sy, float sz, uint32_t qlx,
                            uint32_t qhx, uint32_t qly, uint32_t qhy, uint32_t qlz, uint32_t qhz, float tmn, float tmx, bool live) {
   const float Sx = sx * w.idir.x, Sy = sy * w.idir.y, Sz = sz * w.idir.z;
-  const float Bx = fmaExact(px, w.idir.x, w.odir.x), By = fmaExact(py, w.idir.y, w.odir.y), Bz = fmaExact(pz, w.idir.z, w.odir.z);
+  const float Bnx = fmaExact(px, w.idir.x, w.odn.x), Bny = fmaExact(py, w.idir.y, w.odn.y), Bnz = fmaExact(pz, w.idir.z, w.odn.z);
+  const float Bfx = fmaExact(px, w.idir.x, farOffset(w.odn.x)), Bfy = fmaExact(py, w.idir.y, farOffset(w.odn.y)),
+              Bfz = fmaExact(pz, w.idir.z, farOffset(w.odn.z));
   // bit-select: the hi word where the ray runs against the axis
   const uint32_t nx = (qlx & ~w.mx) | (qhx & w.mx), fx = (qhx & ~w.mx) | (qlx & w.mx);
   const uint32_t ny = (qly & ~w.my) | (qhy & w.my), fy = (qhy & ~w.my) | (qly & w.my);
   const uint32_t nz = (qlz & ~w.mz) | (qhz & w.mz), fz = (qhz & ~w.mz) | (qlz & w.mz);
   WideSlabs r;
-  slabWideChild<0>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bx, By, Bz, tmn, tmx, live);
-  slabWideChild<1>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bx, By, Bz, tmn, tmx, live);
-  slabWideChild<2>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bx, By, Bz, tmn, tmx, live);
-  slabWideChild<3>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bx, By, Bz, tmn, tmx, live);
+  slabWideChild<0>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bnx, Bny, Bnz, Bfx, Bfy, Bfz, tmn, tmx, live);
+  slabWideChild<1>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bnx, Bny, Bnz, Bfx, Bfy, Bfz, tmn, tmx, live);
+  slabWideChild<2>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bnx, Bny, Bnz, Bfx, Bfy, Bfz, tmn, tmx, live);
+  slabWideChild<3>(r, one, nx, ny, nz, fx, fy, fz, Sx, Sy, Sz, Bnx, Bny, Bnz, Bfx, Bfy, Bfz, tmn, tmx, live);
   return r;
 }
 
