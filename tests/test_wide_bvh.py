@@ -4,7 +4,7 @@ triangle ids exact except documented ties (same t to the last bit on another tri
 (in fact bit-exact: the triangle arithmetic is the reference's), frames relMSE < 1e-3 on HDR and after AgX.
 
 CPU part: the product sources compiled for the CPU (tests/hostsim; sequential walk testBVHWide).  The `-m gpu` part
-runs the persistent-warp kernels (trace_wide.cuh) through the same checks."""
+runs the persistent-warp kernels (tracePersistent over WideWalk, trace_kernels.cuh) through the same checks."""
 import os
 
 import numpy as np

@@ -153,19 +153,17 @@ YB_DEV void initTraceState(TraceState& st, float tMax) {
   st.attenuation = V3(1.0f);
 }
 
-// WIDE: walk the collapsed 4-wide BVH (wide_bvh.cuh; scenes without alpha-tested materials only) instead of the
-// reference-order BVH2.
-template <bool ALPHA, bool COUNT, bool WIDE = false>
+// Walk: the BVH layout, Bvh2Walk (reference order, traverse.cuh) or WideWalk (the collapsed 4-wide BVH, wide_bvh.cuh;
+// scenes without alpha-tested materials only).
+template <bool ALPHA, bool COUNT, class Walk = Bvh2Walk>
 YB_DEV void extendStage(const DScene& sc, const WaveParams& w, const PathState& ps, uint32_t i, TravStack& stack,
                         TraceCounters& cnt) {
-  static_assert(!(ALPHA && WIDE), "the wide walk does not reproduce the order of alpha-test sampler draws");
   V3 o, d;
   Sampler smp;
   if (!extendLoad<ALPHA>(w, ps, i, o, d, smp)) return;
   TraceState st;
   initTraceState(st, INFINITY);
-  if (WIDE) traceSceneWide<false, COUNT, false>(sc, o, d, st, stack, cnt);
-  else traceScene<false, ALPHA, COUNT, false>(sc, o, d, st, stack, &smp, cnt);
+  traceScene<Walk, false, ALPHA, COUNT, false>(sc, o, d, st, stack, &smp, cnt);
   extendStore<ALPHA>(ps, i, st, smp);
 }
 
@@ -517,7 +515,7 @@ YB_DEV uint32_t shadowFinish(const PathState& ps, const ShadowQueue& q, uint32_t
 // Without alpha-tested materials nothing observable depends on what an occluded NEE ray finds
 // after its first occluder, so the any-hit walk may stop there (EARLY_OUT = !ALPHA); with them the
 // sampler draws must match the reference's, which keeps walking (ray-integrator.cpp:121).
-template <bool ALPHA, bool COUNT, bool WIDE = false>
+template <bool ALPHA, bool COUNT, class Walk = Bvh2Walk>
 YB_DEV uint32_t shadowStage(const DScene& sc, const WaveParams& w, const PathState& ps, const ShadowQueue& q,
                             uint32_t j, TravStack& stack, TraceCounters& cnt) {
   V3 o, d;
@@ -526,8 +524,7 @@ YB_DEV uint32_t shadowStage(const DScene& sc, const WaveParams& w, const PathSta
   const uint32_t i = shadowLoad<ALPHA>(w, ps, q, j, o, d, tMax, smp);
   TraceState st;
   initTraceState(st, tMax);
-  const bool occluded = WIDE ? traceSceneWide<true, COUNT, true>(sc, o, d, st, stack, cnt)
-                             : traceScene<true, ALPHA, COUNT, !ALPHA>(sc, o, d, st, stack, &smp, cnt);
+  const bool occluded = traceScene<Walk, true, ALPHA, COUNT, !ALPHA>(sc, o, d, st, stack, &smp, cnt);
   return shadowFinish<ALPHA>(ps, q, j, i, st, occluded, smp);
 }
 

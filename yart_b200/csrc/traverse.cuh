@@ -11,6 +11,9 @@
 // carries both children's boxes (one 64-B record per visit), leaves are contiguous runs of
 // pre-gathered triangles, and the traversal stack lives in shared memory (first kShStack
 // entries, one column per thread) with a local-memory spill for deeper trees.
+//
+// Bvh2Walk is this layout as the scene walks see it (traceScene here, tracePersistent in trace_kernels.cuh);
+// WideWalk (wide_bvh.cuh) is the 4-wide one.
 #pragma once
 #include "sampler.cuh"
 #include "scene_dev.cuh"
@@ -103,6 +106,85 @@ struct TravStack {
     }
   }
 };
+
+#ifndef YB_HOSTSIM
+constexpr int kTraceBlock = 128;       // 4 warps per CTA of the persistent kernels (trace_kernels.cuh)
+
+// Scheduling knobs (they change only how lanes are grouped, never a ray's own test sequence).
+struct TraceTuning {
+  int refillMin;  // refill the warp from the queue when at least this many lanes are idle
+  int innerMin;   // keep stepping inner nodes while at least this many lanes sit on one
+  int shEntries;  // shared-memory stack entries in use (2..kPsStack; the rest spills): tests shrink it to exercise the spill path
+};
+
+// Per-lane traversal stack of the persistent kernels: packed (ref, d) entries, [entry][thread] in shared
+// memory (one 64-bit access per push / pop, conflict-free), global spill area beyond kPsStack entries.
+// The stack pointer is the shared-memory byte address of the next free slot, so push / pop are one
+// add and one LDS.64 / STS.64; entry 0 holds a sentinel (kNoRef) written when a mesh is entered, so a
+// pop never tests for "empty": popping the sentinel yields kNoRef = "this mesh is walked".
+constexpr int kPsStack = kShStack + 1;
+constexpr uint32_t kPsStride = kTraceBlock * 8;  // bytes between consecutive entries of one thread
+constexpr int kSpillEntries = kMaxStack;         // global spill entries per thread (covers the smallest shared stack)
+constexpr uint32_t kNoRef = 0xffffffffu;   // "no current node" (has the leaf bit: never stepped as inner)
+constexpr uint32_t kPopRef = 0xfffffffeu;  // "pop at the top of the next inner step" (leaf bit set as well)
+struct WarpStack {
+  uint32_t base;   // shared address of this thread's entry 0
+  uint32_t limit;  // base + kPsStack * kPsStride: first address that lives in the spill area
+  uint2** spillBase;  // in shared memory: the spill area's base pointer (only the rare path reads it)
+  __device__ __forceinline__ void init(uint2* shStack, uint2** shSpill, uint2* spill, int shEntries) {
+    base = uint32_t(__cvta_generic_to_shared(shStack + threadIdx.x));  // rarely needed: may be recomputed
+    const uint32_t l = base + uint32_t(shEntries) * kPsStride;
+    asm volatile("mov.u32 %0, %1;" : "=r"(limit) : "r"(l));  // opaque: compared at every push / pop, kept in a register
+    if (threadIdx.x == 0) *shSpill = spill;
+    __syncthreads();
+    spillBase = shSpill;
+  }
+  // rare path (trees deeper than kShStack): everything is derived here so nothing of it stays live
+  __device__ __noinline__ static uint2* spillSlot(uint2** spillBase, uint32_t off) {
+    return *spillBase + size_t(blockIdx.x * kTraceBlock + threadIdx.x) * kSpillEntries + off / kPsStride;
+  }
+  __device__ __forceinline__ void put(uint32_t sa, uint32_t ref, float d) const {
+    asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(sa), "r"(ref), "r"(__float_as_uint(d)));
+  }
+  // push / pop under a lane predicate: the shared-memory access is a single predicated instruction and
+  // only the (rare) spill case branches.
+  __device__ __forceinline__ void pushIf(bool on, uint32_t& sa, uint32_t ref, float d) const {
+    if (on && sa < limit) put(sa, ref, d);
+    if (on && sa >= limit) {
+      if (sa < base + uint32_t(kMaxStack + 1) * kPsStride) *spillSlot(spillBase, sa - limit) = make_uint2(ref, __float_as_uint(d));
+    }
+    if (on) sa += kPsStride;
+  }
+  __device__ __forceinline__ void popIf(bool on, uint32_t& sa, uint32_t& ref, float& d) const {
+    if (on) sa -= kPsStride;
+    uint32_t x = ref, y = __float_as_uint(d);
+    if (on && sa < limit) asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(x), "=r"(y) : "r"(sa));
+    if (on && sa >= limit) {
+      const uint2 v = *spillSlot(spillBase, sa - limit);
+      x = v.x, y = v.y;
+    }
+    ref = x;
+    d = __uint_as_float(y);
+  }
+  __device__ __forceinline__ void pop(uint32_t& sa, uint32_t& ref, float& d) const { popIf(true, sa, ref, d); }
+};
+
+// One 64-byte inner-node record as two 256-bit read-only loads (LDG.E.256, new on sm_100): half the
+// L1 wavefronts of four 128-bit loads — the traversal kernels are bound by the LSU data pipe.
+struct NodeRec {
+  float f[16];
+};
+__device__ __forceinline__ NodeRec loadNode(const float4* p) {
+  NodeRec n;
+  asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=f"(n.f[0]), "=f"(n.f[1]), "=f"(n.f[2]), "=f"(n.f[3]), "=f"(n.f[4]), "=f"(n.f[5]), "=f"(n.f[6]), "=f"(n.f[7])
+               : "l"(p));
+  asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : "=f"(n.f[8]), "=f"(n.f[9]), "=f"(n.f[10]), "=f"(n.f[11]), "=f"(n.f[12]), "=f"(n.f[13]), "=f"(n.f[14]), "=f"(n.f[15])
+               : "l"(p + 2));
+  return n;
+}
+#endif
 
 // What a NEE (any-hit) ray accumulates: Hit::attenuation (hit.hpp:12).
 struct TraceState {
@@ -225,9 +307,65 @@ YB_DEV bool testBVH(const DScene& sc, const YcMesh& mesh, const LocalRay& r, int
   return didHit;
 }
 
-// testNode over the whole scene graph (DFS pre-order with skip links instead of recursion).
-// `st.hit.t` must be preset (inf for closest hits, tMax for NEE rays).  Returns didHit.
-template <bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT>
+// A BVH layout as the scene walks use it: what differs between the reference-order BVH2 (here) and the 4-wide
+// quantised BVH (WideWalk, wide_bvh.cuh).
+//   Ray               per-ray box state, set(o, d); a LocalRay whose o / d the triangle tests read
+//   box<COUNT>        float-corner box test (scene-graph node boxes, mesh root boxes)
+//   mesh<…>           one mesh's sequential walk (traceScene)
+// and, for the persistent kernels only (CUDA):
+//   nodes, rootRef    mesh mi's node array and root ref
+//   parks(COUNT)      whether the persistent walk parks leaves; kParkBelow: int32_t(ref) < kParkBelow is a leaf to park
+//   inner<COUNT>      one inner-node visit of the persistent walk: the next `cur` / `dcur` (kPopRef: pop), pushes
+struct Bvh2Walk {
+  using Ray = LocalRay;
+  template <bool COUNT>
+  YB_DEV static bool box(const Ray& r, V3 lo, V3 hi, float tmx, float& d, TraceCounters& cnt) {
+    return slab<COUNT>(r, lo, hi, kTMin, tmx, d, cnt);
+  }
+  template <bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT>
+  YB_DEV static bool mesh(const DScene& sc, int mi, const Ray& r, int nodeIdx, TraceState& st, TravStack& stack, Sampler* smp,
+                          TraceCounters& cnt) {
+    return testBVH<NEE, ALPHA, COUNT, EARLY_OUT>(sc, sc.meshes[mi], r, nodeIdx, st, stack, smp, cnt);
+  }
+#ifndef YB_HOSTSIM
+  __device__ __forceinline__ static const float4* nodes(const DScene& sc, int, const YcMesh& mesh) {
+    return sc.bvhNodes + 4 * size_t(mesh.nodeOffset);
+  }
+  __device__ __forceinline__ static uint32_t rootRef(const DScene&, int, const YcMesh& mesh) { return mesh.rootRef; }
+  // counting builds reproduce the reference's box-test counts: no parking there
+  __host__ __device__ static constexpr bool parks(bool count) { return !count; }
+  static constexpr int32_t kParkBelow = -2;  // a leaf (bit 31) other than kNoRef / kPopRef
+  template <bool COUNT>
+  __device__ __forceinline__ static void inner(const Ray& r, const float4* nodes, float hitT, const WarpStack& stack, uint32_t& sp,
+                                               uint32_t& cur, float& dcur, const TraceTuning&, TraceCounters& cnt) {
+    const NodeRec nr = loadNode(nodes + 4 * size_t(cur));
+    // testBVH's pop-time cull `d < hit.t` (ray-integrator.cpp:100): an entry that fails it is
+    // dropped without testing its children — here both tests are made to fail (tmax = -inf)
+    const bool live = dcur < hitT;
+    const float tmx = live ? hitT : -INFINITY;
+    float d1, d2;
+    const bool hit1 = slabLive(r, V3(nr.f[0], nr.f[1], nr.f[2]), V3(nr.f[3], nr.f[4], nr.f[5]), kTMin, tmx, d1);
+    const bool hit2 = slabLive(r, V3(nr.f[6], nr.f[7], nr.f[8]), V3(nr.f[9], nr.f[10], nr.f[11]), kTMin, tmx, d2);
+    if (COUNT && live) cnt.box += 2;
+    const uint32_t c1 = __float_as_uint(nr.f[12]), c2 = __float_as_uint(nr.f[13]);
+    // testBVH's descend / push / pop decisions (ray-integrator.cpp:131-152) as selects
+    const bool both = hit1 && hit2;
+    const bool swapped = both && d1 > d2;
+    const bool first = hit1 && !swapped;
+    const uint32_t farRef = swapped ? c1 : c2;
+    const float farD = swapped ? d1 : d2;
+    const uint32_t nearRef = first ? c1 : c2;
+    const float nearD = first ? d1 : d2;
+    stack.pushIf(both, sp, farRef, farD);
+    cur = (hit1 || hit2) ? nearRef : kPopRef;
+    dcur = nearD;
+  }
+#endif
+};
+
+// testNode over the whole scene graph (DFS pre-order with skip links instead of recursion), each mesh walked in
+// Walk's layout.  `st.hit.t` must be preset (inf for closest hits, tMax for NEE rays).  Returns didHit.
+template <class Walk, bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT>
 YB_DEV bool traceScene(const DScene& sc, V3 origin, V3 dir, TraceState& st, TravStack& stack, Sampler* smp,
                        TraceCounters& cnt) {
   V3 ro[YC_MAX_NODE_DEPTH + 1], rd[YC_MAX_NODE_DEPTH + 1];
@@ -238,18 +376,18 @@ YB_DEV bool traceScene(const DScene& sc, V3 origin, V3 dir, TraceState& st, Trav
   while (i < sc.nNodes) {
     const YcNode& nd = sc.nodes[i];
     const int k = nd.depth;
-    LocalRay r;
+    typename Walk::Ray r;
     // ray-integrator.cpp:26-30: transform.inverse(origin, Point), inverse(dir, Vector); dir NOT renormalised
     r.set(xformRows(nd.inv, ro[k], 1.0f), xformRows(nd.inv, rd[k], 0.0f));
     ro[k + 1] = r.o;
     rd[k + 1] = r.d;
     float d;
-    if (!slab<COUNT>(r, V3(nd.bmin), V3(nd.bmax), kTMin, st.hit.t, d, cnt) || st.hit.t < d) {
+    if (!Walk::template box<COUNT>(r, V3(nd.bmin), V3(nd.bmax), st.hit.t, d, cnt) || st.hit.t < d) {
       i = uint32_t(nd.skip);
       continue;
     }
     if (nd.mesh >= 0) {
-      bool h = testBVH<NEE, ALPHA, COUNT, EARLY_OUT>(sc, sc.meshes[nd.mesh], r, int(i), st, stack, smp, cnt);
+      const bool h = Walk::template mesh<NEE, ALPHA, COUNT, EARLY_OUT>(sc, nd.mesh, r, int(i), st, stack, smp, cnt);
       didHit |= h;
       if (NEE && EARLY_OUT && h) return true;
     }

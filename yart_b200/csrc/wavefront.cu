@@ -24,7 +24,7 @@
 #include "comm.cuh"
 #include "bvh_build.cuh"
 #ifndef YB_HOSTSIM
-#include "trace_wide.cuh"
+#include "trace_kernels.cuh"
 #endif
 
 using namespace yb;
@@ -401,9 +401,9 @@ static void runExtend(yc_ctx* ctx, Lane& L, uint32_t n) {
   HostStack hs;
   TraceCounters cnt;
   if (!ALPHA && ctx->wide && !COUNT)
-    for (uint32_t j = 0; j < n; j++) extendStage<false, false, true>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
+    for (uint32_t j = 0; j < n; j++) extendStage<false, false, WideWalk>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
   else
-    for (uint32_t j = 0; j < n; j++) extendStage<ALPHA, COUNT>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
+    for (uint32_t j = 0; j < n; j++) extendStage<ALPHA, COUNT, Bvh2Walk>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
   ctx->dCounters->boxTests += cnt.box;
   ctx->dCounters->triTests += cnt.tri;
 }
@@ -414,9 +414,9 @@ static void runShadow(yc_ctx* ctx, Lane& L, uint32_t) {
   const uint32_t n = L.ctr[kCtrShadowCount];
   uint32_t contributed = 0;
   if (!ALPHA && ctx->wide && !COUNT)
-    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<false, false, true>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
+    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<false, false, WideWalk>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
   else
-    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<ALPHA, COUNT>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
+    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<ALPHA, COUNT, Bvh2Walk>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
   ctx->dCounters->raysShadow += n;
   ctx->dCounters->raysReference += contributed;
   ctx->dCounters->boxTests += cnt.box;
@@ -432,7 +432,21 @@ static void runNaive(yc_ctx* ctx, Lane& L) {
   ctx->dCounters->raysExtend += rays;
 }
 #else
-// Persistent extend / shadow kernels: IO adapters around tracePersistent (trace_kernels.cuh).
+// Persistent extend / shadow kernels: IO adapters around tracePersistent (trace_kernels.cuh), one kernel per BVH
+// layout; the wide ones serve scenes without alpha-tested materials.
+#ifndef YB_WIDE_MIN_BLOCKS
+#define YB_WIDE_MIN_BLOCKS 7  // 72 registers, no spills (6 CTAs: 80 registers, soup trace 3.32 ms; 7: 3.10 ms; 8 spills: 3.24 ms)
+#endif
+
+// Counting builds add their box and triangle tests to `counters`.
+template <bool COUNT>
+__device__ __forceinline__ void flushCounts(Counters* counters, const TraceCounters& cnt) {
+  if (COUNT) {
+    aggregatedCount(&counters->boxTests, cnt.box);
+    aggregatedCount(&counters->triTests, cnt.tri);
+  }
+}
+
 template <bool ALPHA>
 struct ExtendIO {
   WaveParams w;
@@ -453,11 +467,15 @@ __global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) extendKernel
                                                             TraceTuning tune) {
   ExtendIO<ALPHA> io{w, ps, queue};
   TraceCounters cnt;
-  tracePersistent<false, ALPHA, COUNT, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+  tracePersistent<Bvh2Walk, false, ALPHA, COUNT, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
+  flushCounts<COUNT>(counters, cnt);
+}
+__global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) extendWideKernel(DScene sc, WaveParams w, PathState ps, const uint32_t* queue,
+                                                              uint32_t n, uint32_t* ctr, Counters* counters, uint2* spill,
+                                                              TraceTuning tune) {
+  ExtendIO<false> io{w, ps, queue};
+  TraceCounters cnt;
+  tracePersistent<WideWalk, false, false, false, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
 }
 
 template <bool ALPHA>
@@ -476,52 +494,26 @@ struct ShadowIO {
   }
 };
 
-template <bool ALPHA, bool COUNT>
-__global__ void __launch_bounds__(kTraceBlock, YB_SHADOW_MIN_BLOCKS) shadowKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
-                                                            uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
+// EARLY_OUT = !ALPHA: see shadowStage (integrator.cuh)
+template <class Walk, bool ALPHA, bool COUNT>
+__device__ __forceinline__ void shadowQueue(const DScene& sc, WaveParams w, PathState ps, ShadowQueue sq, uint32_t* ctr, Counters* counters,
+                                            uint2* spill, const TraceTuning& tune) {
   const uint32_t n = ctr[kCtrShadowCount];
   ShadowIO<ALPHA> io{w, ps, sq};
   TraceCounters cnt;
-  // EARLY_OUT = !ALPHA: see shadowStage (integrator.cuh)
-  tracePersistent<true, ALPHA, COUNT, !ALPHA>(sc, io, n, ctr + kCtrShadowHead, spill, tune, cnt);
+  tracePersistent<Walk, true, ALPHA, COUNT, !ALPHA>(sc, io, n, ctr + kCtrShadowHead, spill, tune, cnt);
   aggregatedCount(&counters->raysReference, io.contributed);
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&counters->raysShadow, (unsigned long long)n);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+  flushCounts<COUNT>(counters, cnt);
 }
-
-// The same two kernels over the 4-wide BVH (trace_wide.cuh): scenes without alpha-tested materials.
-#ifndef YB_WIDE_MIN_BLOCKS
-#define YB_WIDE_MIN_BLOCKS 7  // 72 registers, no spills (6 CTAs: 80 registers, soup trace 3.32 ms; 7: 3.10 ms; 8 spills: 3.24 ms)
-#endif
-template <bool COUNT>
-__global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) extendWideKernel(DScene sc, WaveParams w, PathState ps, const uint32_t* queue,
-                                                              uint32_t n, uint32_t* ctr, Counters* counters, uint2* spill,
-                                                              TraceTuning tune) {
-  ExtendIO<false> io{w, ps, queue};
-  TraceCounters cnt;
-  traceWidePersistent<false, COUNT>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+template <bool ALPHA, bool COUNT>
+__global__ void __launch_bounds__(kTraceBlock, YB_SHADOW_MIN_BLOCKS) shadowKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
+                                                            uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
+  shadowQueue<Bvh2Walk, ALPHA, COUNT>(sc, w, ps, sq, ctr, counters, spill, tune);
 }
-
-template <bool COUNT>
 __global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) shadowWideKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
                                                               uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
-  const uint32_t n = ctr[kCtrShadowCount];
-  ShadowIO<false> io{w, ps, sq};
-  TraceCounters cnt;
-  traceWidePersistent<true, COUNT>(sc, io, n, ctr + kCtrShadowHead, spill, tune, cnt);
-  aggregatedCount(&counters->raysReference, io.contributed);
-  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&counters->raysShadow, (unsigned long long)n);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+  shadowQueue<WideWalk, false, false>(sc, w, ps, sq, ctr, counters, spill, tune);
 }
 
 // Tail of a chunk: once only a few thousand paths survive, every further bounce of the wavefront is
@@ -543,7 +535,7 @@ struct TailGatherK {
   }
 };
 
-template <bool ALPHA, bool WIDE>
+template <bool ALPHA, class Walk>
 __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
                                                          const uint32_t* queue, uint32_t n, uint32_t firstBounce,
                                                          Counters* counters, float4* Lout) {
@@ -559,7 +551,7 @@ __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w
     const uint32_t i = queue[j];
     TraceCounters cnt;
     for (uint32_t bounce = firstBounce; bounce < w.maxDepth; bounce++) {
-      extendStage<ALPHA, false, WIDE>(sc, w, ps, i, stack, cnt);
+      extendStage<ALPHA, false, Walk>(sc, w, ps, i, stack, cnt);
       nExtend++;
       ShadowRequest rq;
       const uint32_t r = shadeStage<ALPHA>(sc, w, ps, i, rq, raysRef);
@@ -569,7 +561,7 @@ __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w
         sq.d[j] = make_float4(rq.d.x, rq.d.y, rq.d.z, rq.absDotN);
         sq.lif[j] = make_float4(rq.lif.x, rq.lif.y, rq.lif.z, rq.denom);
         sq.att[j] = make_float4(rq.att.x, rq.att.y, rq.att.z, __uint_as_float(i));
-        raysRef += shadowStage<ALPHA, false, WIDE>(sc, w, ps, sq, j, stack, cnt);
+        raysRef += shadowStage<ALPHA, false, Walk>(sc, w, ps, sq, j, stack, cnt);
         nShadow++;
       }
       if (!(r & kShadeContinue)) break;
@@ -634,22 +626,16 @@ static void runExtend(yc_ctx* ctx, Lane& L, uint32_t n) {
     ev = &ctx->extendEvents[ctx->extendEventsUsed++];
     rt::eventRecord(L.st, ev->first);
   }
-  if (!ALPHA && !COUNT && ctx->wide)
-    extendWideKernel<false><<<traceGrid(ctx, n), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, n, L.ctr, ctx->dCounters,
-                                                                           static_cast<uint2*>(L.spill), tuning(ctx));
-  else
-    extendKernel<ALPHA, COUNT><<<traceGrid(ctx, n), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, n, L.ctr, ctx->dCounters,
-                                                                              static_cast<uint2*>(L.spill), tuning(ctx));
+  const auto kernel = !ALPHA && !COUNT && ctx->wide ? extendWideKernel : extendKernel<ALPHA, COUNT>;
+  kernel<<<traceGrid(ctx, n), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, n, L.ctr, ctx->dCounters, static_cast<uint2*>(L.spill),
+                                                       tuning(ctx));
   if (ev) rt::eventRecord(L.st, ev->second);
 }
 template <bool ALPHA, bool COUNT>
 static void runShadow(yc_ctx* ctx, Lane& L, uint32_t upperBound) {
-  if (!ALPHA && !COUNT && ctx->wide)
-    shadowWideKernel<false><<<traceGrid(ctx, upperBound), kTraceBlock, 0, L.st.s>>>(
-      ctx->ds, L.w, L.ps, L.sq, L.ctr, ctx->dCounters, static_cast<uint2*>(L.spill), tuning(ctx));
-  else
-    shadowKernel<ALPHA, COUNT><<<traceGrid(ctx, upperBound), kTraceBlock, 0, L.st.s>>>(
-      ctx->ds, L.w, L.ps, L.sq, L.ctr, ctx->dCounters, static_cast<uint2*>(L.spill), tuning(ctx));
+  const auto kernel = !ALPHA && !COUNT && ctx->wide ? shadowWideKernel : shadowKernel<ALPHA, COUNT>;
+  kernel<<<traceGrid(ctx, upperBound), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.sq, L.ctr, ctx->dCounters,
+                                                                static_cast<uint2*>(L.spill), tuning(ctx));
 }
 #endif
 
@@ -1189,9 +1175,9 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
     if (tail) {
       const dim3 tg((L.n + kTailBlock - 1) / kTailBlock);
       if (!ALPHA && ctx->wide)
-        tailKernel<false, true><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
+        tailKernel<false, WideWalk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
       else
-        tailKernel<ALPHA, false><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
+        tailKernel<ALPHA, Bvh2Walk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
       rt::eventRecord(L.side, L.evTail);
       ctx->launches++;
     }
@@ -1567,7 +1553,7 @@ YB_DEV Sampler traceHookSampler() {
   return s;
 }
 
-template <bool NEE, bool ALPHA, bool COUNT, bool WIDE = false>
+template <class Walk, bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT>
 YB_DEV void traceOne(const DScene& sc, const YcRay& ray, bool useTMax, YcHit& out, TravStack& stack, TraceCounters& cnt) {
   Sampler smp = traceHookSampler();
   TraceState st;
@@ -1578,8 +1564,7 @@ YB_DEV void traceOne(const DScene& sc, const YcRay& ray, bool useTMax, YcHit& ou
   st.hit.backSide = 0;
   st.attenuation = V3(1.0f);
   const V3 o(ray.o), d(ray.d);
-  const bool did = WIDE ? traceSceneWide<NEE, COUNT, NEE>(sc, o, d, st, stack, cnt)
-                        : traceScene<NEE, ALPHA, COUNT, false>(sc, o, d, st, stack, &smp, cnt);
+  const bool did = traceScene<Walk, NEE, ALPHA, COUNT, EARLY_OUT>(sc, o, d, st, stack, &smp, cnt);
   out.t = st.hit.t;
   out.didHit = did ? 1u : 0u;
   out.prim = did ? st.hit.prim : 0xffffffffu;
@@ -1605,13 +1590,15 @@ struct CompactHit {
 };
 
 #ifdef YB_HOSTSIM
-template <bool NEE, bool ALPHA, bool COUNT, bool WIDE = false>
+// The wide walk stops at an any-hit ray's first occluder, like shadowWideKernel; the reference-order walk keeps the
+// reference's walk (ray-integrator.cpp:121).
+template <bool NEE, bool ALPHA, bool COUNT, bool WIDE>
 static void runTrace(yc_ctx* ctx, const YcRay* rays, uint32_t n, bool useTMax, YcHit* hits, CompactHit* compact) {
   HostStack hs;
   TraceCounters cnt;
   for (uint32_t i = 0; i < n; i++) {
     YcHit h;
-    traceOne<NEE, ALPHA, COUNT, WIDE>(ctx->ds, rays[i], useTMax, h, hs.ts, cnt);
+    traceOne<std::conditional_t<WIDE, WideWalk, Bvh2Walk>, NEE, ALPHA, COUNT, NEE && WIDE>(ctx->ds, rays[i], useTMax, h, hs.ts, cnt);
     if (hits) hits[i] = h;
   }
   (void)compact;
@@ -1671,45 +1658,27 @@ __global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) traceKernel(
                                                            uint2* spill, TraceTuning tune) {
   TraceIO<NEE, ALPHA, COMPACT> io{sc, rays, hits, compact, useTMax};
   TraceCounters cnt;
-  tracePersistent<NEE, ALPHA, COUNT, false>(sc, io, n, head, spill, tune, cnt);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+  tracePersistent<Bvh2Walk, NEE, ALPHA, COUNT, false>(sc, io, n, head, spill, tune, cnt);
+  flushCounts<COUNT>(counters, cnt);
 }
 
+// EARLY_OUT = NEE: an any-hit ray stops at its first occluder, like shadowWideKernel
 template <bool NEE, bool COUNT, bool COMPACT>
 __global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) traceWideKernel(DScene sc, const YcRay* rays, uint32_t n, int useTMax, YcHit* hits,
                                                              CompactHit* compact, uint32_t* head, Counters* counters,
                                                              uint2* spill, TraceTuning tune) {
   TraceIO<NEE, false, COMPACT> io{sc, rays, hits, compact, useTMax};
   TraceCounters cnt;
-  traceWidePersistent<NEE, COUNT>(sc, io, n, head, spill, tune, cnt);
-  if (COUNT) {
-    aggregatedCount(&counters->boxTests, cnt.box);
-    aggregatedCount(&counters->triTests, cnt.tri);
-  }
+  tracePersistent<WideWalk, NEE, false, COUNT, NEE>(sc, io, n, head, spill, tune, cnt);
+  flushCounts<COUNT>(counters, cnt);
 }
 
-template <bool NEE, bool ALPHA, bool COUNT, bool WIDE = false>
+template <bool NEE, bool ALPHA, bool COUNT, bool WIDE>
 static void runTrace(yc_ctx* ctx, const YcRay* rays, uint32_t n, bool useTMax, YcHit* hits, CompactHit* compact) {
-  const int grid = traceGrid(ctx, n);
-  uint2* spill = static_cast<uint2*>(ctx->dSpill);
-  if (WIDE) {
-    if (compact)
-      traceWideKernel<NEE, COUNT, true><<<grid, kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact, ctx->dCtr,
-                                                                             ctx->dCounters, spill, tuning(ctx));
-    else
-      traceWideKernel<NEE, COUNT, false><<<grid, kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact, ctx->dCtr,
-                                                                              ctx->dCounters, spill, tuning(ctx));
-    return;
-  }
-  if (compact)
-    traceKernel<NEE, ALPHA, COUNT, true><<<grid, kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact,
-                                                                              ctx->dCtr, ctx->dCounters, spill, tuning(ctx));
-  else
-    traceKernel<NEE, ALPHA, COUNT, false><<<grid, kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact,
-                                                                               ctx->dCtr, ctx->dCounters, spill, tuning(ctx));
+  const auto kernel = WIDE ? (compact ? traceWideKernel<NEE, COUNT, true> : traceWideKernel<NEE, COUNT, false>)
+                           : (compact ? traceKernel<NEE, ALPHA, COUNT, true> : traceKernel<NEE, ALPHA, COUNT, false>);
+  kernel<<<traceGrid(ctx, n), kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact, ctx->dCtr, ctx->dCounters,
+                                                          static_cast<uint2*>(ctx->dSpill), tuning(ctx));
 }
 #endif
 
@@ -1725,7 +1694,7 @@ static int traceUsesWide(yc_ctx* ctx, int mode, bool* wide) {
 static void dispatchTrace(yc_ctx* ctx, int mode, bool wide, const YcRay* rays, uint32_t n, YcHit* hits, CompactHit* compact) {
   const bool nee = (mode & 0xf) == YC_TRACE_ANY, count = (mode & YC_TRACE_COUNT) != 0, alpha = ctx->ds.hasAlpha != 0;
   const bool useTMax = (mode & YC_TRACE_USE_TMAX) != 0;
-#define YB_TR(N, A, C) runTrace<N, A, C>(ctx, rays, n, useTMax, hits, compact)
+#define YB_TR(N, A, C) runTrace<N, A, C, false>(ctx, rays, n, useTMax, hits, compact)
 #define YB_TW(N, C) runTrace<N, false, C, true>(ctx, rays, n, useTMax, hits, compact)
   if (wide) {
     if (nee) count ? YB_TW(true, true) : YB_TW(true, false);
