@@ -14,8 +14,8 @@ Part B (NEE transparency): stacks of thin transmissive panes with opaque walls a
 A float64 reference decides occlusion and forms the product of |n·d|·base over the panes the ray crosses; both walks
 must match it, and the CUDA records must equal the CPU build's byte for byte.
 
-The CPU part runs the CPU build alone; the `-m gpu` part compares the CUDA kernels (extendWideKernel, shadowWideKernel,
-tailKernel<false, WideWalk>, traceWideKernel) with it.  Every context names its traversal."""
+The CPU part runs the CPU build alone; the `-m gpu` part compares the CUDA kernels (extendKernel, shadowKernel and
+traceKernel over WideWalk, tailKernel<false, WideWalk>) with it.  Every context names its traversal."""
 import functools
 import itertools
 import operator

@@ -50,6 +50,22 @@ def check_trace_wide(path):
     _, st_w = ctx.trace(rays, Y.TRACE_CLOSEST | Y.TRACE_COUNT | Y.TRACE_WIDE)
     _, st_r = ctx.trace(rays, Y.TRACE_CLOSEST | Y.TRACE_COUNT)
     assert st_w.boxTests > 0 and st_r.boxTests > 0 and st_w.triTests > 0
+    # the device-resident hook's compact records (t, u, v, prim, node | backSide << 30) hold what yc_trace reports
+    n = len(rays)
+    rays_dev, hits_dev = ctx.device_alloc(n * 32), ctx.device_alloc(n * 20)
+    ctx.h2d(rays_dev, np.ascontiguousarray(rays, np.float32))
+    for walk in (Y.TRACE_WIDE, Y.TRACE_REFERENCE_ORDER):
+        for mode in (Y.TRACE_CLOSEST, Y.TRACE_ANY):
+            full, _ = ctx.trace(rays, mode | walk)
+            ctx.trace_device(rays_dev, n, hits_dev, mode | walk)
+            c = np.empty(n, Y.COMPACT_HIT_DTYPE)
+            ctx.d2h(c, hits_dev)
+            hit = full["didHit"] == 1
+            assert np.array_equal(c["node"] != -1, hit), f"{name}: compact hit / miss differs ({mode | walk:#x})"
+            assert np.array_equal(c["t"].view(np.uint32), full["t"].view(np.uint32)) and np.array_equal(c["prim"], full["prim"])
+            assert np.array_equal((c["node"][hit] >> 30) & 1, full["backSide"][hit])
+    ctx.device_free(rays_dev)
+    ctx.device_free(hits_dev)
     ctx.close()
     return int(other.sum())
 
@@ -167,7 +183,8 @@ def test_wide_axis_aligned_rays_gpu(cuda_lib):
 @pytest.mark.gpu
 def test_wide_gpu_kernels_equal_the_cpu_build_of_the_same_sources(cuda_lib):
     """The persistent-warp wide kernels and the sequential walk make the same decisions (nearest child by key,
-    slot-order pushes): hit records of 200 K primary rays of the 100 K soup are identical, ties included."""
+    slot-order pushes): hit records of 200 K primary rays of the 100 K soup are identical, ties included, and so are
+    the device-resident hook's compact records of both walks."""
     sc_path = H.scene_file("soup", n_tris=100_000)
     cam = H.scene_camera("soup")
     W, Hh = 640, 360
@@ -179,17 +196,26 @@ def test_wide_gpu_kernels_equal_the_cpu_build_of_the_same_sources(cuda_lib):
         ctx.upload_scene(sc)
         ctx.set_camera(Y.make_camera(W, Hh, cam["focal"], cam["fnum"], cam["pos"], cam["target"]))
         ctx.begin_frame(W, Hh, 1, 64, (0, 0, 0), Y.TONEMAP_NONE)
-        rays_dev = ctx.device_alloc(W * Hh * 32)
+        rays_dev, hits_dev = ctx.device_alloc(W * Hh * 32), ctx.device_alloc(W * Hh * 20)
         ctx.generate_primary_rays(0, 1, rays_dev)
         rays = np.empty((W * Hh, 8), np.float32)
         ctx.d2h(rays, rays_dev)
+        compact = []
+        for mode in (Y.TRACE_CLOSEST, Y.TRACE_ANY):
+            for walk in (Y.TRACE_WIDE, Y.TRACE_REFERENCE_ORDER):
+                ctx.trace_device(rays_dev, W * Hh, hits_dev, mode | walk)
+                c = np.empty(W * Hh, Y.COMPACT_HIT_DTYPE)
+                ctx.d2h(c, hits_dev)
+                compact.append(c.tobytes())
         ctx.device_free(rays_dev)
+        ctx.device_free(hits_dev)
         hits, _ = ctx.trace(rays, Y.TRACE_CLOSEST)
         anyh, _ = ctx.trace(np.concatenate([rays[:, :7], np.full((len(rays), 1), 30.0, np.float32)], 1), Y.TRACE_ANY)
-        recs.append((rays.tobytes(), hits.tobytes(), anyh["didHit"].tobytes()))
+        recs.append((rays.tobytes(), hits.tobytes(), anyh["didHit"].tobytes(), compact))
         ctx.close()
     Y.use_library(cuda_lib)
     assert recs[0][0] == recs[1][0] and recs[0][1] == recs[1][1] and recs[0][2] == recs[1][2]
+    assert recs[0][3] == recs[1][3], "compact records differ"
 
 
 def test_wide_collapse_shared_out_over_threads_cpu_build(hostsim_lib):

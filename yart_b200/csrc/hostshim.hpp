@@ -11,7 +11,22 @@
 struct float4 {
   float x, y, z, w;
 };
+struct uint2 {
+  uint32_t x, y;
+};
+struct uint3 {
+  uint32_t x, y, z;
+};
 static inline float4 make_float4(float x, float y, float z, float w) { return float4{x, y, z, w}; }
+// A kernel is a plain function that rt::launch calls once: one thread of one block runs the whole launch.
+#define __global__
+#define __launch_bounds__(...)
+static const uint3 threadIdx = {0, 0, 0}, blockIdx = {0, 0, 0};
+static inline unsigned long long atomicAdd(unsigned long long* p, unsigned long long v) {
+  const unsigned long long old = *p;
+  *p = old + v;
+  return old;
+}
 template <typename T>
 static inline T __ldg(const T* p) { return *p; }
 static inline uint32_t __brev(uint32_t v) {

@@ -75,6 +75,10 @@ template <int MIN_BLOCKS = 1, class F>
 inline void launchFor(Stream&, uint32_t n, const F& f) {
   for (uint32_t i = 0; i < n; i++) f(i);
 }
+template <class... P, class... A>
+inline void launch(Stream&, int, int, void (*kernel)(P...), const A&... args) {
+  kernel(args...);
+}
 #else
 struct Stream {
   cudaStream_t s = nullptr;
@@ -193,6 +197,11 @@ template <int MIN_BLOCKS = 1, class F>
 inline void launchFor(Stream& st, uint32_t n, const F& f) {
   if (n == 0) return;
   forKernel<F, MIN_BLOCKS><<<(n + 255u) / 256u, 256, 0, st.s>>>(n, f);
+}
+// `kernel` over `grid` CTAs of `block` threads (the CPU build calls it once, hostshim.hpp)
+template <class... P, class... A>
+inline void launch(Stream& st, int grid, int block, void (*kernel)(P...), const A&... args) {
+  kernel<<<grid, block, 0, st.s>>>(args...);
 }
 #endif
 

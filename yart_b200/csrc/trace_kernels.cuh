@@ -1,4 +1,4 @@
-// trace_kernels.cuh — persistent-warp traversal engine (CUDA only) shared by the extend, shadow and
+// trace_kernels.cuh — persistent-warp traversal engine shared by the extend, shadow and
 // ray-hook kernels of both BVH layouts: the reference-order BVH2 (Bvh2Walk, traverse.cuh) and the 4-wide
 // quantised BVH (WideWalk, wide_bvh.cuh).  The layout type supplies the box test, the mesh's nodes, the
 // inner-node step and whether leaves are parked; everything else below is shared.
@@ -21,11 +21,42 @@
 //     through an out-of-line path; no local memory is used.
 // Node records are fetched as two 256-bit read-only loads, triangles as three 128-bit loads.
 // With WideWalk the set of boxes differs, the triangle arithmetic does not (wide_bvh.cuh's header).
+// The CPU build of the product sources has a serial counterpart with the same signature (first below).
 #pragma once
 #include "integrator.cuh"
 
 namespace yb {
 
+#ifdef YB_HOSTSIM
+// A traversal stack for one thread: the shared-memory part as plain arrays.
+struct HostStack {
+  uint32_t ref[kShStack];
+  float d[kShStack];
+  TravStack ts;
+  HostStack() {
+    ts.shRef = ref;
+    ts.shD = d;
+    ts.stride = 1;
+  }
+};
+
+// One lane that takes the items in order: the same load → trace → store bracket per item as the warp engine,
+// with traceScene as the walk.
+template <class Walk, bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT, class IO>
+inline void tracePersistent(const DScene& sc, IO& io, uint32_t n, uint32_t*, uint2*, const TraceTuning, TraceCounters& cnt) {
+  HostStack hs;
+  for (uint32_t j = 0; j < n; j++) {
+    V3 o, d;
+    float tMax;
+    Sampler smp;
+    if (!io.load(j, o, d, tMax, smp)) continue;
+    TraceState st;
+    initTraceState(st, tMax);
+    const bool didHit = traceScene<Walk, NEE, ALPHA, COUNT, EARLY_OUT>(sc, o, d, st, hs.ts, &smp, cnt);
+    io.store(j, st, didHit, smp);
+  }
+}
+#else
 // Ray in the object space of scene node `node`: the chain of inverse transforms root → node, applied
 // in the recursion's order (ray-integrator.cpp:26-30).  The ancestor chain is a host-built table.
 __device__ __forceinline__ void nodeLocalRay(const DScene& sc, uint32_t node, int depth, V3& o, V3& d) {
@@ -213,5 +244,6 @@ __device__ __forceinline__ void tracePersistent(const DScene& sc, IO& io, uint32
     }
   }
 }
+#endif
 
 }  // namespace yb

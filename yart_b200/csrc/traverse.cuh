@@ -107,7 +107,6 @@ struct TravStack {
   }
 };
 
-#ifndef YB_HOSTSIM
 constexpr int kTraceBlock = 128;       // 4 warps per CTA of the persistent kernels (trace_kernels.cuh)
 
 // Scheduling knobs (they change only how lanes are grouped, never a ray's own test sequence).
@@ -123,6 +122,7 @@ struct TraceTuning {
 // add and one LDS.64 / STS.64; entry 0 holds a sentinel (kNoRef) written when a mesh is entered, so a
 // pop never tests for "empty": popping the sentinel yields kNoRef = "this mesh is walked".
 constexpr int kPsStack = kShStack + 1;
+#ifndef YB_HOSTSIM
 constexpr uint32_t kPsStride = kTraceBlock * 8;  // bytes between consecutive entries of one thread
 constexpr int kSpillEntries = kMaxStack;         // global spill entries per thread (covers the smallest shared stack)
 constexpr uint32_t kNoRef = 0xffffffffu;   // "no current node" (has the leaf bit: never stepped as inner)

@@ -16,6 +16,7 @@
 // surviving paths and the NEE requests into the next queues with warp-aggregated appends.
 #include <algorithm>
 #include <cstdarg>
+#include <type_traits>
 #include <vector>
 
 #include "estimator.cuh"
@@ -23,17 +24,17 @@
 #include "rt.cuh"
 #include "comm.cuh"
 #include "bvh_build.cuh"
-#ifndef YB_HOSTSIM
 #include "trace_kernels.cuh"
-#endif
 
 using namespace yb;
 
+// CTAs x 4 warps per SM of the persistent traversal kernels (extend, shadow, ray hooks; both BVH layouts): 72 registers,
+// no spills in the alpha build.  Measured per kernel:
+//   reference-order closest hit: 8 CTAs = 64 registers: Sponza-shaped step 28.4-28.9 ms, 7: 27.2, 6: 27.8 on one box;
+//   reference-order shadow: uncapped 96 registers, 5 CTAs — C2 step 11.5 ms; 7: 10.9; 8 spills: 11.9;
+//   wide walk: 6 CTAs = 80 registers, soup trace 3.32 ms; 7: 3.10 ms; 8 spills: 3.24 ms.
 #ifndef YB_TRACE_MIN_BLOCKS
-#define YB_TRACE_MIN_BLOCKS 7  // CTAs x 4 warps per SM of the reference-order closest-hit kernels: 72 registers, no spills in the alpha build (8 CTAs = 64 registers: Sponza-shaped step 28.4-28.9 ms, 7: 27.2, 6: 27.8 on one box)
-#endif
-#ifndef YB_SHADOW_MIN_BLOCKS
-#define YB_SHADOW_MIN_BLOCKS 7  // 72 registers, no spills (uncapped: 96 registers, 5 CTAs — C2 step 11.5 ms; 7: 10.9; 8 spills: 11.9)
+#define YB_TRACE_MIN_BLOCKS 7
 #endif
 // Resident CTAs (x 256 threads) per SM the three shading kernels are compiled for (registers = 65536 / 256 / CTAs)
 #ifndef YB_RESOLVE_MIN_BLOCKS
@@ -385,62 +386,18 @@ struct RetonemapK {
   }
 };
 
-#ifdef YB_HOSTSIM
-struct HostStack {
-  uint32_t ref[kShStack];
-  float d[kShStack];
-  TravStack ts;
-  HostStack() {
-    ts.shRef = ref;
-    ts.shD = d;
-    ts.stride = 1;
-  }
-};
-template <bool ALPHA, bool COUNT>
-static void runExtend(yc_ctx* ctx, Lane& L, uint32_t n) {
-  HostStack hs;
-  TraceCounters cnt;
-  if (!ALPHA && ctx->wide && !COUNT)
-    for (uint32_t j = 0; j < n; j++) extendStage<false, false, WideWalk>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
-  else
-    for (uint32_t j = 0; j < n; j++) extendStage<ALPHA, COUNT, Bvh2Walk>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt);
-  ctx->dCounters->boxTests += cnt.box;
-  ctx->dCounters->triTests += cnt.tri;
-}
-template <bool ALPHA, bool COUNT>
-static void runShadow(yc_ctx* ctx, Lane& L, uint32_t) {
-  HostStack hs;
-  TraceCounters cnt;
-  const uint32_t n = L.ctr[kCtrShadowCount];
-  uint32_t contributed = 0;
-  if (!ALPHA && ctx->wide && !COUNT)
-    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<false, false, WideWalk>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
-  else
-    for (uint32_t j = 0; j < n; j++) contributed += shadowStage<ALPHA, COUNT, Bvh2Walk>(ctx->ds, L.w, L.ps, L.sq, j, hs.ts, cnt);
-  ctx->dCounters->raysShadow += n;
-  ctx->dCounters->raysReference += contributed;
-  ctx->dCounters->boxTests += cnt.box;
-  ctx->dCounters->triTests += cnt.tri;
-}
-template <bool ALPHA>
-static void runNaive(yc_ctx* ctx, Lane& L) {
-  HostStack hs;
-  TraceCounters cnt;
-  uint32_t rays = 0;
-  for (uint32_t j = 0; j < L.n; j++) naiveStage<ALPHA>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt, rays);
-  ctx->dCounters->raysReference += rays;
-  ctx->dCounters->raysExtend += rays;
-}
-#else
-// Persistent extend / shadow kernels: IO adapters around tracePersistent (trace_kernels.cuh), one kernel per BVH
-// layout; the wide ones serve scenes without alpha-tested materials.
-#ifndef YB_WIDE_MIN_BLOCKS
-#define YB_WIDE_MIN_BLOCKS 7  // 72 registers, no spills (6 CTAs: 80 registers, soup trace 3.32 ms; 7: 3.10 ms; 8 spills: 3.24 ms)
-#endif
+// Which BVH layout a traversal launch walks: the wide one when the context built it (YcOptions::traversal, scenes
+// without alpha-tested materials), unless the launch draws alpha-test samples or counts box / triangle tests (the counts
+// of the reference-order walk define the roofline's algorithmic bytes).  Kernels are picked as
+// `walksWide(…) ? kernel<WideWalk, false, …> : kernel<Bvh2Walk, ALPHA, …>`: the wide walk is never built with ALPHA.
+static bool walksWide(const yc_ctx* ctx, bool alpha, bool count) { return ctx->wide && !alpha && !count; }
+
+// Persistent extend / shadow kernels: IO adapters around tracePersistent (trace_kernels.cuh), one instance per BVH
+// layout.  The CPU build runs the same kernels through tracePersistent's serial counterpart.
 
 // Counting builds add their box and triangle tests to `counters`.
 template <bool COUNT>
-__device__ __forceinline__ void flushCounts(Counters* counters, const TraceCounters& cnt) {
+YB_DEV void flushCounts(Counters* counters, const TraceCounters& cnt) {
   if (COUNT) {
     aggregatedCount(&counters->boxTests, cnt.box);
     aggregatedCount(&counters->triTests, cnt.tri);
@@ -452,30 +409,23 @@ struct ExtendIO {
   WaveParams w;
   PathState ps;
   const uint32_t* queue;
-  __device__ __forceinline__ bool load(uint32_t j, V3& o, V3& d, float& tMax, Sampler& smp) const {
+  YB_DEV bool load(uint32_t j, V3& o, V3& d, float& tMax, Sampler& smp) const {
     tMax = INFINITY;
     return extendLoad<ALPHA>(w, ps, queue[j], o, d, smp);
   }
-  __device__ __forceinline__ void store(uint32_t j, const TraceState& st, bool, const Sampler& smp) const {
+  YB_DEV void store(uint32_t j, const TraceState& st, bool, const Sampler& smp) const {
     extendStore<ALPHA>(ps, queue[j], st, smp);
   }
 };
 
-template <bool ALPHA, bool COUNT>
+template <class Walk, bool ALPHA, bool COUNT>
 __global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) extendKernel(DScene sc, WaveParams w, PathState ps, const uint32_t* queue,
                                                             uint32_t n, uint32_t* ctr, Counters* counters, uint2* spill,
                                                             TraceTuning tune) {
   ExtendIO<ALPHA> io{w, ps, queue};
   TraceCounters cnt;
-  tracePersistent<Bvh2Walk, false, ALPHA, COUNT, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
+  tracePersistent<Walk, false, ALPHA, COUNT, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
   flushCounts<COUNT>(counters, cnt);
-}
-__global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) extendWideKernel(DScene sc, WaveParams w, PathState ps, const uint32_t* queue,
-                                                              uint32_t n, uint32_t* ctr, Counters* counters, uint2* spill,
-                                                              TraceTuning tune) {
-  ExtendIO<false> io{w, ps, queue};
-  TraceCounters cnt;
-  tracePersistent<WideWalk, false, false, false, false>(sc, io, n, ctr + kCtrExtendHead, spill, tune, cnt);
 }
 
 template <bool ALPHA>
@@ -484,20 +434,19 @@ struct ShadowIO {
   PathState ps;
   ShadowQueue sq;
   uint32_t contributed = 0;
-  uint32_t pathOf[1];  // unused
-  __device__ __forceinline__ bool load(uint32_t j, V3& o, V3& d, float& tMax, Sampler& smp) const {
+  YB_DEV bool load(uint32_t j, V3& o, V3& d, float& tMax, Sampler& smp) const {
     shadowLoad<ALPHA>(w, ps, sq, j, o, d, tMax, smp);
     return true;
   }
-  __device__ __forceinline__ void store(uint32_t j, const TraceState& st, bool occluded, const Sampler& smp) {
+  YB_DEV void store(uint32_t j, const TraceState& st, bool occluded, const Sampler& smp) {
     contributed += shadowFinish<ALPHA>(ps, sq, j, __float_as_uint(sq.att[j].w), st, occluded, smp);
   }
 };
 
 // EARLY_OUT = !ALPHA: see shadowStage (integrator.cuh)
 template <class Walk, bool ALPHA, bool COUNT>
-__device__ __forceinline__ void shadowQueue(const DScene& sc, WaveParams w, PathState ps, ShadowQueue sq, uint32_t* ctr, Counters* counters,
-                                            uint2* spill, const TraceTuning& tune) {
+__global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) shadowKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
+                                                            uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
   const uint32_t n = ctr[kCtrShadowCount];
   ShadowIO<ALPHA> io{w, ps, sq};
   TraceCounters cnt;
@@ -506,16 +455,18 @@ __device__ __forceinline__ void shadowQueue(const DScene& sc, WaveParams w, Path
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&counters->raysShadow, (unsigned long long)n);
   flushCounts<COUNT>(counters, cnt);
 }
-template <bool ALPHA, bool COUNT>
-__global__ void __launch_bounds__(kTraceBlock, YB_SHADOW_MIN_BLOCKS) shadowKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
-                                                            uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
-  shadowQueue<Bvh2Walk, ALPHA, COUNT>(sc, w, ps, sq, ctr, counters, spill, tune);
-}
-__global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) shadowWideKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
-                                                              uint32_t* ctr, Counters* counters, uint2* spill, TraceTuning tune) {
-  shadowQueue<WideWalk, false, false>(sc, w, ps, sq, ctr, counters, spill, tune);
-}
 
+#ifdef YB_HOSTSIM
+template <bool ALPHA>
+static void runNaive(yc_ctx* ctx, Lane& L) {
+  HostStack hs;
+  TraceCounters cnt;
+  uint32_t rays = 0;
+  for (uint32_t j = 0; j < L.n; j++) naiveStage<ALPHA>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt, rays);
+  ctx->dCounters->raysReference += rays;
+  ctx->dCounters->raysExtend += rays;
+}
+#else
 // Tail of a chunk: once only a few thousand paths survive, every further bounce of the wavefront is
 // bound by the latency of its slowest ray (launch after launch).  The tail kernel gives each surviving
 // path one thread that runs its remaining bounces to the end — extend → shade → shadow in the same
@@ -598,6 +549,7 @@ template <bool ALPHA>
 static void runNaive(yc_ctx* ctx, Lane& L) {
   naiveKernel<ALPHA><<<(L.n + kTailBlock - 1) / kTailBlock, kTailBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, L.n, ctx->dCounters);
 }
+#endif
 
 static int traceGridMax(const yc_ctx* ctx) { return ctx->smCount * 8; }
 static TraceTuning tuning(const yc_ctx* ctx) {
@@ -626,18 +578,17 @@ static void runExtend(yc_ctx* ctx, Lane& L, uint32_t n) {
     ev = &ctx->extendEvents[ctx->extendEventsUsed++];
     rt::eventRecord(L.st, ev->first);
   }
-  const auto kernel = !ALPHA && !COUNT && ctx->wide ? extendWideKernel : extendKernel<ALPHA, COUNT>;
-  kernel<<<traceGrid(ctx, n), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, n, L.ctr, ctx->dCounters, static_cast<uint2*>(L.spill),
-                                                       tuning(ctx));
+  const auto kernel = walksWide(ctx, ALPHA, COUNT) ? extendKernel<WideWalk, false, false> : extendKernel<Bvh2Walk, ALPHA, COUNT>;
+  rt::launch(L.st, traceGrid(ctx, n), kTraceBlock, kernel, ctx->ds, L.w, L.ps, L.qA, n, L.ctr, ctx->dCounters,
+             static_cast<uint2*>(L.spill), tuning(ctx));
   if (ev) rt::eventRecord(L.st, ev->second);
 }
 template <bool ALPHA, bool COUNT>
 static void runShadow(yc_ctx* ctx, Lane& L, uint32_t upperBound) {
-  const auto kernel = !ALPHA && !COUNT && ctx->wide ? shadowWideKernel : shadowKernel<ALPHA, COUNT>;
-  kernel<<<traceGrid(ctx, upperBound), kTraceBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.sq, L.ctr, ctx->dCounters,
-                                                                static_cast<uint2*>(L.spill), tuning(ctx));
+  const auto kernel = walksWide(ctx, ALPHA, COUNT) ? shadowKernel<WideWalk, false, false> : shadowKernel<Bvh2Walk, ALPHA, COUNT>;
+  rt::launch(L.st, traceGrid(ctx, upperBound), kTraceBlock, kernel, ctx->ds, L.w, L.ps, L.sq, L.ctr, ctx->dCounters,
+             static_cast<uint2*>(L.spill), tuning(ctx));
 }
-#endif
 
 // ---------------------------------------------------------------------------------------
 // lifecycle
@@ -1174,7 +1125,7 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
 #ifndef YB_HOSTSIM
     if (tail) {
       const dim3 tg((L.n + kTailBlock - 1) / kTailBlock);
-      if (!ALPHA && ctx->wide)
+      if (walksWide(ctx, ALPHA, false))  // the tail counts nothing: counting renders keep their wide tail
         tailKernel<false, WideWalk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
       else
         tailKernel<ALPHA, Bvh2Walk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
@@ -1553,35 +1504,6 @@ YB_DEV Sampler traceHookSampler() {
   return s;
 }
 
-template <class Walk, bool NEE, bool ALPHA, bool COUNT, bool EARLY_OUT>
-YB_DEV void traceOne(const DScene& sc, const YcRay& ray, bool useTMax, YcHit& out, TravStack& stack, TraceCounters& cnt) {
-  Sampler smp = traceHookSampler();
-  TraceState st;
-  st.hit.t = (NEE || useTMax) ? ray.tmax : INFINITY;
-  st.hit.node = kHitMiss;
-  st.hit.u = st.hit.v = 0.0f;
-  st.hit.prim = 0xffffffffu;
-  st.hit.backSide = 0;
-  st.attenuation = V3(1.0f);
-  const V3 o(ray.o), d(ray.d);
-  const bool did = traceScene<Walk, NEE, ALPHA, COUNT, EARLY_OUT>(sc, o, d, st, stack, &smp, cnt);
-  out.t = st.hit.t;
-  out.didHit = did ? 1u : 0u;
-  out.prim = did ? st.hit.prim : 0xffffffffu;
-  out.material = -1, out.lightIdx = -1, out.backSide = 0;
-  for (int k = 0; k < 3; k++) out.p[k] = out.n[k] = out.tg[k] = 0.0f;
-  out.uv[0] = out.uv[1] = 0.0f;
-  out.attenuation[0] = st.attenuation.x, out.attenuation[1] = st.attenuation.y, out.attenuation[2] = st.attenuation.z;
-  if (did) {
-    const SurfaceHit s = resolveHit(sc, st.hit, o, d);
-    out.material = s.material, out.lightIdx = s.lightIdx, out.backSide = st.hit.backSide;
-    out.p[0] = s.p.x, out.p[1] = s.p.y, out.p[2] = s.p.z;
-    out.n[0] = s.n.x, out.n[1] = s.n.y, out.n[2] = s.n.z;
-    out.tg[0] = s.tg.x, out.tg[1] = s.tg.y, out.tg[2] = s.tg.z;
-    out.uv[0] = s.uv.x, out.uv[1] = s.uv.y;
-  }
-}
-
 // compact record of the device-resident variant: 20 bytes per hit (t, u, v, prim, node|backSide)
 struct CompactHit {
   float t, u, v;
@@ -1589,23 +1511,6 @@ struct CompactHit {
   int32_t node;
 };
 
-#ifdef YB_HOSTSIM
-// The wide walk stops at an any-hit ray's first occluder, like shadowWideKernel; the reference-order walk keeps the
-// reference's walk (ray-integrator.cpp:121).
-template <bool NEE, bool ALPHA, bool COUNT, bool WIDE>
-static void runTrace(yc_ctx* ctx, const YcRay* rays, uint32_t n, bool useTMax, YcHit* hits, CompactHit* compact) {
-  HostStack hs;
-  TraceCounters cnt;
-  for (uint32_t i = 0; i < n; i++) {
-    YcHit h;
-    traceOne<std::conditional_t<WIDE, WideWalk, Bvh2Walk>, NEE, ALPHA, COUNT, NEE && WIDE>(ctx->ds, rays[i], useTMax, h, hs.ts, cnt);
-    if (hits) hits[i] = h;
-  }
-  (void)compact;
-  ctx->dCounters->boxTests += cnt.box;
-  ctx->dCounters->triTests += cnt.tri;
-}
-#else
 template <bool NEE, bool ALPHA, bool COMPACT>
 struct TraceIO {
   DScene sc;
@@ -1613,7 +1518,7 @@ struct TraceIO {
   YcHit* hits;
   CompactHit* compact;
   int useTMax;
-  __device__ __forceinline__ bool load(uint32_t i, V3& o, V3& d, float& tMax, Sampler& smp) const {
+  YB_DEV bool load(uint32_t i, V3& o, V3& d, float& tMax, Sampler& smp) const {
     const float4 a = __ldg(reinterpret_cast<const float4*>(rays) + 2 * size_t(i));
     const float4 b = __ldg(reinterpret_cast<const float4*>(rays) + 2 * size_t(i) + 1);
     o = V3(a.x, a.y, a.z);
@@ -1622,7 +1527,7 @@ struct TraceIO {
     smp = traceHookSampler();
     return true;
   }
-  __device__ __forceinline__ void store(uint32_t i, const TraceState& st, bool did, const Sampler&) const {
+  YB_DEV void store(uint32_t i, const TraceState& st, bool did, const Sampler&) const {
     if (COMPACT) {
       CompactHit c;
       c.t = st.hit.t, c.u = st.hit.u, c.v = st.hit.v, c.prim = st.hit.prim;
@@ -1652,41 +1557,31 @@ struct TraceIO {
   }
 };
 
-template <bool NEE, bool ALPHA, bool COUNT, bool COMPACT>
+// EARLY_OUT: the wide walk stops at an any-hit ray's first occluder, like the render's shadow kernel; the
+// reference-order walk keeps the reference's walk (ray-integrator.cpp:121), so that `attenuation` is the reference's.
+template <class Walk, bool NEE, bool ALPHA, bool COUNT, bool COMPACT>
 __global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) traceKernel(DScene sc, const YcRay* rays, uint32_t n, int useTMax, YcHit* hits,
                                                            CompactHit* compact, uint32_t* head, Counters* counters,
                                                            uint2* spill, TraceTuning tune) {
   TraceIO<NEE, ALPHA, COMPACT> io{sc, rays, hits, compact, useTMax};
   TraceCounters cnt;
-  tracePersistent<Bvh2Walk, NEE, ALPHA, COUNT, false>(sc, io, n, head, spill, tune, cnt);
+  tracePersistent<Walk, NEE, ALPHA, COUNT, NEE && std::is_same_v<Walk, WideWalk>>(sc, io, n, head, spill, tune, cnt);
   flushCounts<COUNT>(counters, cnt);
 }
 
-// EARLY_OUT = NEE: an any-hit ray stops at its first occluder, like shadowWideKernel
-template <bool NEE, bool COUNT, bool COMPACT>
-__global__ void __launch_bounds__(kTraceBlock, YB_WIDE_MIN_BLOCKS) traceWideKernel(DScene sc, const YcRay* rays, uint32_t n, int useTMax, YcHit* hits,
-                                                             CompactHit* compact, uint32_t* head, Counters* counters,
-                                                             uint2* spill, TraceTuning tune) {
-  TraceIO<NEE, false, COMPACT> io{sc, rays, hits, compact, useTMax};
-  TraceCounters cnt;
-  tracePersistent<WideWalk, NEE, false, COUNT, NEE>(sc, io, n, head, spill, tune, cnt);
-  flushCounts<COUNT>(counters, cnt);
+template <bool NEE, bool ALPHA, bool COUNT>
+static void runTrace(yc_ctx* ctx, bool wide, const YcRay* rays, uint32_t n, bool useTMax, YcHit* hits, CompactHit* compact) {
+  const auto kernel = wide ? (compact ? traceKernel<WideWalk, NEE, false, COUNT, true> : traceKernel<WideWalk, NEE, false, COUNT, false>)
+                           : (compact ? traceKernel<Bvh2Walk, NEE, ALPHA, COUNT, true> : traceKernel<Bvh2Walk, NEE, ALPHA, COUNT, false>);
+  rt::launch(ctx->st, traceGrid(ctx, n), kTraceBlock, kernel, ctx->ds, rays, n, useTMax, hits, compact, ctx->dCtr, ctx->dCounters,
+             static_cast<uint2*>(ctx->dSpill), tuning(ctx));
 }
 
-template <bool NEE, bool ALPHA, bool COUNT, bool WIDE>
-static void runTrace(yc_ctx* ctx, const YcRay* rays, uint32_t n, bool useTMax, YcHit* hits, CompactHit* compact) {
-  const auto kernel = WIDE ? (compact ? traceWideKernel<NEE, COUNT, true> : traceWideKernel<NEE, COUNT, false>)
-                           : (compact ? traceKernel<NEE, ALPHA, COUNT, true> : traceKernel<NEE, ALPHA, COUNT, false>);
-  kernel<<<traceGrid(ctx, n), kTraceBlock, 0, ctx->st.s>>>(ctx->ds, rays, n, useTMax, hits, compact, ctx->dCtr, ctx->dCounters,
-                                                          static_cast<uint2*>(ctx->dSpill), tuning(ctx));
-}
-#endif
-
-// Which walk a ray hook uses: the context's (YcOptions::traversal) unless the mode forces one; counting traces
-// default to the reference-order walk (their box / triangle counts define the roofline's algorithmic bytes).
+// Which walk a ray hook uses: walksWide's choice unless the mode forces one.
 static int traceUsesWide(yc_ctx* ctx, int mode, bool* wide) {
-  const bool count = (mode & YC_TRACE_COUNT) != 0;
-  *wide = (mode & YC_TRACE_WIDE) ? true : (mode & YC_TRACE_REFERENCE_ORDER) ? false : (ctx->wide && !count);
+  *wide = (mode & YC_TRACE_WIDE) ? true
+          : (mode & YC_TRACE_REFERENCE_ORDER) ? false
+                                              : walksWide(ctx, ctx->ds.hasAlpha != 0, (mode & YC_TRACE_COUNT) != 0);
   if (*wide && !ctx->ds.wideNodes) return fail(ctx, YC_ERR_STATE, "no wide BVH for this scene (alpha-tested materials, or traversal = reference order)");
   return YC_OK;
 }
@@ -1694,20 +1589,11 @@ static int traceUsesWide(yc_ctx* ctx, int mode, bool* wide) {
 static void dispatchTrace(yc_ctx* ctx, int mode, bool wide, const YcRay* rays, uint32_t n, YcHit* hits, CompactHit* compact) {
   const bool nee = (mode & 0xf) == YC_TRACE_ANY, count = (mode & YC_TRACE_COUNT) != 0, alpha = ctx->ds.hasAlpha != 0;
   const bool useTMax = (mode & YC_TRACE_USE_TMAX) != 0;
-#define YB_TR(N, A, C) runTrace<N, A, C, false>(ctx, rays, n, useTMax, hits, compact)
-#define YB_TW(N, C) runTrace<N, false, C, true>(ctx, rays, n, useTMax, hits, compact)
-  if (wide) {
-    if (nee) count ? YB_TW(true, true) : YB_TW(true, false);
-    else count ? YB_TW(false, true) : YB_TW(false, false);
-  } else if (nee) {
-    if (alpha) count ? YB_TR(true, true, true) : YB_TR(true, true, false);
-    else count ? YB_TR(true, false, true) : YB_TR(true, false, false);
-  } else {
-    if (alpha) count ? YB_TR(false, true, true) : YB_TR(false, true, false);
-    else count ? YB_TR(false, false, true) : YB_TR(false, false, false);
-  }
+#define YB_TR(N, A) \
+  (count ? runTrace<N, A, true>(ctx, wide, rays, n, useTMax, hits, compact) : runTrace<N, A, false>(ctx, wide, rays, n, useTMax, hits, compact))
+  if (nee) alpha ? YB_TR(true, true) : YB_TR(true, false);
+  else alpha ? YB_TR(false, true) : YB_TR(false, false);
 #undef YB_TR
-#undef YB_TW
 }
 
 extern "C" int yc_trace_device(yc_ctx* ctx, const void* raysDev, size_t n, int mode, void* hitsDev, int repeat, float* ms) {
