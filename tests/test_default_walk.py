@@ -1,7 +1,7 @@
 """The library's default render path, TRAVERSAL_AUTO, which runs the quantised 4-wide walk (csrc/wide_bvh.cuh) on every
 scene without alpha-tested materials, held to two references that do not depend on tolerances.
 
-Part A (frames): the CPU build of the same sources (tests/hostsim; sequential walk, no tail kernel) renders each scene
+Part A (frames): the CPU build of the same sources (tests/hostsim; serial kernels, tail included) renders each scene
 once under AUTO, and that frame is the reference.  The CUDA library must reproduce HDR, LDR and the three ray counts bit
 for bit in every configuration that changes how the work is cut: tail hand-over at every bounce or never, small
 wavefront capacities (many chunks per wave), the global-memory spill of the traversal stack, waves left in flight,

@@ -96,30 +96,59 @@ def test_rng_samplers_render_bit_exact(path):
     PC.check_render(path, exact=True)
 
 
-def test_small_wavefront_capacity_gives_same_image():
-    """Chunking (pixel blocks x sample groups) must not change a single bit."""
-    path = os.path.join(H.GOLDEN, "render_cornell_waves.npz")
-    g = PC.load(path)
+def render_waves(g, **ctx_opts):
+    """The golden's frame through one Context and yc_render_wave, in the golden's progressive waves: hdr, ldr, stats."""
     name, kw = PC.scene_from_golden(g)
     w, h, spp, first, mx, depth = (int(v) for v in g["settings"])
     cam = H.scene_camera(name, **kw)
-    sc = Y.Scene(H.scene_file(name, **kw))
     c = Y.make_camera(w, h, cam["focal"], cam["fnum"], cam["pos"], cam["target"], (0, 0, 0), cam["exposure"])
+    ctx = Y.Context(max_depth=depth, **ctx_opts)
+    ctx.upload_scene(Y.Scene(H.scene_file(name, **kw)))
+    ctx.set_camera(c)
+    ctx.begin_frame(w, h, spp, 64, (0, 0, 0), PC.TONEMAPS[str(g["tonemap"])])
+    taken, wave, waves = 0, first, 0
+    while wave > 0:
+        ctx.render_wave(taken, wave, taken)
+        taken += wave
+        nxt = min(wave * 2, mx) if (waves > 0 or wave > 1) else 1
+        wave = min(nxt, spp - taken)
+        waves += 1
+    hdr, ldr, st = ctx.resolve()
+    ctx.close()
+    return hdr, ldr, st
+
+
+def test_small_wavefront_capacity_gives_same_image():
+    """Chunking (pixel blocks x sample groups) must not change a single bit."""
+    g = PC.load(os.path.join(H.GOLDEN, "render_cornell_waves.npz"))
     for cap in (700, 5000):  # < pixels (pixel blocks, K = 1) and ≈ 2.6 x pixels (K = 2)
-        ctx = Y.Context(max_depth=depth, max_paths=cap)
-        ctx.upload_scene(sc)
-        ctx.set_camera(c)
-        ctx.begin_frame(w, h, spp, 64, (0, 0, 0), Y.TONEMAP_AGX)
-        taken, wave, waves = 0, first, 0
-        while wave > 0:
-            ctx.render_wave(taken, wave, taken)
-            taken += wave
-            nxt = min(wave * 2, mx) if (waves > 0 or wave > 1) else 1
-            wave = min(nxt, spp - taken)
-            waves += 1
-        hdr, ldr, st = ctx.resolve()
+        hdr, ldr, st = render_waves(g, max_paths=cap)
         assert H.bits_equal(hdr, g["hdr"]).all() and H.bits_equal(ldr, g["ldr"]).all()
         assert st.raysReference == int(g["rays"])
+
+
+# (golden, traversal, whether the frame is the golden's): the tail runs as tailKernel<false, Bvh2Walk>,
+# tailKernel<true, Bvh2Walk> (alpha-tested materials) and tailKernel<false, WideWalk>
+TAIL_CASES = [("render_cornell_waves.npz", Y.TRAVERSAL_REFERENCE_ORDER, True), ("render_zoo.npz", Y.TRAVERSAL_REFERENCE_ORDER, True),
+              ("render_mclaren_small.npz", Y.TRAVERSAL_WIDE, False)]
+
+
+@pytest.mark.parametrize("name,traversal,golden", TAIL_CASES, ids=[c[0] for c in TAIL_CASES])
+def test_tail_hand_over_gives_same_image(name, traversal, golden):
+    """The per-path tail kernel that finishes a chunk once few paths survive must not change a single bit: tail never
+    (-1), at the default threshold (0) and from the second bounce on (65536)."""
+    g = PC.load(os.path.join(H.GOLDEN, name))
+    out = {t: render_waves(g, traversal=traversal, tail_threshold=t) for t in (-1, 0, 65536)}
+    hdr, ldr, st = out[-1]
+    if golden:
+        assert H.bits_equal(hdr, g["hdr"]).all() and H.bits_equal(ldr, g["ldr"]).all()
+        assert st.raysReference == int(g["rays"])
+    for t in (0, 65536):
+        h, l, s = out[t]
+        assert H.bits_equal(h, hdr).all() and H.bits_equal(l, ldr).all(), f"tail_threshold {t}: frame differs"
+        assert (s.raysReference, s.raysExtend, s.raysShadow) == (st.raysReference, st.raysExtend, st.raysShadow)
+    # the tail ran: it replaces the six launches of every later bounce by one
+    assert out[65536][2].kernelLaunches < st.kernelLaunches
 
 
 def test_tile_shards_sum_to_the_full_frame():

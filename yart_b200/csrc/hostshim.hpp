@@ -22,6 +22,7 @@ static inline float4 make_float4(float x, float y, float z, float w) { return fl
 #define __global__
 #define __launch_bounds__(...)
 static const uint3 threadIdx = {0, 0, 0}, blockIdx = {0, 0, 0};
+static inline void __syncwarp() {}
 static inline unsigned long long atomicAdd(unsigned long long* p, unsigned long long v) {
   const unsigned long long old = *p;
   *p = old + v;

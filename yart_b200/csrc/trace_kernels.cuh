@@ -21,7 +21,9 @@
 //     through an out-of-line path; no local memory is used.
 // Node records are fetched as two 256-bit read-only loads, triangles as three 128-bit loads.
 // With WideWalk the set of boxes differs, the triangle arithmetic does not (wide_bvh.cuh's header).
-// The CPU build of the product sources has a serial counterpart with the same signature (first below).
+// The per-thread kernels (tail, naive integrator) share one launch shape, forEachThread: one item per thread on the
+// thread's own traversal stack.  The CPU build of the product sources has a serial counterpart of each with the same
+// signature (first below).
 #pragma once
 #include "integrator.cuh"
 
@@ -56,7 +58,28 @@ inline void tracePersistent(const DScene& sc, IO& io, uint32_t n, uint32_t*, uin
     io.store(j, st, didHit, smp);
   }
 }
+
+// One thread that takes the items in order.
+template <int BLOCK, class F>
+inline void forEachThread(uint32_t n, F&& body) {
+  HostStack hs;
+  for (uint32_t j = 0; j < n; j++) body(j, hs.ts);
+}
 #else
+// body(j, stack) for item j = this thread's index in a launch of BLOCK-thread CTAs, if j < n; the stack's
+// shared-memory part is this thread's column of two [entry][thread] arrays.
+template <int BLOCK, class F>
+__device__ __forceinline__ void forEachThread(uint32_t n, F&& body) {
+  __shared__ uint32_t shRef[kShStack * BLOCK];
+  __shared__ float shD[kShStack * BLOCK];
+  TravStack stack;
+  stack.shRef = shRef + threadIdx.x;
+  stack.shD = shD + threadIdx.x;
+  stack.stride = BLOCK;
+  const uint32_t j = blockIdx.x * BLOCK + threadIdx.x;
+  if (j < n) body(j, stack);
+}
+
 // Ray in the object space of scene node `node`: the chain of inverse transforms root → node, applied
 // in the recursion's order (ray-integrator.cpp:26-30).  The ancestor chain is a host-built table.
 __device__ __forceinline__ void nodeLocalRay(const DScene& sc, uint32_t node, int depth, V3& o, V3& d) {

@@ -122,9 +122,9 @@ struct TraceTuning {
 // add and one LDS.64 / STS.64; entry 0 holds a sentinel (kNoRef) written when a mesh is entered, so a
 // pop never tests for "empty": popping the sentinel yields kNoRef = "this mesh is walked".
 constexpr int kPsStack = kShStack + 1;
+constexpr int kSpillEntries = kMaxStack;         // global spill entries per thread (covers the smallest shared stack)
 #ifndef YB_HOSTSIM
 constexpr uint32_t kPsStride = kTraceBlock * 8;  // bytes between consecutive entries of one thread
-constexpr int kSpillEntries = kMaxStack;         // global spill entries per thread (covers the smallest shared stack)
 constexpr uint32_t kNoRef = 0xffffffffu;   // "no current node" (has the leaf bit: never stepped as inner)
 constexpr uint32_t kPopRef = 0xfffffffeu;  // "pop at the top of the next inner step" (leaf bit set as well)
 struct WarpStack {

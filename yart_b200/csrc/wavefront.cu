@@ -64,7 +64,7 @@ struct Lane {
   SurfState ss{};
   uint32_t *qA = nullptr, *qH = nullptr, *qN = nullptr, *ctr = nullptr;  // cur/next, hit, NEE queues; counters
   uint32_t* hCtr = nullptr;  // page-locked copy of the counters
-  void* spill = nullptr;     // traversal-stack spill area of the persistent kernels
+  void* spill = nullptr;     // traversal-stack spill area of the persistent kernels (unused by the CPU build's serial engine)
   rt::Event evCtr;
   uint32_t capacity = 0;
   // A finished chunk leaves the lane at once: its per-path tail (the few paths that survive many bounces) and its
@@ -456,17 +456,6 @@ __global__ void __launch_bounds__(kTraceBlock, YB_TRACE_MIN_BLOCKS) shadowKernel
   flushCounts<COUNT>(counters, cnt);
 }
 
-#ifdef YB_HOSTSIM
-template <bool ALPHA>
-static void runNaive(yc_ctx* ctx, Lane& L) {
-  HostStack hs;
-  TraceCounters cnt;
-  uint32_t rays = 0;
-  for (uint32_t j = 0; j < L.n; j++) naiveStage<ALPHA>(ctx->ds, L.w, L.ps, L.qA[j], hs.ts, cnt, rays);
-  ctx->dCounters->raysReference += rays;
-  ctx->dCounters->raysExtend += rays;
-}
-#else
 // Tail of a chunk: once only a few thousand paths survive, every further bounce of the wavefront is
 // bound by the latency of its slowest ray (launch after launch).  The tail kernel gives each surviving
 // path one thread that runs its remaining bounces to the end — extend → shade → shadow in the same
@@ -490,15 +479,8 @@ template <bool ALPHA, class Walk>
 __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w, PathState ps, ShadowQueue sq,
                                                          const uint32_t* queue, uint32_t n, uint32_t firstBounce,
                                                          Counters* counters, float4* Lout) {
-  __shared__ uint32_t shRef[kShStack * kTailBlock];
-  __shared__ float shD[kShStack * kTailBlock];
-  TravStack stack;
-  stack.shRef = shRef + threadIdx.x;
-  stack.shD = shD + threadIdx.x;
-  stack.stride = kTailBlock;
-  const uint32_t j = blockIdx.x * kTailBlock + threadIdx.x;
   uint32_t raysRef = 0, nExtend = 0, nShadow = 0;
-  if (j < n) {
+  forEachThread<kTailBlock>(n, [&](uint32_t j, TravStack& stack) {
     const uint32_t i = queue[j];
     TraceCounters cnt;
     for (uint32_t bounce = firstBounce; bounce < w.maxDepth; bounce++) {
@@ -518,7 +500,7 @@ __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w
       if (!(r & kShadeContinue)) break;
     }
     Lout[i] = ps.L[i];  // back into the chunk's radiance buffer, where the accumulate reads it
-  }
+  });
   __syncwarp();
   aggregatedCount(&counters->raysReference, raysRef);
   aggregatedCount(&counters->raysExtend, nExtend);
@@ -529,27 +511,20 @@ __global__ void __launch_bounds__(kTailBlock) tailKernel(DScene sc, WaveParams w
 template <bool ALPHA>
 __global__ void __launch_bounds__(kTailBlock) naiveKernel(DScene sc, WaveParams w, PathState ps, const uint32_t* queue, uint32_t n,
                                                           Counters* counters) {
-  __shared__ uint32_t shRef[kShStack * kTailBlock];
-  __shared__ float shD[kShStack * kTailBlock];
-  TravStack stack;
-  stack.shRef = shRef + threadIdx.x;
-  stack.shD = shD + threadIdx.x;
-  stack.stride = kTailBlock;
-  const uint32_t j = blockIdx.x * kTailBlock + threadIdx.x;
   uint32_t rays = 0;
-  if (j < n) {
+  forEachThread<kTailBlock>(n, [&](uint32_t j, TravStack& stack) {
     TraceCounters cnt;
     naiveStage<ALPHA>(sc, w, ps, queue[j], stack, cnt, rays);
-  }
+  });
   __syncwarp();
   aggregatedCount(&counters->raysReference, rays);
   aggregatedCount(&counters->raysExtend, rays);
 }
 template <bool ALPHA>
 static void runNaive(yc_ctx* ctx, Lane& L) {
-  naiveKernel<ALPHA><<<(L.n + kTailBlock - 1) / kTailBlock, kTailBlock, 0, L.st.s>>>(ctx->ds, L.w, L.ps, L.qA, L.n, ctx->dCounters);
+  rt::launch(L.st, int((L.n + kTailBlock - 1) / kTailBlock), kTailBlock, naiveKernel<ALPHA>, ctx->ds, L.w, L.ps, L.qA, L.n,
+             ctx->dCounters);
 }
-#endif
 
 static int traceGridMax(const yc_ctx* ctx) { return ctx->smCount * 8; }
 static TraceTuning tuning(const yc_ctx* ctx) {
@@ -854,11 +829,9 @@ static int ensureWaveStorage(yc_ctx* ctx) {
     void* hp = nullptr;
     YC_TRY(rt::hostAlloc(&hp, kCtrCount * sizeof(uint32_t)));
     L.hCtr = static_cast<uint32_t*>(hp);
-#ifndef YB_HOSTSIM
     uint2* sp = nullptr;
     YC_TRY(devAlloc(own, &sp, size_t(traceGridMax(ctx)) * kTraceBlock * kSpillEntries));
     L.spill = sp;
-#endif
   }
   ctx->dCtr = ctx->lanes[0].ctr;
   ctx->dSpill = ctx->lanes[0].spill;
@@ -868,7 +841,6 @@ static int ensureWaveStorage(yc_ctx* ctx) {
   return YC_OK;
 }
 
-#ifndef YB_HOSTSIM
 // The tail kernel's copies of the surviving paths' state (index-compatible with the lane's own arrays) and its private
 // queues: allocated when a chunk first leaves paths to a tail (renders of depth 1 never do).
 static int ensureTailStorage(yc_ctx* ctx, Lane& L) {
@@ -890,7 +862,6 @@ static int ensureTailStorage(yc_ctx* ctx, Lane& L) {
   YC_TRY(devAlloc(own, &L.tq, size_t(kTailCapacity)));
   return YC_OK;
 }
-#endif
 
 // ---------------------------------------------------------------------------------------
 // frame + waves
@@ -1113,26 +1084,21 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
   // The chunk on lane L is complete as far as the lane's stream is concerned (`tail`: up to a per-path tail that the
   // side stream runs on copies): hand it to the side stream and free the lane.
   auto retire = [&](Lane& L, int l, bool tail) {
-#ifndef YB_HOSTSIM
     if (tail) {
       rt::streamWaitEvent(L.st, L.evTail);  // the previous tail of this lane has let go of `ts` / `tq`
       rt::launchFor(L.st, L.n, TailGatherK{L.ps, L.ts, L.qA, L.tq});
       ctx->launches++;
     }
-#endif
     rt::eventRecord(L.st, L.evChunk);
     rt::streamWaitEvent(L.side, L.evChunk);
-#ifndef YB_HOSTSIM
     if (tail) {
-      const dim3 tg((L.n + kTailBlock - 1) / kTailBlock);
-      if (walksWide(ctx, ALPHA, false))  // the tail counts nothing: counting renders keep their wide tail
-        tailKernel<false, WideWalk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
-      else
-        tailKernel<ALPHA, Bvh2Walk><<<tg, kTailBlock, 0, L.side.s>>>(ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n, L.bounce, ctx->dCounters, L.ps.L);
+      // the tail counts nothing: counting renders keep their wide tail
+      const auto kernel = walksWide(ctx, ALPHA, false) ? tailKernel<false, WideWalk> : tailKernel<ALPHA, Bvh2Walk>;
+      rt::launch(L.side, int((L.n + kTailBlock - 1) / kTailBlock), kTailBlock, kernel, ctx->ds, L.w, L.ts, L.tsq, L.tq, L.n,
+                 L.bounce, ctx->dCounters, L.ps.L);
       rt::eventRecord(L.side, L.evTail);
       ctx->launches++;
     }
-#endif
     Finished& f = finished[L.chunk];
     f.valid = true, f.lane = l, f.buf = L.lSel;
     f.pixBase = L.w.pixBase, f.nPix = L.w.nPix, f.K = L.K, f.sDone = L.sDone, f.stride = L.w.sStrideM1 + 1u;
@@ -1224,13 +1190,11 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
       retire(L, wl, false);
       continue;
     }
-#ifndef YB_HOSTSIM
     if (L.n <= ctx->tailThreshold) {
       if (const int trc = ensureTailStorage(ctx, L)) return trc;
       retire(L, wl, true);
       continue;
     }
-#endif
     const int rc = issueBounce<ALPHA>(ctx, L);
     if (rc != YC_OK) return rc;
     if (L.done) retire(L, wl, false);
@@ -1879,9 +1843,9 @@ static int commSum(yc_ctx* ctx, void* buf, size_t count, int dtype, int root) {
 #else
       // the last arrival adds on its own stream; the contexts share a device (or peer access), so every pointer is valid here
       const int grid = int(std::min<size_t>((count + 255) / 256, size_t(ctx->smCount) * 8));
-      if (dtype == kCommF32) groupSumKernel<float><<<grid, 256, 0, ctx->st.s>>>(bufs, n, count, root);
-      else if (dtype == kCommI32) groupSumKernel<uint32_t><<<grid, 256, 0, ctx->st.s>>>(bufs, n, count, root);
-      else groupSumKernel<unsigned long long><<<grid, 256, 0, ctx->st.s>>>(bufs, n, count, root);
+      if (dtype == kCommF32) rt::launch(ctx->st, grid, 256, groupSumKernel<float>, bufs, n, count, root);
+      else if (dtype == kCommI32) rt::launch(ctx->st, grid, 256, groupSumKernel<uint32_t>, bufs, n, count, root);
+      else rt::launch(ctx->st, grid, 256, groupSumKernel<unsigned long long>, bufs, n, count, root);
       if (const char* se = rt::sync(ctx->st)) return se;
       return rt::lastError();
 #endif
