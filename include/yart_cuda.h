@@ -355,6 +355,33 @@ int yc_finalize_wave(yc_ctx* ctx, YcRect pixels, uint32_t waveSamples, uint32_t 
 /* Copies the frames to host (either pointer may be NULL).  width*height*4 floats each.
  * Replaces reading Renderer::m_buffer (RenderData::buffer, renderer.hpp:22-28). */
 int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
+/* First-hit AOVs: guide buffers for a denoiser, collected while the frame renders (no extra ray).
+ * For each pixel, over the S samples accumulated since yc_begin_frame: H of them are samples whose camera ray hit a
+ * surface at bounce 0 (hitB >= 0). These are the hits after alpha testing, i.e. the surface the integrator shades.
+ *   albedo RGBA:
+ *     rgb = Σ over hit samples of the evaluated base colour (MatEval::base: YcMaterial::base × base texture) / S;
+ *     a = H / S (coverage).
+ *   normalDepth RGBA:
+ *     xyz = Σ over hit samples of the world-space shading normal (SurfRecord::n, which equals YcHit::n; not flipped
+ *           toward the camera, not renormalised after averaging) / S;
+ *     w = Σ t over hit samples / H. Camera rays have unit direction (camera.cuh:51), so t is the distance from the
+ *         ray's lens origin.
+ * Misses contribute 0. Where S = 0 everything is 0, and where H = 0, w is 0. Exposure and background do not apply.
+ * Sums are float32, start at +0.0, and add one sample at a time. The order is call order, then sample order within a
+ * call, which is the order AccumulateK already uses. The final division is IEEE / (__fdiv_rn on the device). This makes
+ * the buffers reproducible by a numpy loop.
+ *
+ *   yc_enable_aovs     switches the collection on (or off) for the frames that follow: valid before yc_begin_frame or
+ *                      before the frame's first wave, YC_ERR_STATE later; YC_ERR_UNSUPPORTED with
+ *                      YC_INTEGRATOR_NAIVE.  The first enable allocates 32 bytes per path in flight (twice, per lane:
+ *                      512 MB at the default capacity) and four float4 and one uint32 per texel of the frame.
+ *                      yc_accumulate_wave with bucketShardCount > 1 returns YC_ERR_UNSUPPORTED while AOVs are on.
+ *   yc_resolve_aovs    copies both planes (width*height*4 floats each; either pointer may be NULL); YC_ERR_STATE
+ *                      when AOVs are not enabled.
+ *   yc_comm_reduce_aovs  tile sharding, collective: combines every participant's planes into the root's, out of place
+ *                      (repeated calls count nothing twice); yc_resolve_aovs_combined copies them out on the root. */
+int yc_enable_aovs(yc_ctx* ctx, int enable);
+int yc_resolve_aovs(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA);
 /* Device pointers of the frames (for NCCL reductions by the caller). */
 int yc_frame_device_ptrs(yc_ctx* ctx, void** hdr, void** ldr, size_t* bytes);
 /* Re-run the tonemap over the whole HDR frame (after a cross-GPU sum). */
@@ -424,6 +451,9 @@ int yc_comm_frames_direct(yc_ctx* ctx, int* direct);
 int yc_resolve_combined(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA);
 /* Bucket sharding (yc_accumulate_wave): all-reduce(sum, int32) of the planes a wave of `waveSamples` samples uses. */
 int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples);
+/* Tile sharding with AOVs (yc_enable_aovs): see there. */
+int yc_comm_reduce_aovs(yc_ctx* ctx, int root);
+int yc_resolve_aovs_combined(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA);
 /* Control values (ray counts, abort votes): in-place sum over all participants. */
 int yc_comm_sum_u64(yc_ctx* ctx, uint64_t* values, uint32_t n);
 /* The reference's binned-SAH BVH (src/core/bvh.hpp:140-184, 273-347) built on the device, level by level: the same
@@ -483,6 +513,10 @@ int ys_decode_texture(const void* png, size_t len, uint32_t type, uint32_t nChan
 int ys_load_hdr(const char* path, uint32_t* width, uint32_t* height, float* rgb, size_t rgbFloats);
 /* output::writePPM (src/output/ppm.cpp:6-21) on an RGBA float frame. */
 int ys_write_ppm(const char* path, const float* rgba, uint32_t width, uint32_t height);
+/* A float image as a Portable Float Map (what denoiser command-line tools read): `channels` 3 ("PF") or 1 ("Pf"), the
+ * first floats of each pixel of `strideFloats` floats (the depth of a normalDepth plane: data = plane + 3, stride 4,
+ * channels 1); little-endian (scale -1.0), rows bottom to top as the format requires. */
+int ys_write_pfm(const char* path, const float* data, uint32_t width, uint32_t height, uint32_t strideFloats, uint32_t channels);
 void ys_scene_destroy(ys_scene* s);
 const char* ys_last_error(void);
 /* Flattened view (valid until ys_scene_destroy). */
@@ -579,6 +613,13 @@ int yr_wait(yr_renderer* r);       /* Renderer::wait() */
 int yr_render_sync(yr_renderer* r, YrRenderData* out); /* Renderer::renderSync() */
 /* Result buffers: LDR (what Renderer::m_buffer holds) and HDR accumulation. */
 int yr_read(yr_renderer* r, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
+/* First-hit AOVs of the renders that follow (yc_enable_aovs; YC_ERR_UNSUPPORTED for the naive integrator and for
+ * YR_SHARD_BUCKETS over more than one participant, YC_ERR_STATE while a render runs). */
+int yr_enable_aovs(yr_renderer* r, int enable);
+/* The AOV planes of the last render (width*height*4 floats each, either pointer may be NULL), valid once it has returned
+ * (yr_render_sync / yr_wait) and YC_ERR_STATE while one runs.  Tile sharding: the combined planes, on the root; other
+ * ranks' buffers are left untouched, as with yr_read. */
+int yr_read_aovs(yr_renderer* r, float* albedoRGBA, float* normalDepthRGBA);
 /* writePPM(out, renderer buffer): the tonemapped frame as a binary PPM (frontend main.cpp writes out.ppm). */
 int yr_write_ppm(yr_renderer* r, const char* path);
 yc_ctx* yr_context(yr_renderer* r);

@@ -125,6 +125,19 @@ def write_ppm(path: str, rgba: np.ndarray):
     _check(lib().ys_write_ppm(path.encode(), rgba.ctypes.data, rgba.shape[1], rgba.shape[0]), "ys_write_ppm")
 
 
+def write_pfm(path: str, array: np.ndarray):
+    """ys_write_pfm: an (h, w, 3) or (h, w) float array as a Portable Float Map ("PF" / "Pf"), what denoiser tools read."""
+    a = np.ascontiguousarray(array, np.float32)
+    if a.ndim == 2:
+        channels = 1
+    elif a.ndim == 3 and a.shape[2] == 3:
+        channels = 3
+    else:
+        raise ValueError(f"write_pfm: expected (h, w) or (h, w, 3), got {a.shape}")
+    _check(lib().ys_write_pfm(path.encode(), a.ctypes.data, a.shape[1], a.shape[0], channels, channels), "ys_write_pfm",
+           lib().ys_last_error() or b"")
+
+
 class Scene:
     """yart::Scene built from a .ysc description or a binary glTF file (stands in for gltf::load)."""
 
@@ -279,7 +292,27 @@ class Context:
     def retonemap(self):
         self._ck(lib().yc_retonemap(self._h), "yc_retonemap")
 
+    def enable_aovs(self, enable: bool = True):
+        """yc_enable_aovs: first-hit albedo / normal / depth planes for the frames that follow (include/yart_cuda.h)."""
+        self._ck(lib().yc_enable_aovs(self._h, int(enable)), "yc_enable_aovs")
+
+    def resolve_aovs(self):
+        """(albedo RGBA, normalDepth RGBA) as two (h, w, 4) float32 arrays."""
+        h, w = self.frame.height, self.frame.width
+        albedo, nd = np.empty((h, w, 4), np.float32), np.empty((h, w, 4), np.float32)
+        self._ck(lib().yc_resolve_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yc_resolve_aovs")
+        return albedo, nd
+
     # ---- collectives (yc_comm_*) ----
+    def comm_reduce_aovs(self, root: int = 0):
+        self._ck(lib().yc_comm_reduce_aovs(self._h, root), "yc_comm_reduce_aovs")
+
+    def resolve_aovs_combined(self):
+        h, w = self.frame.height, self.frame.width
+        albedo, nd = np.empty((h, w, 4), np.float32), np.empty((h, w, 4), np.float32)
+        self._ck(lib().yc_resolve_aovs_combined(self._h, albedo.ctypes.data, nd.ctypes.data), "yc_resolve_aovs_combined")
+        return albedo, nd
+
     def comm_init_rank(self, rank: int, world: int, comm_id: bytes):
         cid = (C.c_char * capi.COMM_ID_BYTES).from_buffer_copy(bytes(comm_id))
         self._ck(lib().yc_comm_init_rank(self._h, rank, world, cid), "yc_comm_init_rank")
@@ -365,8 +398,9 @@ class Renderer:
                  first_wave_samples=None, max_wave_samples=None, tile_size=64, max_depth=30, background=(0, 0, 0),
                  tonemap=TONEMAP_AGX, estimator=ESTIMATOR_GMON, shard_index=0, shard_count=1, device=0,
                  integrator=capi.INTEGRATOR_MIS, scrambler=capi.SCRAMBLER_FAST_OWEN, sampler=capi.SAMPLER_SOBOL,
-                 traversal=None, sharding=capi.SHARD_TILES, devices=None, dist=None):
+                 traversal=None, sharding=capi.SHARD_TILES, devices=None, dist=None, aovs=False):
         """devices=[g0, g1, ...]: one renderer over several GPUs of this process (yr_create_multi).
+        aovs=True: collect the first-hit albedo / normal / depth planes (yr_enable_aovs; read_aovs()).
         dist=(rank, world, comm): one process per GPU (yr_create_dist); comm = the 128 bytes of comm_unique_id() from
         rank 0, or a callable collective(buf_ptr, count, dtype, root) → 0 (yr_create_dist_custom)."""
         traversal = default_traversal if traversal is None else traversal
@@ -395,6 +429,8 @@ class Renderer:
         else:
             rc, what = lib().yr_create(C.byref(s), sh, C.byref(camera), C.byref(self._h)), "yr_create"
         _check(rc, what, _NO_DEVICE if rc == capi.YC_ERR_NO_DEVICE else b"")
+        if aovs:
+            self.enable_aovs()
 
     def close(self):
         if self._h:
@@ -496,6 +532,18 @@ class Renderer:
         self._ck(lib().yr_read(self._h, hdr.ctypes.data if want_hdr else None, ldr.ctypes.data if want_ldr else None,
                                C.byref(st)), "yr_read")
         return hdr, ldr, st
+
+    def enable_aovs(self, enable: bool = True):
+        """yr_enable_aovs: first-hit albedo / normal / depth planes for the renders that follow (read_aovs())."""
+        self._ck(lib().yr_enable_aovs(self._h, int(enable)), "yr_enable_aovs")
+
+    def read_aovs(self) -> dict:
+        """The last render's first-hit AOVs: dict(albedo=(h, w, 3), coverage=(h, w), normal=(h, w, 3), depth=(h, w)),
+        float32 (tile sharding over ranks: the combined planes on rank 0; zeros elsewhere)."""
+        h, w = self.settings.height, self.settings.width
+        albedo, nd = np.zeros((h, w, 4), np.float32), np.zeros((h, w, 4), np.float32)
+        self._ck(lib().yr_read_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yr_read_aovs")
+        return dict(albedo=albedo[..., :3].copy(), coverage=albedo[..., 3].copy(), normal=nd[..., :3].copy(), depth=nd[..., 3].copy())
 
     def write_ppm(self, path: str):
         self._ck(lib().yr_write_ppm(self._h, path.encode()), "yr_write_ppm")

@@ -167,6 +167,10 @@ PROTOTYPES = {
     "yc_resolve_combined": (C.c_int, [P, P, P]),
     "yc_comm_allreduce_buckets": (C.c_int, [P, u32]),
     "yc_comm_sum_u64": (C.c_int, [P, C.POINTER(u64), u32]),
+    "yc_enable_aovs": (C.c_int, [P, C.c_int]),
+    "yc_resolve_aovs": (C.c_int, [P, P, P]),
+    "yc_comm_reduce_aovs": (C.c_int, [P, C.c_int]),
+    "yc_resolve_aovs_combined": (C.c_int, [P, P, P]),
     "yc_kat": (C.c_int, [P, C.c_char_p, P, C.c_size_t, P, C.c_size_t]),
     "ys_scene_load": (C.c_int, [C.c_char_p, C.POINTER(P)]),
     "ys_scene_load_bvh": (C.c_int, [C.c_char_p, u32, C.POINTER(P)]),
@@ -177,6 +181,7 @@ PROTOTYPES = {
     "ys_decode_texture": (C.c_int, [P, C.c_size_t, u32, u32, C.POINTER(i32), P, C.c_size_t, C.POINTER(u32), C.POINTER(u32)]),
     "ys_load_hdr": (C.c_int, [C.c_char_p, C.POINTER(u32), C.POINTER(u32), P, C.c_size_t]),
     "ys_write_ppm": (C.c_int, [C.c_char_p, P, u32, u32]),
+    "ys_write_pfm": (C.c_int, [C.c_char_p, P, u32, u32, u32, u32]),
     "ys_scene_destroy": (None, [P]),
     "ys_last_error": (C.c_char_p, []),
     "ys_scene_flat": (C.POINTER(YcScene), [P]),
@@ -204,6 +209,8 @@ PROTOTYPES = {
     "yr_render_sync": (C.c_int, [P, C.POINTER(YrRenderData)]),
     "yr_read": (C.c_int, [P, P, P, C.POINTER(YcStats)]),
     "yr_write_ppm": (C.c_int, [P, C.c_char_p]),
+    "yr_enable_aovs": (C.c_int, [P, C.c_int]),
+    "yr_read_aovs": (C.c_int, [P, P, P]),
     "yr_context": (P, [P]),
     "yr_last_error": (C.c_char_p, [P]),
 }

@@ -54,3 +54,4 @@ static inline float __uint_as_float(uint32_t u) {
   memcpy(&f, &u, 4);
   return f;
 }
+static inline float __fdiv_rn(float a, float b) { return a / b; }

@@ -75,6 +75,9 @@ struct Lane {
   ShadowQueue tsq{};
   uint32_t* tq = nullptr;
   float4* Lbuf[2] = {nullptr, nullptr};
+  // yc_enable_aovs: the first hit of every path of the chunk in Lbuf[b], 2 float4 per path {base.rgb, 1 (0: miss)},
+  // {n.xyz, t}; guarded by the same events as Lbuf[b]
+  float4* aov[2] = {nullptr, nullptr};
   int lSel = 0;
   bool accPending[2] = {false, false};  // Lbuf[b] holds a finished chunk whose accumulate is not launched yet
   rt::Event evChunk, evTail, evSide[2];  // end of the chunk's lane-stream work; tail buffers free; accumulate of Lbuf[b] done
@@ -109,6 +112,15 @@ struct yc_ctx {
   float4 *dHdr = nullptr, *dLdr = nullptr, *dBuckets = nullptr;
   size_t bucketCapacity = 0;  // pixels per bucket plane
   bool bucketsDirty = false;  // an accumulate was not (or only partly) followed by a finalize: the planes hold sums
+  bool frameRendered = false;  // a wave was issued since yc_begin_frame (AOVs cannot be switched from then on)
+
+  // first-hit AOVs (yc_enable_aovs), per texel of the frame: sums {Σ base.rgb, H (bits)} then {Σ n.xyz, Σ t} (two planes),
+  // sample counts S, the resolved planes {albedo, normalDepth} and the out-of-place planes of yc_comm_reduce_aovs
+  bool aovs = false;
+  size_t aovTexels = 0;
+  float4 *dAovSum = nullptr, *dAov = nullptr, *dAovComm = nullptr;
+  uint32_t* dAovCount = nullptr;
+  bool aovCombined = false;  // this context is the root of a completed yc_comm_reduce_aovs of the current frame
 
   // wavefront storage lives in the lanes; the ray hooks (yc_trace*) use lane 0's counters and spill area
   uint32_t* dCtr = nullptr;
@@ -386,6 +398,73 @@ struct RetonemapK {
   }
 };
 
+// ---- first-hit AOVs (yc_enable_aovs) ----
+// Bounce 0 of a chunk, after ResolveK: each hit's evaluated base colour and shading normal + t (SurfRecord r5 / r1) into
+// the record of its path.  The records were zeroed when the chunk started, so a path that missed reads as a miss.
+// Bounce 0 always runs on the wavefront: a chunk is handed to the tail kernel only after its first bounce.
+struct AovCaptureK {
+  SurfState ss;
+  const uint32_t* queue;
+  const uint32_t* ctr;
+  float4* rec;
+  YB_DEV void operator()(uint32_t j) const {
+    if (j >= ctr[kCtrHitCount]) return;
+    const size_t i = queue[j];
+    const float4 b = ss.r5[j];
+    rec[2 * i] = make_float4(b.x, b.y, b.z, 1.0f);
+    rec[2 * i + 1] = ss.r1[j];
+  }
+};
+
+// After the chunk's AccumulateK, in chunk order: pixel p adds its K samples in sample order (misses add nothing).
+struct AovAccumulateK {
+  const float4* rec;
+  const uint32_t* pixelList;
+  float4* sum;
+  uint32_t* count;
+  size_t texels;
+  uint32_t pixBase, nPix, K, width;
+  YB_DEV void operator()(uint32_t p) const {
+    const uint32_t pix = pixelList[pixBase + p];
+    const size_t idx = size_t(pix >> 16) * width + (pix & 0xffffu);
+    float4 a = sum[idx], b = sum[texels + idx];
+    uint32_t hits = __float_as_uint(a.w);
+    for (uint32_t k = 0; k < K; k++) {
+      const size_t i = size_t(k) * nPix + p;
+      const float4 c = rec[2 * i];
+      if (c.w == 0.0f) continue;
+      const float4 d = rec[2 * i + 1];
+      a.x += c.x, a.y += c.y, a.z += c.z;
+      b.x += d.x, b.y += d.y, b.z += d.z, b.w += d.w;
+      hits++;
+    }
+    a.w = __uint_as_float(hits);
+    sum[idx] = a, sum[texels + idx] = b;
+    count[idx] += K;
+  }
+};
+
+// The two planes of include/yart_cuda.h's AOV definition, per texel: albedo {Σ base / S, H / S}, normalDepth
+// {Σ n / S, Σ t / H}; zero where S = 0 (and w where H = 0).
+struct AovResolveK {
+  const float4* sum;
+  const uint32_t* count;
+  float4 *albedo, *normalDepth;
+  size_t texels;
+  YB_DEV void operator()(uint32_t idx) const {
+    const uint32_t S = count[idx];
+    float4 al = make_float4(0.0f, 0.0f, 0.0f, 0.0f), nd = al;
+    if (S) {
+      const float4 a = sum[idx], b = sum[texels + idx];
+      const uint32_t H = __float_as_uint(a.w);
+      const float s = float(S);
+      al = make_float4(__fdiv_rn(a.x, s), __fdiv_rn(a.y, s), __fdiv_rn(a.z, s), __fdiv_rn(float(H), s));
+      nd = make_float4(__fdiv_rn(b.x, s), __fdiv_rn(b.y, s), __fdiv_rn(b.z, s), H ? __fdiv_rn(b.w, float(H)) : 0.0f);
+    }
+    albedo[idx] = al, normalDepth[idx] = nd;
+  }
+};
+
 // Which BVH layout a traversal launch walks: the wide one when the context built it (YcOptions::traversal, scenes
 // without alpha-tested materials), unless the launch draws alpha-test samples or counts box / triangle tests (the counts
 // of the reference-order walk define the roofline's algorithmic bytes).  Kernels are picked as
@@ -637,6 +716,16 @@ static void freeFrame(yc_ctx* ctx) {
   ctx->inFrame = false;
 }
 
+static void freeAovPlanes(yc_ctx* ctx) {
+  for (void* p : {static_cast<void*>(ctx->dAovSum), static_cast<void*>(ctx->dAov), static_cast<void*>(ctx->dAovComm),
+                  static_cast<void*>(ctx->dAovCount)})
+    rt::release(p);
+  ctx->dAovSum = ctx->dAov = ctx->dAovComm = nullptr;
+  ctx->dAovCount = nullptr;
+  ctx->aovTexels = 0;
+  ctx->aovCombined = false;
+}
+
 static void destroyComm(yc_ctx* ctx);
 static void detachCombinedFrames(yc_ctx* ctx);
 
@@ -646,6 +735,7 @@ extern "C" void yc_destroy(yc_ctx* ctx) {
   rt::sync(ctx->st);
   destroyComm(ctx);
   freeFrame(ctx);
+  freeAovPlanes(ctx);
   freeAll(ctx->sceneAllocs);
   freeAll(ctx->waveAllocs);
   rt::eventDestroy(ctx->ev0);
@@ -883,6 +973,52 @@ static uint32_t roundUpPow2(uint32_t v) {  // math_base.hpp:164-170
   return p;
 }
 
+// The AOV sums of the frame `ctx->frame` describes, allocated for its size and cleared.
+static int prepareAovPlanes(yc_ctx* ctx) {
+  const size_t texels = size_t(ctx->frame.width) * ctx->frame.height;
+  if (ctx->aovTexels != texels) {
+    freeAovPlanes(ctx);
+    const char* e = nullptr;
+    void* p = nullptr;
+    if (!e && !(e = rt::alloc(&p, 2 * texels * sizeof(float4)))) ctx->dAovSum = static_cast<float4*>(p);
+    if (!e && !(e = rt::alloc(&p, 2 * texels * sizeof(float4)))) ctx->dAov = static_cast<float4*>(p);
+    if (!e && !(e = rt::alloc(&p, texels * sizeof(uint32_t)))) ctx->dAovCount = static_cast<uint32_t*>(p);
+    if (e) {
+      freeAovPlanes(ctx);
+      return fail(ctx, YC_ERR_CUDA, "AOV planes: %s", e);
+    }
+    ctx->aovTexels = texels;
+  }
+  YC_TRY(rt::zero(ctx->st, ctx->dAovSum, 2 * texels * sizeof(float4)));
+  YC_TRY(rt::zero(ctx->st, ctx->dAovCount, texels * sizeof(uint32_t)));
+  ctx->aovCombined = false;
+  return YC_OK;
+}
+
+extern "C" int yc_enable_aovs(yc_ctx* ctx, int enable) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (ctx->frameRendered) return fail(ctx, YC_ERR_STATE, "yc_enable_aovs inside a frame (after its first wave)");
+  if (!enable) {
+    ctx->aovs = false;
+    return YC_OK;
+  }
+  if (ctx->opts.integrator == YC_INTEGRATOR_NAIVE)
+    return fail(ctx, YC_ERR_UNSUPPORTED, "yc_enable_aovs: the naive integrator runs whole paths in one kernel");
+  if (int rc = ensureWaveStorage(ctx)) return rc;
+  for (int l = 0; l < kLanes; l++) {
+    Lane& L = ctx->lanes[l];
+    for (int b = 0; b < 2; b++)
+      if (!L.aov[b]) YC_TRY(devAlloc(ctx->waveAllocs, &L.aov[b], 2 * size_t(L.capacity)));
+  }
+  if (ctx->inFrame) {
+    if (int rc = prepareAovPlanes(ctx)) return rc;
+    YC_TRY(rt::sync(ctx->st));
+  }
+  ctx->aovs = true;
+  return YC_OK;
+}
+
 extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   if (!ctx || !f) return YC_ERR_INVALID;
   YC_ENTER(ctx);
@@ -938,6 +1074,9 @@ extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   }
   ctx->frame = *f;
   ctx->frame.shardCount = shardCount;
+  ctx->frameRendered = false;
+  if (ctx->aovs)
+    if (const int arc = prepareAovPlanes(ctx)) return arc;
   // finalize leaves every bucket it reads zeroed, so the planes only need clearing when an accumulate was not
   // followed by its finalize (an error or abort mid-wave, a partial-rectangle finalize) or when they are new
   if (ctx->bucketsDirty) {
@@ -979,6 +1118,10 @@ static int issueBounce(yc_ctx* ctx, Lane& L) {
   rt::launchFor<YB_SAMPLE_MIN_BLOCKS>(L.st, n, SampleK<ALPHA>{ctx->ds, L.w, L.ps, L.ss, L.qH, L.qA, L.qN, L.ctr, ctx->dCounters});
   rt::launchFor<YB_NEE_MIN_BLOCKS>(L.st, n, ShadeNeeK{ctx->ds, L.w, L.ss, L.sq, L.qH, L.qN, L.ctr});
   if (sev) rt::eventRecord(L.st, sev->second);
+  if (ctx->aovs && L.bounce == 0) {  // (the records SurfState slots r1 / r5 hold stay until the next bounce's ResolveK)
+    rt::launchFor(L.st, n, AovCaptureK{L.ss, L.qH, L.ctr, L.aov[L.lSel]});
+    ctx->launches++;
+  }
   if (ctx->countTraversal) runShadow<ALPHA, true>(ctx, L, n);
   else runShadow<ALPHA, false>(ctx, L, n);
   ctx->launches += 6;
@@ -1129,6 +1272,7 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
       rt::streamWaitEvent(L.st, L.evSide[L.lSel]);  // the accumulate that read this buffer last
       rt::launchFor(L.st, L.n, RaygenK{L.w, L.ps, L.qA});
       ctx->launches++;
+      if (ctx->aovs) YC_TRY(rt::zero(L.st, L.aov[L.lSel], 2 * size_t(L.n) * sizeof(float4)));  // every path a miss until AovCaptureK
       if (ctx->opts.integrator == YC_INTEGRATOR_NAIVE) {
         runNaive<ALPHA>(ctx, L);  // the whole path in one launch: nothing to wait for
         ctx->launches++;
@@ -1151,6 +1295,11 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
       rt::launchFor(L.side, f.nPix,
                     AccumulateK{acc, ctx->dBuckets, ctx->bucketCapacity, f.pixBase, f.nPix, f.K, f.sDone, f.stride, m, ctx->frame.estimator,
                                 exposureScale});
+      if (ctx->aovs) {
+        rt::launchFor(L.side, f.nPix, AovAccumulateK{L.aov[f.buf], dList, ctx->dAovSum, ctx->dAovCount, ctx->aovTexels, f.pixBase, f.nPix,
+                                                     f.K, ctx->frame.width});
+        ctx->launches++;
+      }
       rt::eventRecord(L.side, L.evSide[f.buf]);
       lastAcc = &L.evSide[f.buf];
       L.accPending[f.buf] = false;
@@ -1190,6 +1339,7 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
       retire(L, wl, false);
       continue;
     }
+    // the tail takes over after the first bounce at the earliest: bounce 0, where AovCaptureK runs, is always a wavefront one
     if (L.n <= ctx->tailThreshold) {
       if (const int trc = ensureTailStorage(ctx, L)) return trc;
       retire(L, wl, true);
@@ -1302,6 +1452,7 @@ static void noteWave(yc_ctx* ctx, YcRect px) {
 // flight (ctx->wavesPending) and leaves this one in flight.
 static int issueWave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset, uint32_t waveSamples, uint32_t takenBefore) {
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_render_wave before yc_begin_frame");
+  ctx->frameRendered = true;
   noteWave(ctx, px);
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
@@ -1346,6 +1497,9 @@ extern "C" int yc_accumulate_wave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset,
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_accumulate_wave before yc_begin_frame");
   if (bucketShardCount == 0 || bucketShard >= bucketShardCount) return fail(ctx, YC_ERR_INVALID, "bucket shard out of range");
+  // a pixel's samples would be split over the participants, and its AOV sums would lose their order
+  if (ctx->aovs && bucketShardCount > 1) return fail(ctx, YC_ERR_UNSUPPORTED, "AOVs with bucket sharding");
+  ctx->frameRendered = true;
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
   uint32_t nPixCall;
@@ -1418,6 +1572,25 @@ extern "C" int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* 
   if (hdrRGBA) YC_TRY(rt::d2h(ctx->st, hdrRGBA, ctx->dHdr, bytes));
   if (ldrRGBA) YC_TRY(rt::d2h(ctx->st, ldrRGBA, ctx->dLdr, bytes));
   return readStats(ctx, stats);
+}
+
+// AovResolveK over the whole frame into `albedo` / `normalDepth` (texel planes of the frame's size), on the main stream.
+static void resolveAovs(yc_ctx* ctx, float4* albedo, float4* normalDepth) {
+  rt::launchFor(ctx->st, uint32_t(ctx->aovTexels), AovResolveK{ctx->dAovSum, ctx->dAovCount, albedo, normalDepth, ctx->aovTexels});
+  ctx->launches++;
+}
+
+extern "C" int yc_resolve_aovs(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->aovs || !ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_resolve_aovs: AOVs are not enabled for this frame");
+  const size_t n = ctx->aovTexels;
+  resolveAovs(ctx, ctx->dAov, ctx->dAov + n);
+  if (albedoRGBA) YC_TRY(rt::d2h(ctx->st, albedoRGBA, ctx->dAov, n * sizeof(float4)));
+  if (normalDepthRGBA) YC_TRY(rt::d2h(ctx->st, normalDepthRGBA, ctx->dAov + n, n * sizeof(float4)));
+  YC_TRY(rt::sync(ctx->st));
+  YC_TRY(rt::lastError());
+  return YC_OK;
 }
 
 extern "C" int yc_frame_device_ptrs(yc_ctx* ctx, void** hdr, void** ldr, size_t* bytes) {
@@ -2086,6 +2259,38 @@ extern "C" int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples) {
   YC_TRY(rt::sync(ctx->st));
   YC_TRY(rt::lastError());
   ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
+  return YC_OK;
+}
+
+// Tile sharding: every participant resolves its planes (zero outside its tiles) into a buffer of its own and the buffers
+// are summed into the root's as 32-bit integers — each texel is non-zero on one participant only, so the integer sum
+// keeps every bit pattern, -0.0 included.  Out of place: the sums keep accumulating and repeated calls count nothing twice.
+extern "C" int yc_comm_reduce_aovs(yc_ctx* ctx, int root) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->comm) return fail(ctx, YC_ERR_STATE, "yc_comm_reduce_aovs without a communicator");
+  if (!ctx->aovs || !ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_comm_reduce_aovs: AOVs are not enabled for this frame");
+  if (root < 0 || root >= ctx->comm->world) return fail(ctx, YC_ERR_INVALID, "bad root");
+  const size_t n = ctx->aovTexels;
+  if (!ctx->dAovComm) YC_TRY(rt::alloc(reinterpret_cast<void**>(&ctx->dAovComm), 2 * n * sizeof(float4)));
+  rt::eventRecord(ctx->st, ctx->ev0);
+  resolveAovs(ctx, ctx->dAovComm, ctx->dAovComm + n);
+  if (const int rc = commSum(ctx, ctx->dAovComm, 2 * n * 4, kCommI32, root)) return rc;
+  rt::eventRecord(ctx->st, ctx->ev1);
+  YC_TRY(rt::sync(ctx->st));
+  YC_TRY(rt::lastError());
+  ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
+  ctx->aovCombined = ctx->comm->rank == root;
+  return YC_OK;
+}
+
+extern "C" int yc_resolve_aovs_combined(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->aovCombined) return fail(ctx, YC_ERR_STATE, "yc_resolve_aovs_combined: not the root of a completed yc_comm_reduce_aovs");
+  const size_t n = ctx->aovTexels;
+  if (albedoRGBA) YC_TRY(rt::d2h(ctx->st, albedoRGBA, ctx->dAovComm, n * sizeof(float4)));
+  if (normalDepthRGBA) YC_TRY(rt::d2h(ctx->st, normalDepthRGBA, ctx->dAovComm + n, n * sizeof(float4)));
   return YC_OK;
 }
 

@@ -192,6 +192,34 @@ extern "C" int ys_write_ppm(const char* path, const float* rgba, uint32_t width,
   return writePpm(path, rgba, width, height) ? YC_OK : YC_ERR_IO;
 }
 
+// Portable Float Map: "PF" (RGB) or "Pf" (grey) header, negative scale = little-endian, rows from the bottom up.
+extern "C" int ys_write_pfm(const char* path, const float* data, uint32_t width, uint32_t height, uint32_t strideFloats,
+                            uint32_t channels) {
+  if (!path || !data || !width || !height || (channels != 1 && channels != 3) || strideFloats < channels) return YC_ERR_INVALID;
+  return guarded([&]() -> int {
+    FILE* f = fopen(path, "wb");
+    if (!f) {
+      g_ysError = std::string("cannot write ") + path;
+      return YC_ERR_IO;
+    }
+    bool ok = fprintf(f, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height) > 0;
+    std::vector<uint8_t> row(size_t(width) * channels * 4);
+    for (uint32_t y = height; ok && y-- > 0;) {
+      uint8_t* o = row.data();
+      for (uint32_t x = 0; x < width; x++)
+        for (uint32_t c = 0; c < channels; c++) {
+          uint32_t u;
+          memcpy(&u, data + (size_t(y) * width + x) * strideFloats + c, 4);
+          for (int k = 0; k < 4; k++) *o++ = uint8_t(u >> (8 * k));
+        }
+      ok = fwrite(row.data(), 1, row.size(), f) == row.size();
+    }
+    ok = (fclose(f) == 0) && ok;
+    if (!ok) g_ysError = std::string("cannot write ") + path;
+    return ok ? YC_OK : YC_ERR_IO;
+  });
+}
+
 extern "C" void ys_scene_destroy(ys_scene* s) { delete s; }
 extern "C" const YcScene* ys_scene_flat(const ys_scene* s) { return s ? &s->host.flat : nullptr; }
 extern "C" double ys_scene_build_ms(const ys_scene* s) { return s ? s->host.buildMs : 0.0; }
@@ -282,6 +310,8 @@ struct yr_renderer {
   std::mutex m;
   YrRenderData last{};
   int lastRc = YC_OK;
+  bool aovs = false;                // yr_enable_aovs
+  std::atomic<bool> running{false}; // a render is in progress (yr_render's worker, or yr_render_sync)
 };
 
 static int rfail(yr_renderer* r, int rc, const std::string& msg) {
@@ -499,7 +529,8 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
     // tile sharding: this shard renders the tiles with index % world == its rank; bucket sharding: every shard holds
     // the whole frame and takes its (bucket, pixel class) units of every wave
     f.shardIndex = buckets ? 0u : r->rank0 + uint32_t(i), f.shardCount = buckets ? 1u : r->world;
-    return yc_begin_frame(sh.ctx, &f);
+    if ((e = yc_begin_frame(sh.ctx, &f)) != YC_OK) return e;
+    return yc_enable_aovs(sh.ctx, r->aovs ? 1 : 0);
   });
   if (rc != YC_OK) return rfail(r, rc, r->err);
 
@@ -582,6 +613,12 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
     waveSamples = std::min<uint64_t>(next, remaining);
     wave++;
   }
+  if (r->aovs && r->comm) {
+    // tile sharding (bucket sharding refuses AOVs): the shards' planes into the root's, once per render — after an abort
+    // too, since the abort vote has brought every participant here
+    rc = onShards(r, [&](size_t i) { return yc_comm_reduce_aovs(r->shards[i].ctx, 0); });
+    if (rc != YC_OK) return rfail(r, rc, r->err);
+  }
   {
     std::lock_guard<std::mutex> lk(r->m);
     r->last = data;
@@ -595,7 +632,10 @@ extern "C" int yr_render_sync(yr_renderer* r, YrRenderData* out) {
   if (!r) return YC_ERR_INVALID;
   if (r->worker.joinable()) r->worker.join();
   r->stop = 0;
-  return r->lastRc = renderBlocking(r, out);
+  r->running = true;
+  r->lastRc = renderBlocking(r, out);
+  r->running = false;
+  return r->lastRc;
 }
 
 extern "C" int yr_render(yr_renderer* r) {
@@ -603,7 +643,11 @@ extern "C" int yr_render(yr_renderer* r) {
   r->stop = 1;  // Renderer::render aborts a render in progress first (tile-renderer.hpp:40-43)
   if (r->worker.joinable()) r->worker.join();
   r->stop = 0;
-  r->worker = std::thread([r] { r->lastRc = renderBlocking(r, nullptr); });
+  r->running = true;
+  r->worker = std::thread([r] {
+    r->lastRc = renderBlocking(r, nullptr);
+    r->running = false;
+  });
   return YC_OK;
 }
 
@@ -644,6 +688,31 @@ extern "C" int yr_read(yr_renderer* r, float* hdrRGBA, float* ldrRGBA, YcStats* 
     }
   }
   return YC_OK;
+}
+
+extern "C" int yr_enable_aovs(yr_renderer* r, int enable) {
+  if (!r) return YC_ERR_INVALID;
+  if (r->running) return rfail(r, YC_ERR_STATE, "yr_enable_aovs while a render runs");
+  if (enable && r->s.integrator == YC_INTEGRATOR_NAIVE)
+    return rfail(r, YC_ERR_UNSUPPORTED, "AOVs: the naive integrator runs whole paths in one kernel");
+  if (enable && r->comm && r->s.sharding == YR_SHARD_BUCKETS)
+    return rfail(r, YC_ERR_UNSUPPORTED, "AOVs with bucket sharding: a pixel's samples are split over the participants");
+  r->aovs = enable != 0;  // applied to the contexts by the next render's yc_begin_frame
+  return YC_OK;
+}
+
+extern "C" int yr_read_aovs(yr_renderer* r, float* albedoRGBA, float* normalDepthRGBA) {
+  if (!r) return YC_ERR_INVALID;
+  if (r->running) return rfail(r, YC_ERR_STATE, "yr_read_aovs while a render runs");
+  if (!r->aovs) return rfail(r, YC_ERR_STATE, "yr_read_aovs: AOVs are not enabled (yr_enable_aovs)");
+  yc_ctx* c0 = r->shards[0].ctx;
+  int rc = YC_OK;
+  if (r->comm && r->s.sharding == YR_SHARD_TILES) {
+    if (rootHere(r)) rc = yc_resolve_aovs_combined(c0, albedoRGBA, normalDepthRGBA);
+  } else {
+    rc = yc_resolve_aovs(c0, albedoRGBA, normalDepthRGBA);
+  }
+  return rc != YC_OK ? rfail(r, rc, yc_last_error(c0)) : YC_OK;
 }
 
 extern "C" const float* ys_lut_tables(size_t* count) {
