@@ -1,4 +1,5 @@
-// comm.cuh — combining per-GPU accumulation buffers (included by wavefront.cu after yc_ctx is defined).
+// comm.cuh — combining per-GPU accumulation buffers: the transports and the communicator state behind wavefront.cu's
+// yc_comm_* entry points.
 //
 // BASELINE.json north_star: "Work is partitioned across the 8 GPUs of one box by image tile or sample wave, with the
 // scene replicated per GPU.  Per-GPU radiance, median-of-means and GMoN accumulation buffers are combined with NCCL
@@ -6,14 +7,15 @@
 // m_bufferMutex (src/cpu/tile-renderer.hpp:205-239).
 //
 // Three transports behind the same yc_comm_* entry points:
-//   * NCCL (product build): libnccl.so.2 loaded with dlopen at the first yc_comm_* call — the library has no link-time
-//     dependency on it, and a process that already holds NCCL (PyTorch) shares that copy.  Collectives run on the
-//     context's own stream, so they order after the wave's kernels without a host round trip.
+//   * NCCL (product build; the CPU build has none): libnccl.so.2 loaded with dlopen at the first yc_comm_* call — the
+//     library has no link-time dependency on it, and a process that already holds NCCL (PyTorch) shares that copy.
+//     Collectives run on the context's own stream, so they order after the wave's kernels without a host round trip.
 //   * the caller's sum collective (yc_comm_init_custom): MPI, gloo, a test double.
 //   * an in-process group: the contexts of yc_comm_init_all meet at a barrier and the last one to arrive adds the
-//     buffers (a plain loop in the CPU build of the product sources, one kernel over the participants' device
-//     pointers in the CUDA build).  Used when two contexts of a communicator share a GPU — NCCL refuses that — so the
-//     multi-GPU renderer logic runs in the CPU test-suite and on a one-GPU box.
+//     buffers with one kernel over the participants' device pointers (groupSumKernel, which the CPU build of the
+//     product sources runs as one loop).  Used when two contexts of a communicator share a GPU — NCCL refuses that —
+//     and always in the CPU build, whose contexts share one address space; so the multi-GPU renderer logic runs in
+//     the CPU test-suite and on a one-GPU box.
 // Tile sharding needs no reduction at all where every participant can address the root GPU's memory (NVLink peer
 // access: the other devices of the process, or other processes through an exported allocation): the finalize kernel
 // stores every finished pixel into the root's combined frame as it produces it, and the per-wave collective shrinks to
@@ -29,16 +31,21 @@
 #include <thread>
 #include <unistd.h>
 
+#include "rt.cuh"
+
+struct ncclComm;  // what nccl.h's ncclComm_t points to: Comm holds one in both builds
+
+namespace yb {
+enum { kCommF32 = 0, kCommI32 = 1, kCommU64 = 2 };
+}  // namespace yb
+
+// NCCL behind six calls with the same signatures in both builds, returning nullptr or an error as rt.cuh's calls do.
+// The product build resolves the library at the first call; the CPU build has none and says so.
 #ifndef YB_HOSTSIM
 #include <dlfcn.h>
 #include <nccl.h>
-#endif
 
 namespace yb {
-
-enum { kCommF32 = 0, kCommI32 = 1, kCommU64 = 2 };
-
-#ifndef YB_HOSTSIM
 // The handful of NCCL entry points used, resolved once from libnccl.so.2.
 struct NcclApi {
   ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
@@ -77,14 +84,53 @@ inline NcclApi& nccl() {
   return api;
 }
 static_assert(sizeof(ncclUniqueId) == YC_COMM_ID_BYTES, "YC_COMM_ID_BYTES must match ncclUniqueId");
+
+inline const char* ncclErrstr(ncclResult_t r) { return r == ncclSuccess ? nullptr : nccl().GetErrorString(r); }
+// Why NCCL cannot be used (nullptr: it can).  The other calls assume it can.
+inline const char* ncclUnavailable() { return nccl().ok ? nullptr : nccl().error.c_str(); }
+inline const char* ncclNewId(void* id128) {
+  ncclUniqueId id;
+  if (const char* e = ncclErrstr(nccl().GetUniqueId(&id))) return e;
+  memcpy(id128, &id, sizeof id);
+  return nullptr;
+}
+inline const char* ncclJoin(ncclComm** comm, int rank, int world, const void* id128) {
+  ncclUniqueId id;
+  memcpy(&id, id128, sizeof id);
+  return ncclErrstr(nccl().CommInitRank(comm, world, id, rank));
+}
+inline const char* ncclJoinAll(ncclComm** comms, int n, const int* devices) {
+  return ncclErrstr(nccl().CommInitAll(comms, n, devices));
+}
+inline void ncclRelease(ncclComm* comm) {
+  if (comm) nccl().CommDestroy(comm);
+}
+// In place on `st`: into every participant (root < 0, AllReduce) or into `root` only (Reduce).
+inline const char* ncclStreamSum(ncclComm* comm, void* buf, size_t count, int dtype, int root, rt::Stream& st) {
+  const ncclDataType_t t = dtype == kCommF32 ? ncclFloat32 : dtype == kCommI32 ? ncclInt32 : ncclUint64;
+  if (root < 0) return ncclErrstr(nccl().AllReduce(buf, buf, count, t, ncclSum, comm, st.s));
+  return ncclErrstr(nccl().Reduce(buf, buf, count, t, ncclSum, root, comm, st.s));
+}
+}  // namespace yb
+#else
+namespace yb {
+inline const char* ncclUnavailable() { return "the CPU build has no NCCL: use yc_comm_init_custom or yc_comm_init_all"; }
+inline const char* ncclNewId(void*) { return ncclUnavailable(); }
+inline const char* ncclJoin(ncclComm**, int, int, const void*) { return ncclUnavailable(); }
+inline const char* ncclJoinAll(ncclComm**, int, const int*) { return ncclUnavailable(); }
+inline void ncclRelease(ncclComm*) {}
+inline const char* ncclStreamSum(ncclComm*, void*, size_t, int, int, rt::Stream&) { return ncclUnavailable(); }
+}  // namespace yb
 #endif
+
+namespace yb {
 
 // In-process group: n participants, each on its own thread, meet per collective.
 constexpr int kGroupMax = 16;
 struct GroupPtrs {
   void* p[kGroupMax];
 };
-#ifndef YB_HOSTSIM
+// The last arrival's add.  One launch covers `count` in both builds: grid-stride on the GPU, one thread on the CPU.
 template <typename T>
 __global__ void groupSumKernel(GroupPtrs bufs, int n, size_t count, int root) {
   for (size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < count; i += size_t(gridDim.x) * blockDim.x) {
@@ -94,7 +140,6 @@ __global__ void groupSumKernel(GroupPtrs bufs, int n, size_t count, int root) {
       if (root < 0 || r == root) static_cast<T*>(bufs.p[r])[i] = total;
   }
 }
-#endif
 struct HostGroup {
   std::mutex m;
   std::condition_variable cv;
@@ -120,20 +165,9 @@ struct HostGroup {
     return error;
   }
 };
-template <typename T>
-inline void hostSum(const GroupPtrs& bufs, int n, size_t count, int root) {
-  std::vector<T> total(count, T(0));
-  for (int r = 0; r < n; r++)
-    for (size_t i = 0; i < count; i++) total[i] += static_cast<const T*>(bufs.p[r])[i];
-  for (int r = 0; r < n; r++)
-    if (root < 0 || r == root) memcpy(bufs.p[r], total.data(), count * sizeof(T));
-}
-
 struct Comm {
   int rank = 0, world = 1;
-#ifndef YB_HOSTSIM
-  ncclComm_t nccl = nullptr;
-#endif
+  ncclComm* nccl = nullptr;
   yc_collective_fn custom = nullptr;
   void* customUser = nullptr;
   std::shared_ptr<HostGroup> group;

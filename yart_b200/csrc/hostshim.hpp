@@ -21,7 +21,7 @@ static inline float4 make_float4(float x, float y, float z, float w) { return fl
 // A kernel is a plain function that rt::launch calls once: one thread of one block runs the whole launch.
 #define __global__
 #define __launch_bounds__(...)
-static const uint3 threadIdx = {0, 0, 0}, blockIdx = {0, 0, 0};
+static const uint3 threadIdx = {0, 0, 0}, blockIdx = {0, 0, 0}, blockDim = {1, 1, 1}, gridDim = {1, 1, 1};
 static inline void __syncwarp() {}
 static inline unsigned long long atomicAdd(unsigned long long* p, unsigned long long v) {
   const unsigned long long old = *p;

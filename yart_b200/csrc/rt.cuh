@@ -62,6 +62,7 @@ inline const char* d2hAsync(Stream&, void* d, const void* s, size_t n) {
 inline float eventElapsedMs(Event& a, Event& b) { return std::chrono::duration<float, std::milli>(b.t - a.t).count(); }
 inline const char* lastError() { return nullptr; }
 // peer memory: the CPU build's "devices" are one address space, and there is nothing to map across processes
+constexpr bool kOneAddressSpace = true;
 constexpr size_t kIpcHandleBytes = 64;
 inline const char* ipcExport(void*, void* handle) {
   memset(handle, 0, kIpcHandleBytes);
@@ -161,6 +162,7 @@ inline const char* lastError() { return errstr(cudaGetLastError()); }
 // Peer memory (comm.cuh: finished pixels are stored straight into the root GPU's frame over NVLink).  A cudaMalloc
 // block is exported as an opaque handle, imported by another PROCESS (mapping enables peer access), or — for another
 // device of the same process — reached through plain peer access.
+constexpr bool kOneAddressSpace = false;  // every device has memory of its own
 constexpr size_t kIpcHandleBytes = sizeof(cudaIpcMemHandle_t);
 inline const char* ipcExport(void* p, void* handle) {
   return errstr(cudaIpcGetMemHandle(static_cast<cudaIpcMemHandle_t*>(handle), p));

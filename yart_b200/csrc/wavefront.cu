@@ -1880,110 +1880,83 @@ extern "C" int yc_set_abort_flag(yc_ctx* ctx, const volatile int32_t* flag) {
 static void destroyComm(yc_ctx* ctx) {
   if (!ctx->comm) return;
   Comm& c = *ctx->comm;
-#ifndef YB_HOSTSIM
-  if (c.nccl) nccl().CommDestroy(c.nccl);
-#endif
+  ncclRelease(c.nccl);
   detachCombinedFrames(ctx);
   rt::release(c.scratch);
   ctx->comm.reset();
 }
 
-#ifndef YB_HOSTSIM
-#define YC_NCCL(expr)                                                                    \
-  do {                                                                                   \
-    const ncclResult_t r_ = (expr);                                                      \
-    if (r_ != ncclSuccess) return fail(ctx, YC_ERR_CUDA, "%s: %s", #expr, nccl().GetErrorString(r_)); \
-  } while (0)
-#endif
+// Replaces the context's communicator by a new one without a transport.  Waves still in flight are settled first: a
+// pending finalize kernel may still be storing into the old communicator's combined frames.
+static int attachComm(yc_ctx* ctx, int rank, int world) {
+  YC_ENTER(ctx);
+  destroyComm(ctx);
+  ctx->comm = std::make_unique<Comm>();
+  ctx->comm->rank = rank, ctx->comm->world = world;
+  return YC_OK;
+}
 
 extern "C" int yc_comm_unique_id(void* id128) {
   if (!id128) return YC_ERR_INVALID;
-#ifdef YB_HOSTSIM
-  return YC_ERR_UNSUPPORTED;
-#else
-  if (!nccl().ok) {
-    fprintf(stderr, "yart_b200: %s\n", nccl().error.c_str());
+  if (const char* e = ncclUnavailable()) {
+    fprintf(stderr, "yart_b200: %s\n", e);
     return YC_ERR_UNSUPPORTED;
   }
-  ncclUniqueId id;
-  if (nccl().GetUniqueId(&id) != ncclSuccess) return YC_ERR_CUDA;
-  memcpy(id128, &id, sizeof id);
-  return YC_OK;
-#endif
+  return ncclNewId(id128) ? YC_ERR_CUDA : YC_OK;
 }
 
 extern "C" int yc_comm_init_rank(yc_ctx* ctx, int rank, int world, const void* id128) {
   if (!ctx || !id128 || world < 1 || rank < 0 || rank >= world) return YC_ERR_INVALID;
-  YC_ENTER(ctx);
-#ifdef YB_HOSTSIM
-  return fail(ctx, YC_ERR_UNSUPPORTED, "the CPU build has no NCCL: use yc_comm_init_custom or yc_comm_init_all");
-#else
-  if (!nccl().ok) return fail(ctx, YC_ERR_UNSUPPORTED, "%s", nccl().error.c_str());
-  destroyComm(ctx);
-  ctx->comm = std::make_unique<Comm>();
-  ctx->comm->rank = rank, ctx->comm->world = world;
-  ncclUniqueId id;
-  memcpy(&id, id128, sizeof id);
-  YC_NCCL(nccl().CommInitRank(&ctx->comm->nccl, world, id, rank));
+  if (const char* e = ncclUnavailable()) return fail(ctx, YC_ERR_UNSUPPORTED, "%s", e);
+  if (const int rc = attachComm(ctx, rank, world)) return rc;
+  if (const char* e = ncclJoin(&ctx->comm->nccl, rank, world, id128)) return fail(ctx, YC_ERR_CUDA, "ncclCommInitRank: %s", e);
   return YC_OK;
-#endif
 }
 
 extern "C" int yc_comm_init_all(yc_ctx** ctxs, int n) {
   if (!ctxs || n < 1) return YC_ERR_INVALID;
   for (int i = 0; i < n; i++)
     if (!ctxs[i]) return YC_ERR_INVALID;
-  if (n > 1) {
-    bool shared = false;  // two contexts on one GPU: NCCL refuses duplicate devices
+  bool shared = rt::kOneAddressSpace;  // two contexts on one GPU: NCCL refuses duplicate devices
+  for (int i = 0; i < n; i++)
+    for (int j = i + 1; j < n; j++) shared |= ctxs[i]->device == ctxs[j]->device;
+  if (shared) {
+    if (n > kGroupMax) return fail(ctxs[0], YC_ERR_INVALID, "at most %d contexts in an in-process group", kGroupMax);
+    // the group's sums read every participant's buffer from one device: distinct devices need peer access
     for (int i = 0; i < n; i++)
-      for (int j = i + 1; j < n; j++) shared |= ctxs[i]->device == ctxs[j]->device;
-#ifdef YB_HOSTSIM
-    shared = true;  // the CPU build has no devices at all
-#endif
-    if (shared) {
-      if (n > kGroupMax) return fail(ctxs[0], YC_ERR_INVALID, "at most %d contexts in an in-process group", kGroupMax);
-      // the group's sums read every participant's buffer from one device: distinct devices need peer access
-      for (int i = 0; i < n; i++)
-        for (int j = 0; j < n; j++) {
-          rt::useDevice(ctxs[i]->device);
-          if (const char* e = rt::enablePeer(ctxs[i]->device, ctxs[j]->device))
-            return fail(ctxs[0], YC_ERR_UNSUPPORTED, "in-process group over devices %d and %d: %s", ctxs[i]->device, ctxs[j]->device, e);
-        }
-      auto group = std::make_shared<HostGroup>();
-      group->n = n;
-      for (int i = 0; i < n; i++) {
-        destroyComm(ctxs[i]);
-        ctxs[i]->comm = std::make_unique<Comm>();
-        ctxs[i]->comm->rank = i, ctxs[i]->comm->world = n, ctxs[i]->comm->group = group;
+      for (int j = 0; j < n; j++) {
+        rt::useDevice(ctxs[i]->device);
+        if (const char* e = rt::enablePeer(ctxs[i]->device, ctxs[j]->device))
+          return fail(ctxs[0], YC_ERR_UNSUPPORTED, "in-process group over devices %d and %d: %s", ctxs[i]->device, ctxs[j]->device, e);
       }
-      return YC_OK;
+    auto group = std::make_shared<HostGroup>();
+    group->n = n;
+    for (int i = 0; i < n; i++) {
+      if (const int rc = attachComm(ctxs[i], i, n)) return rc;
+      ctxs[i]->comm->group = group;
     }
+    return YC_OK;
   }
-#ifdef YB_HOSTSIM
-  destroyComm(ctxs[0]);
-  ctxs[0]->comm = std::make_unique<Comm>();
-  return YC_OK;
-#else
   yc_ctx* ctx = ctxs[0];
-  if (!nccl().ok) return fail(ctx, YC_ERR_UNSUPPORTED, "%s", nccl().error.c_str());
+  if (const char* e = ncclUnavailable()) return fail(ctx, YC_ERR_UNSUPPORTED, "%s", e);
   std::vector<int> devs;
-  std::vector<ncclComm_t> comms(size_t(n), nullptr);
+  std::vector<ncclComm*> comms(size_t(n), nullptr);
   for (int i = 0; i < n; i++) devs.push_back(ctxs[i]->device);
-  YC_NCCL(nccl().CommInitAll(comms.data(), n, devs.data()));
+  if (const char* e = ncclJoinAll(comms.data(), n, devs.data())) return fail(ctx, YC_ERR_CUDA, "ncclCommInitAll: %s", e);
   for (int i = 0; i < n; i++) {
-    destroyComm(ctxs[i]);
-    ctxs[i]->comm = std::make_unique<Comm>();
-    ctxs[i]->comm->rank = i, ctxs[i]->comm->world = n, ctxs[i]->comm->nccl = comms[size_t(i)];
+    if (const int rc = attachComm(ctxs[i], i, n)) {
+      for (int j = i; j < n; j++) ncclRelease(comms[size_t(j)]);
+      return rc;
+    }
+    ctxs[i]->comm->nccl = comms[size_t(i)];
   }
   return YC_OK;
-#endif
 }
 
 extern "C" int yc_comm_init_custom(yc_ctx* ctx, int rank, int world, yc_collective_fn fn, void* user) {
   if (!ctx || !fn || world < 1 || rank < 0 || rank >= world) return YC_ERR_INVALID;
-  destroyComm(ctx);
-  ctx->comm = std::make_unique<Comm>();
-  ctx->comm->rank = rank, ctx->comm->world = world, ctx->comm->custom = fn, ctx->comm->customUser = user;
+  if (const int rc = attachComm(ctx, rank, world)) return rc;
+  ctx->comm->custom = fn, ctx->comm->customUser = user;
   return YC_OK;
 }
 
@@ -2008,47 +1981,60 @@ static int commSum(yc_ctx* ctx, void* buf, size_t count, int dtype, int root) {
   if (c.group) {
     YC_TRY(rt::sync(ctx->st));  // this participant's buffer is final before the group meets
     const char* e = c.group->sum(c.rank, buf, [&](const GroupPtrs& bufs, int n) -> const char* {
-#ifdef YB_HOSTSIM
-      if (dtype == kCommF32) hostSum<float>(bufs, n, count, root);
-      else if (dtype == kCommI32) hostSum<uint32_t>(bufs, n, count, root);  // wrap-around add of bit patterns: x + 0 is exact
-      else hostSum<uint64_t>(bufs, n, count, root);
-      return nullptr;
-#else
       // the last arrival adds on its own stream; the contexts share a device (or peer access), so every pointer is valid here
       const int grid = int(std::min<size_t>((count + 255) / 256, size_t(ctx->smCount) * 8));
       if (dtype == kCommF32) rt::launch(ctx->st, grid, 256, groupSumKernel<float>, bufs, n, count, root);
-      else if (dtype == kCommI32) rt::launch(ctx->st, grid, 256, groupSumKernel<uint32_t>, bufs, n, count, root);
+      else if (dtype == kCommI32) rt::launch(ctx->st, grid, 256, groupSumKernel<uint32_t>, bufs, n, count, root);  // bit patterns: x + 0 is exact
       else rt::launch(ctx->st, grid, 256, groupSumKernel<unsigned long long>, bufs, n, count, root);
       if (const char* se = rt::sync(ctx->st)) return se;
       return rt::lastError();
-#endif
     });
     if (e) return fail(ctx, YC_ERR_CUDA, "in-process group sum: %s", e);
     return YC_OK;
   }
-#ifndef YB_HOSTSIM
-  const ncclDataType_t t = dtype == kCommF32 ? ncclFloat32 : dtype == kCommI32 ? ncclInt32 : ncclUint64;
-  if (root < 0) YC_NCCL(nccl().AllReduce(buf, buf, count, t, ncclSum, c.nccl, ctx->st.s));
-  else YC_NCCL(nccl().Reduce(buf, buf, count, t, ncclSum, root, c.nccl, ctx->st.s));
+  if (const char* e = ncclStreamSum(c.nccl, buf, count, dtype, root, ctx->st)) return fail(ctx, YC_ERR_CUDA, "NCCL sum: %s", e);
   return YC_OK;
-#else
-  return fail(ctx, YC_ERR_STATE, "communicator without a transport");
-#endif
+}
+
+// The communicator's device staging buffer for small host-value collectives and barriers (64 words, zeroed).
+static int allocScratch(yc_ctx* ctx) {
+  Comm& c = *ctx->comm;
+  if (c.scratch) return YC_OK;
+  void* p = nullptr;
+  YC_TRY(rt::alloc(&p, 64 * sizeof(uint64_t)));
+  c.scratch = static_cast<uint64_t*>(p);
+  YC_TRY(rt::zero(ctx->st, c.scratch, 64 * sizeof(uint64_t)));
+  return YC_OK;
+}
+
+// The smallest collective there is, on the stream, no host values involved (the staging word's content is irrelevant):
+// every participant's earlier work on its stream is done before anybody's later work starts.
+static int commBarrier(yc_ctx* ctx) {
+  if (const int rc = allocScratch(ctx)) return rc;
+  return commSum(ctx, ctx->comm->scratch, 1, kCommU64, -1);
 }
 
 // Sum of n (<= 64) host values over all participants, in place.
 static int commSumHost(yc_ctx* ctx, uint64_t* values, uint32_t n) {
   Comm& c = *ctx->comm;
-  if (!c.scratch) {
-    void* p = nullptr;
-    YC_TRY(rt::alloc(&p, 64 * sizeof(uint64_t)));
-    c.scratch = static_cast<uint64_t*>(p);
-  }
+  if (const int rc = allocScratch(ctx)) return rc;
   YC_TRY(rt::h2d(ctx->st, c.scratch, values, n * sizeof(uint64_t)));
   const int rc = commSum(ctx, c.scratch, n, kCommU64, -1);
   if (rc != YC_OK) return rc;
   YC_TRY(rt::d2h(ctx->st, values, c.scratch, n * sizeof(uint64_t)));
   c.barrierSinceFinalize = true;
+  return YC_OK;
+}
+
+// Runs `collective` (which returns a YC_ code) on the context's stream to completion and adds its time to commMs.
+template <class F>
+static int timedCollective(yc_ctx* ctx, F&& collective) {
+  rt::eventRecord(ctx->st, ctx->ev0);
+  if (const int rc = collective()) return rc;
+  rt::eventRecord(ctx->st, ctx->ev1);
+  YC_TRY(rt::sync(ctx->st));
+  YC_TRY(rt::lastError());
+  ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
   return YC_OK;
 }
 
@@ -2149,79 +2135,63 @@ static int reduceFrames(yc_ctx* ctx, int root, bool async) {
   Comm& c = *ctx->comm;
   if (root < 0 || root >= c.world) return fail(ctx, YC_ERR_INVALID, "bad root");
   const size_t texels = size_t(ctx->frame.width) * ctx->frame.height;
-#ifndef YB_HOSTSIM
   if (async && ctx->wavesPending && c.direct && !c.stale && c.nccl && c.frameTexels == texels && c.root == root) {
     // Chained behind waves in flight: the barrier is enqueued on the main stream after the wave's finalize kernel and
     // nobody waits for it here.  (The stores of wave k + 2 into this copy are issued after barrier k + 1, which the
     // root enters only once it has read what it wanted of wave k.)
-    if (!c.barrierSinceFinalize) {
-      if (!c.scratch) return fail(ctx, YC_ERR_STATE, "no staging buffer");
-      if (const int rc = commSum(ctx, c.scratch, 1, kCommU64, -1)) return rc;
-    }
+    if (!c.barrierSinceFinalize)
+      if (const int rc = commBarrier(ctx)) return rc;
     rt::eventRecord(ctx->st, ctx->ev1);
     c.barrierSinceFinalize = false;
     c.cur = int(c.epoch & 1u);
     c.epoch++;
     return YC_OK;
   }
-#endif
-  (void)async;
   if (ctx->wavesPending)
     if (const int rc = settleWaves(ctx)) return rc;
   if (c.frameTexels != texels || c.root != root) {
     if (const int rc = mapCombinedFrames(ctx, root, texels)) return rc;
   }
-  rt::eventRecord(ctx->st, ctx->ev0);
-  if (c.direct) {
-    // Every finished pixel is already in the root's copy `epoch & 1` (FinalizeK stored it there), unless this context
-    // has to catch up.  What is left is the guarantee that everybody's stores have landed: one small collective on
-    // the streams that ran the finalize kernels — or none, if the caller has run one since (yc_comm_sum_u64).
-    const int k = int(c.epoch & 1u);
-    bool barrier = !c.barrierSinceFinalize;
-    if (c.stale) {
-      rt::launchFor(ctx->st, uint32_t(ctx->pixels.size()),
-                    PushFramesK{ctx->dPixels, ctx->dHdr, ctx->dLdr, c.hdrAll[k], c.ldrAll[k], ctx->frame.width});
-      ctx->launches++;
-      c.stale = false;
-      barrier = true;
-    }
-    if (barrier) {
-      // the smallest collective there is, on the stream, no host values involved (the staging word's content is irrelevant)
-      if (!c.scratch) {
-        void* p = nullptr;
-        YC_TRY(rt::alloc(&p, 64 * sizeof(uint64_t)));
-        c.scratch = static_cast<uint64_t*>(p);
-        YC_TRY(rt::zero(ctx->st, c.scratch, 64 * sizeof(uint64_t)));
+  return timedCollective(ctx, [&] {
+    if (c.direct) {
+      // Every finished pixel is already in the root's copy `epoch & 1` (FinalizeK stored it there), unless this context
+      // has to catch up.  What is left is the guarantee that everybody's stores have landed: one small collective on
+      // the streams that ran the finalize kernels — or none, if the caller has run one since (yc_comm_sum_u64).
+      const int k = int(c.epoch & 1u);
+      bool barrier = !c.barrierSinceFinalize;
+      if (c.stale) {
+        rt::launchFor(ctx->st, uint32_t(ctx->pixels.size()),
+                      PushFramesK{ctx->dPixels, ctx->dHdr, ctx->dLdr, c.hdrAll[k], c.ldrAll[k], ctx->frame.width});
+        ctx->launches++;
+        c.stale = false;
+        barrier = true;
       }
-      if (const int rc = commSum(ctx, c.scratch, 1, kCommU64, -1)) return rc;
-    }
-    c.barrierSinceFinalize = false;
-    c.cur = k;
-    c.epoch++;
-  } else {
-    // out of place: the context's own frames keep blending its tiles in later waves
-    float4 *hdr = c.hdrAll[0], *ldr = c.ldrAll[0];
-    if (c.rank != root) {
-      // a non-root participant of a summing transport needs a send buffer of its own
-      if (!c.block) {
-        void* p = nullptr;
-        YC_TRY(rt::alloc(&p, 2 * texels * sizeof(float4)));
-        c.block = static_cast<float4*>(p);
+      if (barrier)
+        if (const int rc = commBarrier(ctx)) return rc;
+      c.barrierSinceFinalize = false;
+      c.cur = k;
+      c.epoch++;
+    } else {
+      // out of place: the context's own frames keep blending its tiles in later waves
+      float4 *hdr = c.hdrAll[0], *ldr = c.ldrAll[0];
+      if (c.rank != root) {
+        // a non-root participant of a summing transport needs a send buffer of its own
+        if (!c.block) {
+          void* p = nullptr;
+          YC_TRY(rt::alloc(&p, 2 * texels * sizeof(float4)));
+          c.block = static_cast<float4*>(p);
+        }
+        hdr = c.block, ldr = c.block + texels;
       }
-      hdr = c.block, ldr = c.block + texels;
+      YC_TRY(rt::d2d(ctx->st, hdr, ctx->dHdr, texels * sizeof(float4)));
+      YC_TRY(rt::d2d(ctx->st, ldr, ctx->dLdr, texels * sizeof(float4)));
+      int rc = commSum(ctx, hdr, texels * 4, kCommF32, root);
+      if (rc == YC_OK) rc = commSum(ctx, ldr, texels * 4, kCommF32, root);
+      if (rc != YC_OK) return rc;
+      c.cur = 0;
     }
-    YC_TRY(rt::d2d(ctx->st, hdr, ctx->dHdr, texels * sizeof(float4)));
-    YC_TRY(rt::d2d(ctx->st, ldr, ctx->dLdr, texels * sizeof(float4)));
-    int rc = commSum(ctx, hdr, texels * 4, kCommF32, root);
-    if (rc == YC_OK) rc = commSum(ctx, ldr, texels * 4, kCommF32, root);
-    if (rc != YC_OK) return rc;
-    c.cur = 0;
-  }
-  rt::eventRecord(ctx->st, ctx->ev1);
-  YC_TRY(rt::sync(ctx->st));
-  YC_TRY(rt::lastError());
-  ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
-  return YC_OK;
+    return YC_OK;
+  });
 }
 
 extern "C" int yc_comm_reduce_frames(yc_ctx* ctx, int root) { return reduceFrames(ctx, root, false); }
@@ -2252,14 +2222,7 @@ extern "C" int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples) {
   if (!ctx->comm) return fail(ctx, YC_ERR_STATE, "yc_comm_allreduce_buckets without a communicator");
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "no frame");
   const size_t words = size_t(waveBuckets(ctx->frame, waveSamples)) * ctx->bucketCapacity * 4;
-  rt::eventRecord(ctx->st, ctx->ev0);
-  const int rc = commSum(ctx, ctx->dBuckets, words, kCommI32, -1);
-  if (rc != YC_OK) return rc;
-  rt::eventRecord(ctx->st, ctx->ev1);
-  YC_TRY(rt::sync(ctx->st));
-  YC_TRY(rt::lastError());
-  ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
-  return YC_OK;
+  return timedCollective(ctx, [&] { return commSum(ctx, ctx->dBuckets, words, kCommI32, -1); });
 }
 
 // Tile sharding: every participant resolves its planes (zero outside its tiles) into a buffer of its own and the buffers
@@ -2273,13 +2236,11 @@ extern "C" int yc_comm_reduce_aovs(yc_ctx* ctx, int root) {
   if (root < 0 || root >= ctx->comm->world) return fail(ctx, YC_ERR_INVALID, "bad root");
   const size_t n = ctx->aovTexels;
   if (!ctx->dAovComm) YC_TRY(rt::alloc(reinterpret_cast<void**>(&ctx->dAovComm), 2 * n * sizeof(float4)));
-  rt::eventRecord(ctx->st, ctx->ev0);
-  resolveAovs(ctx, ctx->dAovComm, ctx->dAovComm + n);
-  if (const int rc = commSum(ctx, ctx->dAovComm, 2 * n * 4, kCommI32, root)) return rc;
-  rt::eventRecord(ctx->st, ctx->ev1);
-  YC_TRY(rt::sync(ctx->st));
-  YC_TRY(rt::lastError());
-  ctx->commMs += rt::eventElapsedMs(ctx->ev0, ctx->ev1);
+  const int rc = timedCollective(ctx, [&] {
+    resolveAovs(ctx, ctx->dAovComm, ctx->dAovComm + n);
+    return commSum(ctx, ctx->dAovComm, 2 * n * 4, kCommI32, root);
+  });
+  if (rc != YC_OK) return rc;
   ctx->aovCombined = ctx->comm->rank == root;
   return YC_OK;
 }
