@@ -313,8 +313,22 @@ void yc_destroy(yc_ctx* ctx);
 const char* yc_last_error(const yc_ctx* ctx);
 /* Replaces `renderer.scene = scene` (src/core/renderer.hpp:53). */
 int yc_upload_scene(yc_ctx* ctx, const YcScene* scene);
-/* Replaces the `const Camera&` the renderer holds (src/core/renderer.hpp:97). */
+/* Replaces the `const Camera&` the renderer holds (src/core/renderer.hpp:97).  yc_set_cameras(ctx, cam, 1). */
 int yc_set_camera(yc_ctx* ctx, const YcCamera* cam);
+/* Several views of the scene in one frame: n cameras (1 <= n <= 65535; YC_ERR_INVALID otherwise or for NULL) that share
+ * the YcFrameDesc — size, samples, tile size, tonemap, estimator, background.  Each view is the frame its camera renders
+ * alone, bit for bit (HDR, LDR, AOVs; the ray counts of YcStats add up over the views): the sampler depends on the
+ * view-local pixel, the sample index and the frame's totalSamples / tileSize only.
+ *   Layout: the views are stacked by rows.  View v occupies rows [v·height, (v+1)·height) of a frame of width x
+ *     (height·n) texels: every frame and AOV plane is [n][height][width][4] floats.  YcRect arguments are in these
+ *     stacked rows (a rectangle may span views); yc_generate_primary_rays writes the rays of every view.
+ *   Tiles: the tile list is the reference's (tile-renderer.hpp:127-144) of each view, view after view; tile k of that
+ *     list goes to shard k % shardCount.
+ *   The view count of a frame is fixed by yc_begin_frame from the cameras set then.  Setting the same number of cameras
+ *     later is allowed (the next wave uses them); after a different number, yc_render_wave[_async], yc_accumulate_wave,
+ *     yc_finalize_wave and yc_generate_primary_rays return YC_ERR_STATE until the next yc_begin_frame.
+ *   A frame holds at most 2^32 texels (YC_ERR_INVALID from yc_begin_frame). */
+int yc_set_cameras(yc_ctx* ctx, const YcCamera* cams, uint32_t n);
 /* Replaces TileRenderer::renderImpl's state reset (tile-renderer.hpp:118-124). */
 int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* frame);
 /* Replaces one wave of the worker loop + finishTile for every tile
@@ -352,7 +366,7 @@ int yc_accumulate_wave(yc_ctx* ctx, YcRect pixels, uint32_t sampleOffset, uint32
 int yc_bucket_device_ptrs(yc_ctx* ctx, void** buckets, size_t* bytes, uint32_t* planes, size_t* planePixels);
 int yc_wave_buckets(yc_ctx* ctx, uint32_t waveSamples, uint32_t* m);
 int yc_finalize_wave(yc_ctx* ctx, YcRect pixels, uint32_t waveSamples, uint32_t takenBefore);
-/* Copies the frames to host (either pointer may be NULL).  width*height*4 floats each.
+/* Copies the frames to host (either pointer may be NULL).  width·height·V·4 floats each (V views, yc_set_cameras).
  * Replaces reading Renderer::m_buffer (RenderData::buffer, renderer.hpp:22-28). */
 int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
 /* First-hit AOVs: guide buffers for a denoiser, collected while the frame renders (no extra ray).
@@ -376,13 +390,13 @@ int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
  *                      YC_INTEGRATOR_NAIVE.  The first enable allocates 32 bytes per path in flight (twice, per lane:
  *                      512 MB at the default capacity) and four float4 and one uint32 per texel of the frame.
  *                      yc_accumulate_wave with bucketShardCount > 1 returns YC_ERR_UNSUPPORTED while AOVs are on.
- *   yc_resolve_aovs    copies both planes (width*height*4 floats each; either pointer may be NULL); YC_ERR_STATE
+ *   yc_resolve_aovs    copies both planes (width·height·V·4 floats each; either pointer may be NULL); YC_ERR_STATE
  *                      when AOVs are not enabled.
  *   yc_comm_reduce_aovs  tile sharding, collective: combines every participant's planes into the root's, out of place
  *                      (repeated calls count nothing twice); yc_resolve_aovs_combined copies them out on the root. */
 int yc_enable_aovs(yc_ctx* ctx, int enable);
 int yc_resolve_aovs(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA);
-/* Device pointers of the frames (for NCCL reductions by the caller). */
+/* Device pointers of the frames (for NCCL reductions by the caller); *bytes = width·height·V·4 floats. */
 int yc_frame_device_ptrs(yc_ctx* ctx, void** hdr, void** ldr, size_t* bytes);
 /* Re-run the tonemap over the whole HDR frame (after a cross-GPU sum). */
 int yc_retonemap(yc_ctx* ctx);
@@ -409,7 +423,8 @@ int yc_host_free(yc_ctx* ctx, void* p);
 int yc_memcpy_h2d(yc_ctx* ctx, void* dst, const void* src, size_t bytes);
 int yc_memcpy_d2h(yc_ctx* ctx, void* dst, const void* src, size_t bytes);
 /* Primary rays exactly as RayIntegrator::sample generates them (ray-integrator.cpp:11-18),
- * written to a device YcRay array of width*height*spp entries (sample-major). */
+ * written to a device YcRay array of width*height*V*spp entries (sample-major; within a sample, the shard's pixel list
+ * order: view after view). */
 int yc_generate_primary_rays(yc_ctx* ctx, uint32_t sampleOffset, uint32_t spp, void* raysDev);
 int yc_synchronize(yc_ctx* ctx);
 /* Renderer::abort (src/core/renderer.hpp:77-83, tile-renderer.hpp:40-63): `flag` is polled between chunks and between
@@ -448,6 +463,7 @@ int yc_comm_reduce_frames(yc_ctx* ctx, int root);
  * and not waited for (otherwise the same as yc_comm_reduce_frames, waiting included). */
 int yc_comm_reduce_frames_async(yc_ctx* ctx, int root);
 int yc_comm_frames_direct(yc_ctx* ctx, int* direct);
+/* The root's combined frames: width·height·V·4 floats each (either pointer may be NULL). */
 int yc_resolve_combined(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA);
 /* Bucket sharding (yc_accumulate_wave): all-reduce(sum, int32) of the planes a wave of `waveSamples` samples uses. */
 int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples);
@@ -603,10 +619,15 @@ void yr_destroy(yr_renderer* r);
 int yr_set_wave_callback(yr_renderer* r, yr_wave_callback cb, void* user);
 int yr_set_tile_callback(yr_renderer* r, yr_tile_callback cb, void* user);
 int yr_set_done_callback(yr_renderer* r, yr_done_callback cb, void* user);
-/* Host frame (width*height*4 floats) that receives the tonemapped frame — the HDR one when tonemap is NONE, like
+/* Host frame (width*height*V*4 floats, V views of yr_set_cameras stacked by rows) that receives the tonemapped frame — the HDR one when tonemap is NONE, like
  * Renderer::m_buffer (tile-renderer.hpp:238) — after every wave, before the callbacks fire. */
 int yr_set_frame_target(yr_renderer* r, float* ldrRGBA);
 int yr_set_camera(yr_renderer* r, const YcCamera* camera); /* the camera moved between renders */
+/* n views of the scene per render (yc_set_cameras: 1 <= n <= 65535, stacked by rows, each bit-identical to a render of
+ * its camera alone).  Like yr_set_camera it waits for a render in progress and applies to the next one; the count may
+ * change between renders.  Frames, AOV planes, the frame target and the PPM are width x (height·n); the tile callback
+ * reports every tile of every view per wave (stacked x, y, w, h; index over all n views, total = n x tiles per view). */
+int yr_set_cameras(yr_renderer* r, const YcCamera* cameras, uint32_t n);
 int yr_render(yr_renderer* r);     /* Renderer::render(): asynchronous */
 int yr_abort(yr_renderer* r);      /* Renderer::abort(): returns at once, the render stops at its next chunk / bounce */
 int yr_wait(yr_renderer* r);       /* Renderer::wait() */
@@ -616,11 +637,12 @@ int yr_read(yr_renderer* r, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
 /* First-hit AOVs of the renders that follow (yc_enable_aovs; YC_ERR_UNSUPPORTED for the naive integrator and for
  * YR_SHARD_BUCKETS over more than one participant, YC_ERR_STATE while a render runs). */
 int yr_enable_aovs(yr_renderer* r, int enable);
-/* The AOV planes of the last render (width*height*4 floats each, either pointer may be NULL), valid once it has returned
+/* The AOV planes of the last render (width*height*V*4 floats each, either pointer may be NULL), valid once it has returned
  * (yr_render_sync / yr_wait) and YC_ERR_STATE while one runs.  Tile sharding: the combined planes, on the root; other
  * ranks' buffers are left untouched, as with yr_read. */
 int yr_read_aovs(yr_renderer* r, float* albedoRGBA, float* normalDepthRGBA);
-/* writePPM(out, renderer buffer): the tonemapped frame as a binary PPM (frontend main.cpp writes out.ppm). */
+/* writePPM(out, renderer buffer): the tonemapped frame as a binary PPM (frontend main.cpp writes out.ppm); width x
+ * (height·V) with several views. */
 int yr_write_ppm(yr_renderer* r, const char* path);
 yc_ctx* yr_context(yr_renderer* r);
 const char* yr_last_error(const yr_renderer* r);

@@ -180,6 +180,12 @@ class Scene:
                 np.ctypeslib.as_array(idx, (n_tris.value,)).copy())
 
 
+def _camera_array(cameras):
+    """(ctypes array of YcCamera, count) from a sequence of cameras."""
+    cams = list(cameras)
+    return (capi.YcCamera * len(cams))(*cams), len(cams)
+
+
 def make_camera(width, height, focal=35.0, fnum=0.0, pos=(0, 0, 5), target=(0, 0, 0), up=(0, 0, 0), exposure=0.0,
                 sides=0) -> capi.YcCamera:
     """Camera({w,h}, focal, fnum) + moveAndLookAt(pos, target, up) (camera.hpp:77-136)."""
@@ -207,6 +213,8 @@ class Context:
         rc = lib().yc_create(device, C.byref(opts), C.byref(self._h))
         _check(rc, "yc_create", _SAMPLERS_HINT if rc == capi.YC_ERR_UNSUPPORTED else _NO_DEVICE)
         self.frame = None
+        self.cameras = 1  # cameras set (yc_set_cameras)
+        self.views = 1    # views of the current frame, stacked by rows: frames are (views * height, width, 4)
 
     def close(self):
         if self._h:
@@ -227,17 +235,23 @@ class Context:
 
     def set_camera(self, cam: capi.YcCamera):
         self._ck(lib().yc_set_camera(self._h, C.byref(cam)), "yc_set_camera")
+        self.cameras = 1
+
+    def set_cameras(self, cams):
+        """yc_set_cameras: one view per camera; the next begin_frame's frame stacks them by rows."""
+        arr, n = _camera_array(cams)
+        self._ck(lib().yc_set_cameras(self._h, arr, n), "yc_set_cameras")
+        self.cameras = n
 
     def begin_frame(self, width, height, total_samples, tile_size=64, background=(0, 0, 0), tonemap=TONEMAP_AGX,
                     estimator=ESTIMATOR_GMON, shard_index=0, shard_count=1):
         f = capi.YcFrameDesc(width, height, total_samples, tile_size, _f3(background), tonemap, estimator, shard_index,
                              shard_count)
         self._ck(lib().yc_begin_frame(self._h, C.byref(f)), "yc_begin_frame")
-        self.frame = f
+        self.frame, self.views = f, self.cameras
 
     def render_wave(self, sample_offset, wave_samples, taken_before, rect=None):
-        r = capi.YcRect(0, 0, self.frame.width, self.frame.height) if rect is None else capi.YcRect(*rect)
-        self._ck(lib().yc_render_wave(self._h, r, sample_offset, wave_samples, taken_before), "yc_render_wave")
+        self._ck(lib().yc_render_wave(self._h, self._rect(rect), sample_offset, wave_samples, taken_before), "yc_render_wave")
 
     def render_wave_async(self, sample_offset, wave_samples, taken_before, rect=None):
         """yc_render_wave_async: the wave stays in flight; wave_sync() (or any other call) waits for it."""
@@ -247,7 +261,8 @@ class Context:
         self._ck(lib().yc_wave_sync(self._h), "yc_wave_sync")
 
     def _rect(self, rect):
-        return capi.YcRect(0, 0, self.frame.width, self.frame.height) if rect is None else capi.YcRect(*rect)
+        """rect = (x, y, w, h) in the frame's stacked rows; None: the whole frame."""
+        return capi.YcRect(0, 0, self.frame.width, self.frame.height * self.views) if rect is None else capi.YcRect(*rect)
 
     def accumulate_wave(self, sample_offset, wave_samples, bucket_shard=0, bucket_shard_count=1, rect=None):
         """Sample loop of a wave into the estimator buckets; with bucket_shard_count > 1 only the samples of
@@ -271,7 +286,7 @@ class Context:
         return p.value, n.value, planes.value, pix.value
 
     def resolve(self, want_hdr=True, want_ldr=True):
-        h, w = self.frame.height, self.frame.width
+        h, w = self.frame.height * self.views, self.frame.width
         hdr = np.empty((h, w, 4), np.float32) if want_hdr else None
         ldr = np.empty((h, w, 4), np.float32) if want_ldr else None
         st = capi.YcStats()
@@ -297,8 +312,8 @@ class Context:
         self._ck(lib().yc_enable_aovs(self._h, int(enable)), "yc_enable_aovs")
 
     def resolve_aovs(self):
-        """(albedo RGBA, normalDepth RGBA) as two (h, w, 4) float32 arrays."""
-        h, w = self.frame.height, self.frame.width
+        """(albedo RGBA, normalDepth RGBA) as two (views * h, w, 4) float32 arrays."""
+        h, w = self.frame.height * self.views, self.frame.width
         albedo, nd = np.empty((h, w, 4), np.float32), np.empty((h, w, 4), np.float32)
         self._ck(lib().yc_resolve_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yc_resolve_aovs")
         return albedo, nd
@@ -308,7 +323,7 @@ class Context:
         self._ck(lib().yc_comm_reduce_aovs(self._h, root), "yc_comm_reduce_aovs")
 
     def resolve_aovs_combined(self):
-        h, w = self.frame.height, self.frame.width
+        h, w = self.frame.height * self.views, self.frame.width
         albedo, nd = np.empty((h, w, 4), np.float32), np.empty((h, w, 4), np.float32)
         self._ck(lib().yc_resolve_aovs_combined(self._h, albedo.ctypes.data, nd.ctypes.data), "yc_resolve_aovs_combined")
         return albedo, nd
@@ -334,7 +349,7 @@ class Context:
         self._ck(lib().yc_comm_allreduce_buckets(self._h, wave_samples), "yc_comm_allreduce_buckets")
 
     def resolve_combined(self, want_hdr=True, want_ldr=True):
-        h, w = self.frame.height, self.frame.width
+        h, w = self.frame.height * self.views, self.frame.width
         hdr = np.empty((h, w, 4), np.float32) if want_hdr else None
         ldr = np.empty((h, w, 4), np.float32) if want_ldr else None
         self._ck(lib().yc_resolve_combined(self._h, hdr.ctypes.data if want_hdr else None, ldr.ctypes.data if want_ldr else None),
@@ -394,12 +409,14 @@ class Renderer:
     """Mirror of cpu::TileRenderer's public surface (tile-renderer.hpp:27-38) + Renderer
     (renderer.hpp:53-95): knobs as attributes, render()/abort()/wait()/render_sync()."""
 
-    def __init__(self, width, height, camera: capi.YcCamera, scene: Scene | None = None, samples=64,
+    def __init__(self, width, height, camera, scene: Scene | None = None, samples=64,
                  first_wave_samples=None, max_wave_samples=None, tile_size=64, max_depth=30, background=(0, 0, 0),
                  tonemap=TONEMAP_AGX, estimator=ESTIMATOR_GMON, shard_index=0, shard_count=1, device=0,
                  integrator=capi.INTEGRATOR_MIS, scrambler=capi.SCRAMBLER_FAST_OWEN, sampler=capi.SAMPLER_SOBOL,
                  traversal=None, sharding=capi.SHARD_TILES, devices=None, dist=None, aovs=False):
-        """devices=[g0, g1, ...]: one renderer over several GPUs of this process (yr_create_multi).
+        """camera: a YcCamera, or a sequence of them: one view per camera in every frame (yr_set_cameras), and the
+        frames, AOV planes, pinned buffers and frame target get a leading view axis (V, height, width, ...).
+        devices=[g0, g1, ...]: one renderer over several GPUs of this process (yr_create_multi).
         aovs=True: collect the first-hit albedo / normal / depth planes (yr_enable_aovs; read_aovs()).
         dist=(rank, world, comm): one process per GPU (yr_create_dist); comm = the 128 bytes of comm_unique_id() from
         rank 0, or a callable collective(buf_ptr, count, dtype, root) → 0 (yr_create_dist_custom)."""
@@ -413,6 +430,12 @@ class Renderer:
         self.scene = scene
         self._h = C.c_void_p()
         self._cb = self._tile_cb = self._done_cb = self._coll = None
+        self._target = None
+        camera_arg = camera
+        cams = [camera] if isinstance(camera, capi.YcCamera) else list(camera)
+        if not cams:
+            raise ValueError("Renderer: no camera")
+        camera = cams[0]
         sh = scene._h if scene else None
         if devices is not None:
             arr = (C.c_int * len(devices))(*devices)
@@ -429,6 +452,12 @@ class Renderer:
         else:
             rc, what = lib().yr_create(C.byref(s), sh, C.byref(camera), C.byref(self._h)), "yr_create"
         _check(rc, what, _NO_DEVICE if rc == capi.YC_ERR_NO_DEVICE else b"")
+        # None: one camera given as such, and shapes without a view axis; else the number of views.  _frame_views: the
+        # same for the frame of the last render, which read() and read_aovs() return
+        self._views = self._frame_views = None
+        if not isinstance(camera_arg, capi.YcCamera):
+            self.set_camera(cams)
+            self._frame_views = self._views
         if aovs:
             self.enable_aovs()
 
@@ -477,18 +506,38 @@ class Renderer:
         self._done_cb = capi.DONE_CALLBACK(tramp)
         self._ck(lib().yr_set_done_callback(self._h, self._done_cb, None), "yr_set_done_callback")
 
-    def set_camera(self, camera: capi.YcCamera):
-        self._ck(lib().yr_set_camera(self._h, C.byref(camera)), "yr_set_camera")
+    def set_camera(self, camera):
+        """A YcCamera, or a sequence of them (yr_set_cameras: one view each, a leading view axis on the frames of the
+        renders that follow)."""
+        if isinstance(camera, capi.YcCamera):
+            self._ck(lib().yr_set_camera(self._h, C.byref(camera)), "yr_set_camera")
+            self._views = None
+        else:
+            arr, n = _camera_array(camera)
+            self._ck(lib().yr_set_cameras(self._h, arr, n), "yr_set_cameras")
+            self._views = n
+
+    def _shape(self, views, *tail):
+        """Frame shape (h, w, *tail), with a leading view axis when the cameras came as a sequence."""
+        h, w = self.settings.height, self.settings.width
+        return (h, w, *tail) if views is None else (views, h, w, *tail)
 
     def set_frame_target(self, ldr: np.ndarray):
-        """(height, width, 4) float32, C-contiguous: receives the tonemapped frame after every wave, before the callbacks
-        (Renderer::m_buffer; yr_set_frame_target).  None detaches."""
+        """(height, width, 4) float32, C-contiguous — (V, height, width, 4) with a sequence of cameras: receives the
+        tonemapped frame after every wave, before the callbacks (Renderer::m_buffer; yr_set_frame_target).  None detaches."""
         if ldr is not None:
-            assert ldr.dtype == np.float32 and ldr.flags.c_contiguous and ldr.size == self.settings.width * self.settings.height * 4
+            assert ldr.dtype == np.float32 and ldr.flags.c_contiguous and ldr.shape == self._shape(self._views, 4)
         self._target = ldr
         self._ck(lib().yr_set_frame_target(self._h, ldr.ctypes.data if ldr is not None else None), "yr_set_frame_target")
 
+    def _start(self):
+        """The frame of the render about to start has the current cameras' views; the frame target must hold it."""
+        if self._target is not None and self._target.shape != self._shape(self._views, 4):
+            raise ValueError(f"frame target of shape {self._target.shape} for a frame of {self._shape(self._views, 4)}")
+        self._frame_views = self._views
+
     def render(self):
+        self._start()
         self._ck(lib().yr_render(self._h), "yr_render")
 
     def abort(self):
@@ -503,31 +552,34 @@ class Renderer:
         return True
 
     def render_sync(self) -> dict:
+        self._start()
         d = capi.YrRenderData()
         self._ck(lib().yr_render_sync(self._h, C.byref(d)), "yr_render_sync")
         return dict(samples_taken=d.samplesTaken, total_samples=d.totalSamples, total_rays=d.totalRays,
                     total_time_ms=d.totalTimeMs)
 
-    def _pinned_frame(self, key):
-        """A page-locked (h, w, 4) float32 array owned by this renderer (allocated once)."""
+    def _pinned_frame(self, key, shape):
+        """A page-locked float32 array of `shape` owned by this renderer (allocated once per key and shape)."""
         if not hasattr(self, "_pinned"):
             self._pinned = {}
+        key = (key, shape)
         if key not in self._pinned:
-            h, w = self.settings.height, self.settings.width
+            n = int(np.prod(shape))
             p = C.c_void_p()
-            _check(lib().yc_host_alloc(self.context_handle(), h * w * 16, C.byref(p)), "yc_host_alloc")
-            buf = (C.c_float * (h * w * 4)).from_address(p.value)
-            self._pinned[key] = (p, np.frombuffer(buf, np.float32).reshape(h, w, 4))
+            _check(lib().yc_host_alloc(self.context_handle(), n * 4, C.byref(p)), "yc_host_alloc")
+            buf = (C.c_float * n).from_address(p.value)
+            self._pinned[key] = (p, np.frombuffer(buf, np.float32).reshape(shape))
         return self._pinned[key][1]
 
     def read(self, want_hdr=True, want_ldr=True, pinned=False):
-        h, w = self.settings.height, self.settings.width
+        """(hdr, ldr, stats) of the last render: (h, w, 4) float32 frames, (V, h, w, 4) with a sequence of cameras."""
+        shape = self._shape(self._frame_views, 4)
         if pinned:
-            hdr = self._pinned_frame("hdr") if want_hdr else None
-            ldr = self._pinned_frame("ldr") if want_ldr else None
+            hdr = self._pinned_frame("hdr", shape) if want_hdr else None
+            ldr = self._pinned_frame("ldr", shape) if want_ldr else None
         else:
-            hdr = np.empty((h, w, 4), np.float32) if want_hdr else None
-            ldr = np.empty((h, w, 4), np.float32) if want_ldr else None
+            hdr = np.empty(shape, np.float32) if want_hdr else None
+            ldr = np.empty(shape, np.float32) if want_ldr else None
         st = capi.YcStats()
         self._ck(lib().yr_read(self._h, hdr.ctypes.data if want_hdr else None, ldr.ctypes.data if want_ldr else None,
                                C.byref(st)), "yr_read")
@@ -539,9 +591,10 @@ class Renderer:
 
     def read_aovs(self) -> dict:
         """The last render's first-hit AOVs: dict(albedo=(h, w, 3), coverage=(h, w), normal=(h, w, 3), depth=(h, w)),
-        float32 (tile sharding over ranks: the combined planes on rank 0; zeros elsewhere)."""
-        h, w = self.settings.height, self.settings.width
-        albedo, nd = np.zeros((h, w, 4), np.float32), np.zeros((h, w, 4), np.float32)
+        float32 (tile sharding over ranks: the combined planes on rank 0; zeros elsewhere); a leading view axis with a
+        sequence of cameras."""
+        shape = self._shape(self._frame_views, 4)
+        albedo, nd = np.zeros(shape, np.float32), np.zeros(shape, np.float32)
         self._ck(lib().yr_read_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yr_read_aovs")
         return dict(albedo=albedo[..., :3].copy(), coverage=albedo[..., 3].copy(), normal=nd[..., :3].copy(), depth=nd[..., 3].copy())
 

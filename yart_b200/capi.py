@@ -131,6 +131,7 @@ PROTOTYPES = {
     "yc_last_error": (C.c_char_p, [P]),
     "yc_upload_scene": (C.c_int, [P, C.POINTER(YcScene)]),
     "yc_set_camera": (C.c_int, [P, C.POINTER(YcCamera)]),
+    "yc_set_cameras": (C.c_int, [P, C.POINTER(YcCamera), u32]),
     "yc_begin_frame": (C.c_int, [P, C.POINTER(YcFrameDesc)]),
     "yc_render_wave": (C.c_int, [P, YcRect, u32, u32, u32]),
     "yc_render_wave_async": (C.c_int, [P, YcRect, u32, u32, u32]),
@@ -203,6 +204,7 @@ PROTOTYPES = {
     "yr_set_done_callback": (C.c_int, [P, DONE_CALLBACK, P]),
     "yr_set_frame_target": (C.c_int, [P, P]),
     "yr_set_camera": (C.c_int, [P, C.POINTER(YcCamera)]),
+    "yr_set_cameras": (C.c_int, [P, C.POINTER(YcCamera), u32]),
     "yr_render": (C.c_int, [P]),
     "yr_abort": (C.c_int, [P]),
     "yr_wait": (C.c_int, [P]),

@@ -55,15 +55,22 @@ struct Counters {
 
 // Everything a stage needs besides the scene.
 struct WaveParams {
-  YcCamera cam;
+  const YcCamera* cams;         // one per view of the frame (yc_set_cameras), read by raygen only
+  const uint16_t* pixelViews;   // the view of each entry of pixelList, read by raygen only
+  // Keeps `smp` and everything after it at offset 96 of the struct, and the struct's size: ptxas's register allocation
+  // of the traversal, tail and naive kernels depends on their parameter layout, and with these 80 bytes gone the
+  // alpha-tested and naive variants spill (tailKernel<false, Bvh2Walk> 28 bytes, naiveKernel<true> 24 bytes).
+  uint32_t layoutPad[20];
   SamplerConfig smp;
   float bg[3];
   uint32_t maxDepth;
-  // chunk geometry: path i ↔ pixel pixelList[pixBase + i % nPix], sample s0 + (i / nPix) * (sStrideM1 + 1)
-  const uint32_t* pixelList;  // x | y << 16
+  // chunk geometry: path i ↔ pixel pixelList[pixBase + i % nPix] of view pixelViews[pixBase + i % nPix],
+  // sample s0 + (i / nPix) * (sStrideM1 + 1)
+  const uint32_t* pixelList;  // x | y << 16, view-local coordinates (what the sampler sees)
   uint32_t pixBase, nPix, s0;
   uint32_t sStrideM1;  // sample stride - 1: 0 for consecutive samples, m - 1 when a chunk holds one estimator bucket's samples
 };
+static_assert(offsetof(WaveParams, smp) == 96, "WaveParams layout: see layoutPad");
 
 YB_DEV void pathPixelSample(const WaveParams& w, uint32_t i, uint32_t& px, uint32_t& py, uint32_t& sample) {
   const uint32_t pix = w.pixelList[w.pixBase + i % w.nPix];
@@ -88,7 +95,7 @@ YB_DEV void raygenStage(const WaveParams& w, const PathState& ps, uint32_t i) {
   Sampler smp;
   smp.start(w.smp, px, py, s);  // Integrator::render, integrator.cpp:20
   V3 o, d;
-  primaryRay(w.cam, smp, px, py, o, d);
+  primaryRay(w.cams[w.pixelViews[w.pixBase + i % w.nPix]], smp, px, py, o, d);
   ps.rayO[i] = make_float4(o.x, o.y, o.z, 0.0f);
   ps.rayD[i] = make_float4(d.x, d.y, d.z, 0.0f);
   ps.L[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);

@@ -257,7 +257,7 @@ extern "C" int yc_kat(yc_ctx* ctx, const char* kind, const void* in, size_t inBy
   else return fail(ctx, YC_ERR_INVALID, "unknown kat kind %s", kind);
   if (inWords < header + size_t(n) * recWords || outBytes < size_t(n) * outWords * 4)
     return fail(ctx, YC_ERR_INVALID, "yc_kat(%s): buffer sizes do not match %u records", kind, n);
-  if (k == "camera" && !ctx->hasCamera) return fail(ctx, YC_ERR_STATE, "yc_kat(camera) needs yc_set_camera");
+  if (k == "camera" && ctx->cams.empty()) return fail(ctx, YC_ERR_STATE, "yc_kat(camera) needs yc_set_camera");
   if (n == 0) return YC_OK;
   void *din = nullptr, *dout = nullptr;
   YC_TRY(rt::alloc(&din, inBytes));
@@ -283,7 +283,7 @@ extern "C" int yc_kat(yc_ctx* ctx, const char* kind, const void* in, size_t inBy
     else if (k == "gmon") rt::launchFor(ctx->st, n, KatGmon{io, hin[0]});
     else if (k == "gmonb") rt::launchFor(ctx->st, n, KatGmonb{io, hin[0]});
     else if (k == "agx") rt::launchFor(ctx->st, n, KatAgx{io, hin[0] == 1 ? uint32_t(YC_TONEMAP_AGX_GOLDEN) : hin[0] == 2 ? uint32_t(YC_TONEMAP_AGX_PUNCHY) : uint32_t(YC_TONEMAP_AGX)});
-    else if (k == "camera") rt::launchFor(ctx->st, n, KatCamera{io, ctx->cam});
+    else if (k == "camera") rt::launchFor(ctx->st, n, KatCamera{io, ctx->cams[0]});
     else rt::launchFor(ctx->st, n, KatTexture{io, ctx->ds});
     ctx->launches++;
     e = rt::d2h(ctx->st, out, dout, size_t(n) * outWords * 4);

@@ -100,15 +100,22 @@ struct yc_ctx {
   std::vector<void*> sceneAllocs;
   DScene ds{};
   bool hasScene = false;
-  YcCamera cam{};
-  bool hasCamera = false;
+  // yc_set_cameras: one camera per view, and exp2(exposure) of each (integrator.cpp:23), on the host and the device
+  std::vector<YcCamera> cams;
+  std::vector<float> exposureScales;
+  YcCamera* dCams = nullptr;
+  float* dExposureScales = nullptr;
 
-  // frame
+  // frame: `views` stacked views of frame.width x frame.height (view v = rows [v·height, (v+1)·height))
   bool inFrame = false;
   YcFrameDesc frame{};
-  std::vector<uint32_t> pixels;  // this shard's pixels, tile-major: x | y << 16
+  uint32_t views = 0;
+  std::vector<uint32_t> pixels;  // this shard's pixels, view-major then tile-major: x | y << 16 in view-local coordinates
+  std::vector<uint16_t> pixelViews;  // the view of each entry of `pixels`
   uint32_t* dPixels = nullptr;
   uint32_t* dPixelsScratch = nullptr;
+  uint16_t* dPixelViews = nullptr;
+  uint16_t* dPixelViewsScratch = nullptr;
   float4 *dHdr = nullptr, *dLdr = nullptr, *dBuckets = nullptr;
   size_t bucketCapacity = 0;  // pixels per bucket plane
   bool bucketsDirty = false;  // an accumulate was not (or only partly) followed by a finalize: the planes hold sums
@@ -211,6 +218,15 @@ static void freeAll(std::vector<void*>& v) {
 // ---------------------------------------------------------------------------------------
 // stages as functors (run by rt::launchFor) and the two persistent traversal kernels
 // ---------------------------------------------------------------------------------------
+// The frame as a texel array: the views stacked by rows, [views][height][width].
+static size_t frameTexels(const YcFrameDesc& f, uint32_t views) { return size_t(f.width) * f.height * views; }
+static size_t frameTexels(const yc_ctx* ctx) { return frameTexels(ctx->frame, ctx->views); }
+
+// Texel of a pixel-list entry (view-local x | y << 16) of view `view`.
+YB_DEV size_t texelIndex(uint32_t pix, uint32_t view, uint32_t width, uint32_t height) {
+  return (size_t(view) * height + (pix >> 16)) * width + (pix & 0xffffu);
+}
+
 struct RaygenK {
   WaveParams w;
   PathState ps;
@@ -313,9 +329,11 @@ struct AccumulateK {
   PathState ps;
   float4* buckets;
   size_t planeStride;
+  const uint16_t* pixelViews;     // the call's pixel list's views
+  const float* exposureScales;    // per view
   uint32_t pixBase, nPix, K, waveSampleBase, sampleStride, m, estimator;
-  float exposureScale;
   YB_DEV void operator()(uint32_t p) const {
+    const float exposureScale = exposureScales[pixelViews[pixBase + p]];
     for (uint32_t k = 0; k < K; k++) {
       const float4 L4 = ps.L[size_t(k) * nPix + p];
       const V3 s = V3(L4.x, L4.y, L4.z) * exposureScale;
@@ -334,11 +352,12 @@ struct AccumulateK {
 // Estimator::getValue + TileRenderer::finishTile's blend and tonemap (tile-renderer.hpp:220-239).
 struct FinalizeK {
   const uint32_t* pixelList;
+  const uint16_t* pixelViews;
   float4* buckets;
   size_t planeStride;
   float4 *hdr, *ldr;
   float4 *hdrRoot, *ldrRoot;  // tile sharding over GPUs that reach the root's memory (comm.cuh): the combined frames, else null
-  uint32_t width, m, estimator, waveSamples, tonemap;
+  uint32_t width, height, m, estimator, waveSamples, tonemap;
   float wCurrent, wWave;
   YB_DEV void operator()(uint32_t p) const {
     V3 acc[kMaxBuckets];
@@ -351,8 +370,7 @@ struct FinalizeK {
       *slot = make_float4(0.0f, 0.0f, 0.0f, 0.0f);  // ready for the next wave
     }
     const V3 wave = estimatorValue(int(estimator), acc, cnt, int(m), waveSamples);
-    const uint32_t pix = pixelList[p];
-    const size_t idx = size_t(pix >> 16) * width + (pix & 0xffffu);
+    const size_t idx = texelIndex(pixelList[p], pixelViews[p], width, height);
     const float4 cur = hdr[idx];
     float4 h;
     h.x = cur.x * wCurrent + wave.x * wWave;
@@ -374,12 +392,12 @@ struct FinalizeK {
 // wave after the frames were mapped, or after a wave that finalized only part of the shard).
 struct PushFramesK {
   const uint32_t* pixelList;
+  const uint16_t* pixelViews;
   const float4 *hdr, *ldr;
   float4 *hdrRoot, *ldrRoot;
-  uint32_t width;
+  uint32_t width, height;
   YB_DEV void operator()(uint32_t p) const {
-    const uint32_t pix = pixelList[p];
-    const size_t idx = size_t(pix >> 16) * width + (pix & 0xffffu);
+    const size_t idx = texelIndex(pixelList[p], pixelViews[p], width, height);
     hdrRoot[idx] = hdr[idx], ldrRoot[idx] = ldr[idx];
   }
 };
@@ -420,13 +438,13 @@ struct AovCaptureK {
 struct AovAccumulateK {
   const float4* rec;
   const uint32_t* pixelList;
+  const uint16_t* pixelViews;
   float4* sum;
   uint32_t* count;
   size_t texels;
-  uint32_t pixBase, nPix, K, width;
+  uint32_t pixBase, nPix, K, width, height;
   YB_DEV void operator()(uint32_t p) const {
-    const uint32_t pix = pixelList[pixBase + p];
-    const size_t idx = size_t(pix >> 16) * width + (pix & 0xffffu);
+    const size_t idx = texelIndex(pixelList[pixBase + p], pixelViews[pixBase + p], width, height);
     float4 a = sum[idx], b = sum[texels + idx];
     uint32_t hits = __float_as_uint(a.w);
     for (uint32_t k = 0; k < K; k++) {
@@ -711,7 +729,10 @@ static void freeFrame(yc_ctx* ctx) {
   rt::release(ctx->dHdr);
   rt::release(ctx->dLdr);
   rt::release(ctx->dBuckets);
+  rt::release(ctx->dPixelViews);
+  rt::release(ctx->dPixelViewsScratch);
   ctx->dPixels = ctx->dPixelsScratch = nullptr;
+  ctx->dPixelViews = ctx->dPixelViewsScratch = nullptr;
   ctx->dHdr = ctx->dLdr = ctx->dBuckets = nullptr;
   ctx->inFrame = false;
 }
@@ -738,6 +759,8 @@ extern "C" void yc_destroy(yc_ctx* ctx) {
   freeAovPlanes(ctx);
   freeAll(ctx->sceneAllocs);
   freeAll(ctx->waveAllocs);
+  rt::release(ctx->dCams);
+  rt::release(ctx->dExposureScales);
   rt::eventDestroy(ctx->ev0);
   rt::eventDestroy(ctx->ev1);
   rt::eventDestroy(ctx->evFinal);
@@ -881,13 +904,27 @@ extern "C" int yc_upload_scene(yc_ctx* ctx, const YcScene* s) {
   return YC_OK;
 }
 
-extern "C" int yc_set_camera(yc_ctx* ctx, const YcCamera* cam) {
-  if (!ctx || !cam) return YC_ERR_INVALID;
+extern "C" int yc_set_cameras(yc_ctx* ctx, const YcCamera* cams, uint32_t n) {
+  if (!ctx || !cams || n == 0 || n > 65535) return YC_ERR_INVALID;
   YC_ENTER(ctx);
-  ctx->cam = *cam;
-  ctx->hasCamera = true;
+  if (n != ctx->cams.size()) {
+    YC_TRY(rt::sync(ctx->st));
+    rt::release(ctx->dCams);
+    rt::release(ctx->dExposureScales);
+    ctx->dCams = nullptr, ctx->dExposureScales = nullptr;
+    ctx->cams.clear(), ctx->exposureScales.clear();
+    YC_TRY(rt::alloc(reinterpret_cast<void**>(&ctx->dCams), n * sizeof(YcCamera)));
+    YC_TRY(rt::alloc(reinterpret_cast<void**>(&ctx->dExposureScales), n * sizeof(float)));
+  }
+  ctx->cams.assign(cams, cams + n);
+  ctx->exposureScales.resize(n);
+  for (uint32_t v = 0; v < n; v++) ctx->exposureScales[v] = std::exp2(cams[v].exposure);  // integrator.cpp:23
+  YC_TRY(rt::h2d(ctx->st, ctx->dCams, ctx->cams.data(), n * sizeof(YcCamera)));
+  YC_TRY(rt::h2d(ctx->st, ctx->dExposureScales, ctx->exposureScales.data(), n * sizeof(float)));
   return YC_OK;
 }
+
+extern "C" int yc_set_camera(yc_ctx* ctx, const YcCamera* cam) { return yc_set_cameras(ctx, cam, 1); }
 
 static int ensureWaveStorage(yc_ctx* ctx) {
   if (!ctx->waveAllocs.empty()) return YC_OK;
@@ -975,7 +1012,7 @@ static uint32_t roundUpPow2(uint32_t v) {  // math_base.hpp:164-170
 
 // The AOV sums of the frame `ctx->frame` describes, allocated for its size and cleared.
 static int prepareAovPlanes(yc_ctx* ctx) {
-  const size_t texels = size_t(ctx->frame.width) * ctx->frame.height;
+  const size_t texels = frameTexels(ctx);
   if (ctx->aovTexels != texels) {
     freeAovPlanes(ctx);
     const char* e = nullptr;
@@ -1023,49 +1060,60 @@ extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   if (!ctx || !f) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->hasScene) return fail(ctx, YC_ERR_NO_SCENE, "yc_begin_frame before yc_upload_scene");
-  if (!ctx->hasCamera) return fail(ctx, YC_ERR_STATE, "yc_begin_frame before yc_set_camera");
+  if (ctx->cams.empty()) return fail(ctx, YC_ERR_STATE, "yc_begin_frame before yc_set_camera");
   if (f->width == 0 || f->height == 0 || f->width > 65535 || f->height > 65535 || f->tileSize == 0 ||
       f->totalSamples == 0 || f->estimator > YC_ESTIMATOR_GMONB || f->tonemap > YC_TONEMAP_AGX_PUNCHY)
     return fail(ctx, YC_ERR_INVALID, "bad frame description");
+  // the frame's view count is fixed here, from the cameras set now
+  const uint32_t views = uint32_t(ctx->cams.size());
+  const size_t texels = frameTexels(*f, views);
+  if (texels > 0xffffffffull) return fail(ctx, YC_ERR_INVALID, "frame of %u views of %ux%u: more than 2^32 texels", views, f->width, f->height);
   const uint32_t shardCount = f->shardCount ? f->shardCount : 1;
   if (f->shardIndex >= shardCount) return fail(ctx, YC_ERR_INVALID, "shardIndex >= shardCount");
   YC_TRY(rt::sync(ctx->st));
   int rc = ensureWaveStorage(ctx);
   if (rc != YC_OK) return rc;
   // same geometry as the previous frame: keep the allocations and the pixel list, just clear
-  const bool sameLayout = ctx->dHdr && ctx->frame.width == f->width && ctx->frame.height == f->height &&
+  const bool sameLayout = ctx->dHdr && ctx->frame.width == f->width && ctx->frame.height == f->height && ctx->views == views &&
                           ctx->frame.tileSize == f->tileSize && ctx->frame.shardIndex == f->shardIndex &&
                           ctx->frame.shardCount == shardCount;
   ctx->inFrame = false;
-  const size_t frameTexels = size_t(f->width) * f->height;
   if (!sameLayout) {
     // a failure part-way must not leave a half-allocated frame that the next call's sameLayout test accepts:
     // the descriptor is committed only after every allocation succeeded
     freeFrame(ctx);
     ctx->frame = YcFrameDesc{};
-    // tile list as TileRenderer::renderImpl builds it (tile-renderer.hpp:127-144), sharded by index
+    ctx->views = 0;
+    // tile list as TileRenderer::renderImpl builds it (tile-renderer.hpp:127-144), once per view, sharded by index over
+    // all views
     ctx->pixels.clear();
+    ctx->pixelViews.clear();
     const uint32_t ts = f->tileSize;
     const uint32_t tilesX = (f->width + ts - 1) / ts, tilesY = (f->height + ts - 1) / ts;
-    for (uint32_t ty = 0; ty < tilesY; ty++)
-      for (uint32_t tx = 0; tx < tilesX; tx++) {
-        const uint32_t index = ty * tilesX + tx;
-        if (index % shardCount != f->shardIndex) continue;
-        const uint32_t x0 = tx * ts, y0 = ty * ts;
-        const uint32_t tw = std::min(ts, f->width - x0), th = std::min(ts, f->height - y0);
-        for (uint32_t y = 0; y < th; y++)
-          for (uint32_t x = 0; x < tw; x++) ctx->pixels.push_back((x0 + x) | ((y0 + y) << 16));
-      }
+    for (uint32_t v = 0; v < views; v++)
+      for (uint32_t ty = 0; ty < tilesY; ty++)
+        for (uint32_t tx = 0; tx < tilesX; tx++) {
+          const uint64_t index = (uint64_t(v) * tilesY + ty) * tilesX + tx;
+          if (index % shardCount != f->shardIndex) continue;
+          const uint32_t x0 = tx * ts, y0 = ty * ts;
+          const uint32_t tw = std::min(ts, f->width - x0), th = std::min(ts, f->height - y0);
+          for (uint32_t y = 0; y < th; y++)
+            for (uint32_t x = 0; x < tw; x++) ctx->pixels.push_back((x0 + x) | ((y0 + y) << 16));
+          ctx->pixelViews.insert(ctx->pixelViews.end(), size_t(tw) * th, uint16_t(v));
+        }
     const size_t nPixNew = ctx->pixels.size();
     ctx->bucketCapacity = std::max<size_t>(nPixNew, 1);
     const char* e = nullptr;
     void* p = nullptr;
     if (!e && !(e = rt::alloc(&p, std::max<size_t>(nPixNew, 1) * 4))) ctx->dPixels = static_cast<uint32_t*>(p);
     if (!e && !(e = rt::alloc(&p, std::max<size_t>(nPixNew, 1) * 4))) ctx->dPixelsScratch = static_cast<uint32_t*>(p);
-    if (!e && !(e = rt::alloc(&p, frameTexels * sizeof(float4)))) ctx->dHdr = static_cast<float4*>(p);
-    if (!e && !(e = rt::alloc(&p, frameTexels * sizeof(float4)))) ctx->dLdr = static_cast<float4*>(p);
+    if (!e && !(e = rt::alloc(&p, std::max<size_t>(nPixNew, 1) * 2))) ctx->dPixelViews = static_cast<uint16_t*>(p);
+    if (!e && !(e = rt::alloc(&p, std::max<size_t>(nPixNew, 1) * 2))) ctx->dPixelViewsScratch = static_cast<uint16_t*>(p);
+    if (!e && !(e = rt::alloc(&p, texels * sizeof(float4)))) ctx->dHdr = static_cast<float4*>(p);
+    if (!e && !(e = rt::alloc(&p, texels * sizeof(float4)))) ctx->dLdr = static_cast<float4*>(p);
     if (!e && !(e = rt::alloc(&p, ctx->bucketCapacity * kMaxBuckets * sizeof(float4)))) ctx->dBuckets = static_cast<float4*>(p);
     if (!e) e = rt::h2d(ctx->st, ctx->dPixels, ctx->pixels.data(), nPixNew * 4);
+    if (!e) e = rt::h2d(ctx->st, ctx->dPixelViews, ctx->pixelViews.data(), nPixNew * 2);
     if (e) {
       freeFrame(ctx);
       return fail(ctx, YC_ERR_CUDA, "yc_begin_frame: %s", e);
@@ -1074,6 +1122,7 @@ extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   }
   ctx->frame = *f;
   ctx->frame.shardCount = shardCount;
+  ctx->views = views;
   ctx->frameRendered = false;
   if (ctx->aovs)
     if (const int arc = prepareAovPlanes(ctx)) return arc;
@@ -1083,8 +1132,8 @@ extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
     YC_TRY(rt::zero(ctx->st, ctx->dBuckets, ctx->bucketCapacity * kMaxBuckets * sizeof(float4)));
     ctx->bucketsDirty = false;
   }
-  YC_TRY(rt::zero(ctx->st, ctx->dHdr, frameTexels * sizeof(float4)));
-  YC_TRY(rt::zero(ctx->st, ctx->dLdr, frameTexels * sizeof(float4)));
+  YC_TRY(rt::zero(ctx->st, ctx->dHdr, texels * sizeof(float4)));
+  YC_TRY(rt::zero(ctx->st, ctx->dLdr, texels * sizeof(float4)));
   YC_TRY(rt::zero(ctx->st, ctx->dCounters, sizeof(Counters)));
   YC_TRY(rt::sync(ctx->st));
   ctx->launches = 0;
@@ -1138,11 +1187,11 @@ static int issueBounce(yc_ctx* ctx, Lane& L) {
 }
 
 template <bool ALPHA>
-static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, uint32_t sampleOffset, uint32_t waveSamples,
+static int renderChunks(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dViews, uint32_t nPixCall, uint32_t sampleOffset, uint32_t waveSamples,
                         uint32_t m, uint32_t bucketShard, uint32_t bucketShardCount) {
   const YcFrameDesc& f = ctx->frame;
   WaveParams w{};
-  w.cam = ctx->cam;
+  w.cams = ctx->dCams;
   // SobolSampler ctor (sampler.hpp:74-82) as TileRenderer calls it: (totalSamples, {tileSize, tileSize})
   w.smp.log2spp = log2IntU(f.totalSamples);
   w.smp.nBase4Digits = log2IntU(roundUpPow2(f.tileSize)) + (w.smp.log2spp + 1) / 2;
@@ -1152,7 +1201,7 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
   memcpy(w.bg, f.background, sizeof w.bg);
   w.maxDepth = ctx->opts.maxDepth;
   w.pixelList = dList;
-  const float exposureScale = std::exp2(ctx->cam.exposure);  // integrator.cpp:23
+  w.pixelViews = dViews;
 
   // chunk list: pixel blocks x sample groups, each at most one lane's capacity of paths
   // Bucket sharding (bucketShardCount = G > 1): the wave's work is cut into units (estimator bucket b, pixel class c)
@@ -1293,11 +1342,11 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
       PathState acc = L.ps;
       acc.L = L.Lbuf[f.buf];
       rt::launchFor(L.side, f.nPix,
-                    AccumulateK{acc, ctx->dBuckets, ctx->bucketCapacity, f.pixBase, f.nPix, f.K, f.sDone, f.stride, m, ctx->frame.estimator,
-                                exposureScale});
+                    AccumulateK{acc, ctx->dBuckets, ctx->bucketCapacity, dViews, ctx->dExposureScales, f.pixBase, f.nPix, f.K, f.sDone,
+                                f.stride, m, ctx->frame.estimator});
       if (ctx->aovs) {
-        rt::launchFor(L.side, f.nPix, AovAccumulateK{L.aov[f.buf], dList, ctx->dAovSum, ctx->dAovCount, ctx->aovTexels, f.pixBase, f.nPix,
-                                                     f.K, ctx->frame.width});
+        rt::launchFor(L.side, f.nPix, AovAccumulateK{L.aov[f.buf], dList, dViews, ctx->dAovSum, ctx->dAovCount, ctx->aovTexels, f.pixBase,
+                                                     f.nPix, f.K, ctx->frame.width, ctx->frame.height});
         ctx->launches++;
       }
       rt::eventRecord(L.side, L.evSide[f.buf]);
@@ -1355,22 +1404,41 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, u
   return YC_OK;
 }
 
-// Pixel list of a call: the whole shard, or its intersection with `px` (uploaded to the scratch list).
-static int wavePixels(yc_ctx* ctx, YcRect px, const uint32_t** dList, uint32_t* nPixCall) {
+// Rows of the frame: its views stacked (YcRect arguments are in these coordinates).
+static uint32_t frameRows(const yc_ctx* ctx) { return ctx->frame.height * ctx->views; }
+static bool wholeFrame(const yc_ctx* ctx, YcRect px) {
+  return px.x == 0 && px.y == 0 && px.w == ctx->frame.width && px.h == frameRows(ctx);
+}
+
+// The frame's view count was fixed by yc_begin_frame: a wave with another camera count set since is refused.
+static int checkViews(yc_ctx* ctx) {
+  if (ctx->cams.size() != ctx->views)
+    return fail(ctx, YC_ERR_STATE, "%zu cameras set, the frame has %u views (set them before yc_begin_frame)", ctx->cams.size(),
+                ctx->views);
+  return YC_OK;
+}
+
+// Pixel list of a call: the whole shard, or its intersection with `px` (uploaded to the scratch lists).
+static int wavePixels(yc_ctx* ctx, YcRect px, const uint32_t** dList, const uint16_t** dViews, uint32_t* nPixCall) {
   const YcFrameDesc& f = ctx->frame;
-  if (uint64_t(px.x) + px.w > f.width || uint64_t(px.y) + px.h > f.height)
+  if (uint64_t(px.x) + px.w > f.width || uint64_t(px.y) + px.h > frameRows(ctx))
     return fail(ctx, YC_ERR_INVALID, "pixel rectangle outside the frame");
   *dList = ctx->dPixels;
+  *dViews = ctx->dPixelViews;
   *nPixCall = uint32_t(ctx->pixels.size());
-  if (!(px.x == 0 && px.y == 0 && px.w == f.width && px.h == f.height)) {
+  if (!wholeFrame(ctx, px)) {
     std::vector<uint32_t> sub;
-    for (uint32_t v : ctx->pixels) {
-      const uint32_t x = v & 0xffffu, y = v >> 16;
-      if (x >= px.x && x < px.x + px.w && y >= px.y && y < px.y + px.h) sub.push_back(v);
+    std::vector<uint16_t> subViews;
+    for (size_t i = 0; i < ctx->pixels.size(); i++) {
+      const uint32_t v = ctx->pixels[i];
+      const uint32_t x = v & 0xffffu, y = ctx->pixelViews[i] * f.height + (v >> 16);  // stacked row
+      if (x >= px.x && x < px.x + px.w && y >= px.y && y < px.y + px.h) sub.push_back(v), subViews.push_back(ctx->pixelViews[i]);
     }
     *nPixCall = uint32_t(sub.size());
     YC_TRY(rt::h2d(ctx->st, ctx->dPixelsScratch, sub.data(), sub.size() * 4));
+    YC_TRY(rt::h2d(ctx->st, ctx->dPixelViewsScratch, subViews.data(), subViews.size() * 2));
     *dList = ctx->dPixelsScratch;
+    *dViews = ctx->dPixelViewsScratch;
   }
   return YC_OK;
 }
@@ -1410,16 +1478,16 @@ static int settleWaves(yc_ctx* ctx) {
 }
 
 // The sample loop of a wave (Integrator::render, integrator.cpp:5-28) into the estimator buckets.
-static int accumulateWave(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, uint32_t sampleOffset, uint32_t waveSamples,
+static int accumulateWave(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dViews, uint32_t nPixCall, uint32_t sampleOffset, uint32_t waveSamples,
                           uint32_t bucketShard, uint32_t bucketShardCount) {
   const uint32_t m = waveBuckets(ctx->frame, waveSamples);
   ctx->bucketsDirty = true;
-  return ctx->ds.hasAlpha ? renderChunks<true>(ctx, dList, nPixCall, sampleOffset, waveSamples, m, bucketShard, bucketShardCount)
-                          : renderChunks<false>(ctx, dList, nPixCall, sampleOffset, waveSamples, m, bucketShard, bucketShardCount);
+  return ctx->ds.hasAlpha ? renderChunks<true>(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, m, bucketShard, bucketShardCount)
+                          : renderChunks<false>(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, m, bucketShard, bucketShardCount);
 }
 
 // Estimator value of the wave + finishTile's blend and tonemap (tile-renderer.hpp:220-239).
-static void finalizeWave(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, uint32_t waveSamples, uint32_t takenBefore) {
+static void finalizeWave(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dViews, uint32_t nPixCall, uint32_t waveSamples, uint32_t takenBefore) {
   const YcFrameDesc& f = ctx->frame;
   const uint32_t takenAfter = takenBefore + waveSamples;
   const float wCurrent = float(takenBefore) / float(takenAfter), wWave = float(waveSamples) / float(takenAfter);
@@ -1427,10 +1495,10 @@ static void finalizeWave(yc_ctx* ctx, const uint32_t* dList, uint32_t nPixCall, 
   if (ctx->comm && ctx->comm->direct) {
     Comm& c = *ctx->comm;
     // the copy the next yc_comm_reduce_frames publishes (noteWave has marked it stale if this wave is a partial one)
-    if (dList == ctx->dPixels && !c.stale && c.frameTexels == size_t(f.width) * f.height) hdrRoot = c.hdrAll[c.epoch & 1u], ldrRoot = c.ldrAll[c.epoch & 1u];
+    if (dList == ctx->dPixels && !c.stale && c.frameTexels == frameTexels(ctx)) hdrRoot = c.hdrAll[c.epoch & 1u], ldrRoot = c.ldrAll[c.epoch & 1u];
   }
   rt::launchFor(ctx->st, nPixCall,
-                FinalizeK{dList, ctx->dBuckets, ctx->bucketCapacity, ctx->dHdr, ctx->dLdr, hdrRoot, ldrRoot, f.width,
+                FinalizeK{dList, dViews, ctx->dBuckets, ctx->bucketCapacity, ctx->dHdr, ctx->dLdr, hdrRoot, ldrRoot, f.width, f.height,
                           waveBuckets(f, waveSamples), f.estimator, waveSamples, f.tonemap, wCurrent, wWave});
   rt::eventRecord(ctx->st, ctx->evFinal);
   ctx->launches++;
@@ -1444,28 +1512,29 @@ static void noteWave(yc_ctx* ctx, YcRect px) {
   if (!ctx->comm) return;
   Comm& c = *ctx->comm;
   c.barrierSinceFinalize = false;
-  const YcFrameDesc& f = ctx->frame;
-  if (!(px.x == 0 && px.y == 0 && px.w == f.width && px.h == f.height) || c.frameTexels != size_t(f.width) * f.height) c.stale = true;
+  if (!wholeFrame(ctx, px) || c.frameTexels != frameTexels(ctx)) c.stale = true;
 }
 
 // One wave: the sample loop into the buckets, then estimator + blend + tonemap.  Chains behind waves that are still in
 // flight (ctx->wavesPending) and leaves this one in flight.
 static int issueWave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset, uint32_t waveSamples, uint32_t takenBefore) {
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_render_wave before yc_begin_frame");
+  if (const int vrc = checkViews(ctx)) return vrc;
   ctx->frameRendered = true;
   noteWave(ctx, px);
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
+  const uint16_t* dViews;
   uint32_t nPixCall;
-  if (const int prc = wavePixels(ctx, px, &dList, &nPixCall)) return prc;
+  if (const int prc = wavePixels(ctx, px, &dList, &dViews, &nPixCall)) return prc;
   if (nPixCall == 0) return YC_OK;
   if (!ctx->wavesPending) rt::eventRecord(ctx->st, ctx->ev0);
-  const int rc = accumulateWave(ctx, dList, nPixCall, sampleOffset, waveSamples, 0, 1);
+  const int rc = accumulateWave(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, 0, 1);
   if (rc != YC_OK) {
     ctx->wavesPending = true;  // whatever was issued is waited for by the next entry point
     return rc;
   }
-  finalizeWave(ctx, dList, nPixCall, waveSamples, takenBefore);
+  finalizeWave(ctx, dList, dViews, nPixCall, waveSamples, takenBefore);
   rt::eventRecord(ctx->st, ctx->ev1);
   ctx->wavesPending = true;
   return YC_OK;
@@ -1496,17 +1565,19 @@ extern "C" int yc_accumulate_wave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset,
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_accumulate_wave before yc_begin_frame");
+  if (const int vrc = checkViews(ctx)) return vrc;
   if (bucketShardCount == 0 || bucketShard >= bucketShardCount) return fail(ctx, YC_ERR_INVALID, "bucket shard out of range");
   // a pixel's samples would be split over the participants, and its AOV sums would lose their order
   if (ctx->aovs && bucketShardCount > 1) return fail(ctx, YC_ERR_UNSUPPORTED, "AOVs with bucket sharding");
   ctx->frameRendered = true;
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
+  const uint16_t* dViews;
   uint32_t nPixCall;
-  if (const int prc = wavePixels(ctx, px, &dList, &nPixCall)) return prc;
+  if (const int prc = wavePixels(ctx, px, &dList, &dViews, &nPixCall)) return prc;
   if (nPixCall == 0) return YC_OK;
   rt::eventRecord(ctx->st, ctx->ev0);
-  const int rc = accumulateWave(ctx, dList, nPixCall, sampleOffset, waveSamples, bucketShard, bucketShardCount);
+  const int rc = accumulateWave(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, bucketShard, bucketShardCount);
   if (rc != YC_OK) return rc;
   return endTimedRegion(ctx);
 }
@@ -1515,14 +1586,16 @@ extern "C" int yc_finalize_wave(yc_ctx* ctx, YcRect px, uint32_t waveSamples, ui
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_finalize_wave before yc_begin_frame");
+  if (const int vrc = checkViews(ctx)) return vrc;
   noteWave(ctx, px);
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
+  const uint16_t* dViews;
   uint32_t nPixCall;
-  if (const int prc = wavePixels(ctx, px, &dList, &nPixCall)) return prc;
+  if (const int prc = wavePixels(ctx, px, &dList, &dViews, &nPixCall)) return prc;
   if (nPixCall == 0) return YC_OK;
   rt::eventRecord(ctx->st, ctx->ev0);
-  finalizeWave(ctx, dList, nPixCall, waveSamples, takenBefore);
+  finalizeWave(ctx, dList, dViews, nPixCall, waveSamples, takenBefore);
   return endTimedRegion(ctx);
 }
 
@@ -1568,7 +1641,7 @@ extern "C" int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* 
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_resolve before yc_begin_frame");
-  const size_t bytes = size_t(ctx->frame.width) * ctx->frame.height * sizeof(float4);
+  const size_t bytes = frameTexels(ctx) * sizeof(float4);
   if (hdrRGBA) YC_TRY(rt::d2h(ctx->st, hdrRGBA, ctx->dHdr, bytes));
   if (ldrRGBA) YC_TRY(rt::d2h(ctx->st, ldrRGBA, ctx->dLdr, bytes));
   return readStats(ctx, stats);
@@ -1599,7 +1672,7 @@ extern "C" int yc_frame_device_ptrs(yc_ctx* ctx, void** hdr, void** ldr, size_t*
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "no frame");
   if (hdr) *hdr = ctx->dHdr;
   if (ldr) *ldr = ctx->dLdr;
-  if (bytes) *bytes = size_t(ctx->frame.width) * ctx->frame.height * sizeof(float4);
+  if (bytes) *bytes = frameTexels(ctx) * sizeof(float4);
   return YC_OK;
 }
 
@@ -1607,7 +1680,7 @@ extern "C" int yc_retonemap(yc_ctx* ctx) {
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "no frame");
-  rt::launchFor(ctx->st, ctx->frame.width * ctx->frame.height, RetonemapK{ctx->dHdr, ctx->dLdr, ctx->frame.tonemap});
+  rt::launchFor(ctx->st, uint32_t(frameTexels(ctx)), RetonemapK{ctx->dHdr, ctx->dLdr, ctx->frame.tonemap});
   ctx->launches++;
   YC_TRY(rt::sync(ctx->st));
   YC_TRY(rt::lastError());
@@ -1837,7 +1910,7 @@ struct PrimaryRayK {
     Sampler smp;
     smp.start(w.smp, px, py, s);
     V3 o, d;
-    primaryRay(w.cam, smp, px, py, o, d);
+    primaryRay(w.cams[w.pixelViews[w.pixBase + i % w.nPix]], smp, px, py, o, d);
     YcRay r;
     r.o[0] = o.x, r.o[1] = o.y, r.o[2] = o.z, r.tmin = kTMin;
     r.d[0] = d.x, r.d[1] = d.y, r.d[2] = d.z, r.tmax = INFINITY;
@@ -1849,15 +1922,17 @@ extern "C" int yc_generate_primary_rays(yc_ctx* ctx, uint32_t sampleOffset, uint
   if (!ctx || !raysDev) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_generate_primary_rays before yc_begin_frame");
+  if (const int vrc = checkViews(ctx)) return vrc;
   const YcFrameDesc& f = ctx->frame;
   WaveParams w{};
-  w.cam = ctx->cam;
+  w.cams = ctx->dCams;
   w.smp.log2spp = log2IntU(f.totalSamples);
   w.smp.nBase4Digits = log2IntU(roundUpPow2(f.tileSize)) + (w.smp.log2spp + 1) / 2;
   w.smp.scrambler = ctx->opts.scrambler;
   w.smp.kind = ctx->opts.sampler;
   w.smp.strata = uint32_t(std::ceil(std::sqrt(double(f.totalSamples))));  // StratifiedSampler ctor, sampler.hpp:49-51
   w.pixelList = ctx->dPixels;
+  w.pixelViews = ctx->dPixelViews;
   w.pixBase = 0, w.nPix = uint32_t(ctx->pixels.size()), w.s0 = sampleOffset;
   const uint64_t n = uint64_t(w.nPix) * spp;
   if (n > 0xffffffffull) return fail(ctx, YC_ERR_INVALID, "too many rays");
@@ -2134,7 +2209,7 @@ static int reduceFrames(yc_ctx* ctx, int root, bool async) {
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "no frame");
   Comm& c = *ctx->comm;
   if (root < 0 || root >= c.world) return fail(ctx, YC_ERR_INVALID, "bad root");
-  const size_t texels = size_t(ctx->frame.width) * ctx->frame.height;
+  const size_t texels = frameTexels(ctx);
   if (async && ctx->wavesPending && c.direct && !c.stale && c.nccl && c.frameTexels == texels && c.root == root) {
     // Chained behind waves in flight: the barrier is enqueued on the main stream after the wave's finalize kernel and
     // nobody waits for it here.  (The stores of wave k + 2 into this copy are issued after barrier k + 1, which the
@@ -2161,7 +2236,8 @@ static int reduceFrames(yc_ctx* ctx, int root, bool async) {
       bool barrier = !c.barrierSinceFinalize;
       if (c.stale) {
         rt::launchFor(ctx->st, uint32_t(ctx->pixels.size()),
-                      PushFramesK{ctx->dPixels, ctx->dHdr, ctx->dLdr, c.hdrAll[k], c.ldrAll[k], ctx->frame.width});
+                      PushFramesK{ctx->dPixels, ctx->dPixelViews, ctx->dHdr, ctx->dLdr, c.hdrAll[k], c.ldrAll[k],
+                                  ctx->frame.width, ctx->frame.height});
         ctx->launches++;
         c.stale = false;
         barrier = true;

@@ -292,7 +292,8 @@ struct Shard {
 struct yr_renderer {
   YrSettings s{};
   const YcScene* flat = nullptr;  // the scene (owned by a ys_scene or by the caller of yr_create_flat)
-  YcCamera cam{};
+  std::vector<YcCamera> cams;     // one per view (yr_set_cameras)
+  uint32_t frameViews = 1;        // the view count of the current (or last) render's frame
   std::vector<Shard> shards;      // 1, or one per GPU of yr_create_multi
   // sharding across `world` participants: the local shards are ranks rank0 .. rank0 + shards.size() - 1
   uint32_t rank0 = 0, world = 1;
@@ -352,7 +353,7 @@ static int newRenderer(const YrSettings* settings, const YcScene* flat, const Yc
   if (!r) return YC_ERR_INVALID;
   r->s = *settings;
   r->flat = flat;
-  r->cam = *camera;
+  r->cams.assign(camera, camera + 1);
   *out = r;
   return YC_OK;
 }
@@ -468,12 +469,17 @@ extern "C" int yr_set_frame_target(yr_renderer* r, float* ldrRGBA) {
   r->target = ldrRGBA;
   return YC_OK;
 }
-extern "C" int yr_set_camera(yr_renderer* r, const YcCamera* cam) {
-  if (!r || !cam) return YC_ERR_INVALID;
+extern "C" int yr_set_cameras(yr_renderer* r, const YcCamera* cams, uint32_t n) {
+  if (!r || !cams || n == 0 || n > 65535) return YC_ERR_INVALID;
   if (r->worker.joinable()) r->worker.join();
-  r->cam = *cam;
+  r->cams.assign(cams, cams + n);
   return YC_OK;
 }
+
+extern "C" int yr_set_camera(yr_renderer* r, const YcCamera* cam) { return yr_set_cameras(r, cam, 1); }
+
+// Rows of the current (or last) render's frame: its views stacked.
+static uint32_t frameRows(const yr_renderer* r) { return r->s.height * r->frameViews; }
 
 extern "C" yc_ctx* yr_context(yr_renderer* r) { return r && !r->shards.empty() ? r->shards[0].ctx : nullptr; }
 extern "C" const char* yr_last_error(const yr_renderer* r) { return r ? r->err.c_str() : "null renderer"; }
@@ -513,6 +519,7 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
   using clock = std::chrono::high_resolution_clock;
   if (!r->flat) return rfail(r, YC_ERR_NO_SCENE, "no scene (reference: `if (!scene) return;`, integrator.cpp:6)");
   const bool buckets = r->comm && r->s.sharding == YR_SHARD_BUCKETS;
+  r->frameViews = uint32_t(r->cams.size());
   int rc = onShards(r, [&](size_t i) {
     Shard& sh = r->shards[i];
     int e;
@@ -520,7 +527,7 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
       if ((e = yc_upload_scene(sh.ctx, r->flat)) != YC_OK) return e;
       sh.sceneUploaded = true;
     }
-    if ((e = yc_set_camera(sh.ctx, &r->cam)) != YC_OK) return e;
+    if ((e = yc_set_cameras(sh.ctx, r->cams.data(), uint32_t(r->cams.size()))) != YC_OK) return e;
     YcFrameDesc f{};
     f.width = r->s.width, f.height = r->s.height;
     f.totalSamples = r->s.samples, f.tileSize = r->s.tileSize;
@@ -544,7 +551,7 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
   data.totalSamples = total;
   uint64_t raysBefore = 0;
   bool aborted = false;
-  const YcRect full{0, 0, r->s.width, r->s.height};
+  const YcRect full{0, 0, r->s.width, frameRows(r)};
   while (waveSamples > 0) {
     const auto w0 = clock::now();
     const uint32_t taken = uint32_t(total - remaining), ws = uint32_t(waveSamples);
@@ -589,20 +596,22 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
     const double waveMs = std::chrono::duration<double, std::milli>(now - w0).count();
     if (r->tileCb) {
       // the reference reports every tile of every wave (finishTile, tile-renderer.hpp:205-262); a wave here covers the
-      // frame at once, so the tiles are reported after it, in tile-list order, with the wave's rays and time shared
-      // out by pixel count
+      // frame at once, so the tiles are reported after it, in tile-list order (view after view, in stacked
+      // coordinates), with the wave's rays and time shared out by pixel count
       const uint32_t ts = r->s.tileSize, tilesX = (r->s.width + ts - 1) / ts, tilesY = (r->s.height + ts - 1) / ts;
-      const double px = double(r->s.width) * r->s.height;
-      for (uint32_t ty = 0; ty < tilesY; ty++)
-        for (uint32_t tx = 0; tx < tilesX; tx++) {
-          YrTileData td{};
-          td.x = tx * ts, td.y = ty * ts;
-          td.w = std::min(ts, r->s.width - td.x), td.h = std::min(ts, r->s.height - td.y);
-          td.index = uint64_t(ty) * tilesX + tx, td.total = uint64_t(tilesX) * tilesY;
-          const double share = double(td.w) * td.h / px;
-          td.rays = uint64_t(double(waveRays) * share), td.timeMs = waveMs * share;
-          r->tileCb(&data, &td, r->tileUser);
-        }
+      const uint32_t views = r->frameViews;
+      const double px = double(r->s.width) * frameRows(r);
+      for (uint32_t v = 0; v < views; v++)
+        for (uint32_t ty = 0; ty < tilesY; ty++)
+          for (uint32_t tx = 0; tx < tilesX; tx++) {
+            YrTileData td{};
+            td.x = tx * ts, td.y = v * r->s.height + ty * ts;
+            td.w = std::min(ts, r->s.width - td.x), td.h = std::min(ts, r->s.height - ty * ts);
+            td.index = (uint64_t(v) * tilesY + ty) * tilesX + tx, td.total = uint64_t(views) * tilesX * tilesY;
+            const double share = double(td.w) * td.h / px;
+            td.rays = uint64_t(double(waveRays) * share), td.timeMs = waveMs * share;
+            r->tileCb(&data, &td, r->tileUser);
+          }
     }
     if (r->cb) {
       YrWaveData wd{wave, waveSamples, waveRays, waveMs};
@@ -667,10 +676,10 @@ extern "C" int yr_wait(yr_renderer* r) {
 
 extern "C" int yr_write_ppm(yr_renderer* r, const char* path) {
   if (!r || !path) return YC_ERR_INVALID;
-  std::vector<float> ldr(size_t(r->s.width) * r->s.height * 4);
+  std::vector<float> ldr(size_t(r->s.width) * frameRows(r) * 4);
   int rc = readFrames(r, nullptr, ldr.data());
   if (rc != YC_OK) return rfail(r, rc, yc_last_error(r->shards[0].ctx));
-  return writePpm(path, ldr.data(), r->s.width, r->s.height) ? YC_OK : rfail(r, YC_ERR_IO, std::string("cannot write ") + path);
+  return writePpm(path, ldr.data(), r->s.width, frameRows(r)) ? YC_OK : rfail(r, YC_ERR_IO, std::string("cannot write ") + path);
 }
 
 extern "C" int yr_read(yr_renderer* r, float* hdrRGBA, float* ldrRGBA, YcStats* stats) {
