@@ -270,7 +270,8 @@ typedef struct YcStats {
                                (mis-integrator.cpp:22,126) */
   uint64_t raysExtend;      /* closest-hit rays traced */
   uint64_t raysShadow;      /* any-hit rays traced */
-  uint64_t samples;         /* pixel samples taken */
+  uint64_t samples;         /* pixel samples taken since begin_frame, counted while adaptive sampling is on (ΣS of
+                               yc_resolve_adaptive); 0 otherwise */
   uint64_t kernelLaunches;  /* CUDA kernels launched by this context since begin_frame */
   double gpuMs;             /* CUDA-event time spent inside yc_render_wave since begin_frame */
   uint64_t boxTests, triTests; /* only filled by counting traces (yc_trace with YC_TRACE_COUNT): the reference-order
@@ -282,6 +283,14 @@ typedef struct YcStats {
   uint64_t hitsShaded;      /* queue entries those launches shaded */
   double commMs;            /* CUDA-event time of the yc_comm_* data collectives since begin_frame */
 } YcStats;
+
+/* Adaptive sampling parameters (yc_set_adaptive, yr_set_adaptive). */
+typedef struct YcAdaptive {
+  float threshold;     /* a pixel stops once every e of its neighbourhood is below it; finite, >= 0 (0: none ever stops) */
+  uint32_t minSamples; /* samples a pixel takes at least */
+  float lumaFloor;     /* the denominator's floor: finite, > 0 */
+  uint32_t reserved;
+} YcAdaptive;
 
 typedef struct YcRay { float o[3], tmin, d[3], tmax; } YcRay;
 
@@ -396,6 +405,42 @@ int yc_resolve(yc_ctx* ctx, float* hdrRGBA, float* ldrRGBA, YcStats* stats);
  *                      (repeated calls count nothing twice); yc_resolve_aovs_combined copies them out on the root. */
 int yc_enable_aovs(yc_ctx* ctx, int enable);
 int yc_resolve_aovs(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA);
+/* Adaptive sampling: a pixel stops taking samples once its noise estimate, and its neighbours', is below a threshold.
+ * Per texel, over the samples it has taken since yc_begin_frame:
+ *   S  the samples taken in the wave calls that finalized (an aborted call adds none).
+ *   n, s1, s2  over the samples the frame's estimator accepts (GMoN: no negative channel; all: no NaN), with Y = luma
+ *      (0.2126 r + 0.7152 g + 0.0722 b, in that order) of the exposure-scaled sample the estimator adds: n is their
+ *      count, s1 = ΣY and s2 = Σ(Y·Y), float32 from +0, one sample at a time in sample order (AccumulateK's order).
+ *   e  after each finalizing wave call (yc_render_wave[_async]), for every pixel of the call still sampling:
+ *      +inf if n < 2; otherwise mean = s1 / n, var = (s2 - s1·mean) / (n - 1), var = 0 unless var > 0, and
+ *      e = sqrt(var / n) / (mean > lumaFloor ? mean : lumaFloor).  float32, IEEE division and sqrt, no contraction.
+ *      Texels never sampled read e = +inf.
+ *   Stop rule, after e: a pixel of the call stops when S >= minSamples and every e of its neighbourhood is < threshold.
+ *      The neighbourhood is the pixel and its 8 neighbours that lie in the same view and the same reference tile (so the
+ *      decision never needs another shard's pixels and is the same for any shard count).  The comparison is strict:
+ *      NaN never stops a pixel, threshold = 0 stops none.
+ *   A stopped pixel takes no further sample in the frame: every later wave call, whatever its rectangle, skips it, so
+ *   its HDR, LDR, AOV sums and S keep the values of the wave it stopped at — bit for bit the frame the same calls give
+ *   without adaptive sampling after that wave.  Pixels still sampling get exactly the bits of that render.
+ *   Scheduling: a wave call starts only after the previous one's stop test (the host reads the count of pixels still
+ *   sampling to cut the wave), so yc_render_wave_async overlaps less; the results are the same bits.
+ *   Abort: S and e keep describing the waves finished before an aborted call; its partly added n, s1, s2 stay until the
+ *   next yc_begin_frame, like the half-filled estimator buckets (yc_set_abort_flag).
+ *
+ *   yc_set_adaptive    params (NULL: off) for the frames that follow: valid before yc_begin_frame or before the frame's
+ *                      first wave, YC_ERR_STATE later; YC_ERR_INVALID for a threshold that is negative or not finite or
+ *                      a lumaFloor that is not finite and > 0.  Per texel of the frame it allocates 32 bytes (40 once
+ *                      yc_comm_reduce_adaptive ran), per pixel of the shard 32.  While it is on, yc_accumulate_wave
+ *                      and yc_finalize_wave return YC_ERR_UNSUPPORTED (bucket sharding would split a pixel's samples
+ *                      over the participants, and the sums would lose their order).
+ *   yc_resolve_adaptive  copies the planes samples (S, uint32) and error (e, float32), width·height·V texels each, and
+ *                      *activePixels, the pixels of this context still sampling (any pointer may be NULL).  YC_ERR_STATE
+ *                      when adaptive sampling is off for the frame.
+ *   yc_comm_reduce_adaptive  tile sharding, collective: combines every participant's planes into the root's, as
+ *                      yc_comm_reduce_aovs does (bit-identical to one context's planes); yc_resolve_adaptive_combined
+ *                      copies them out on the root. */
+int yc_set_adaptive(yc_ctx* ctx, const YcAdaptive* params);
+int yc_resolve_adaptive(yc_ctx* ctx, uint32_t* samples, float* error, uint64_t* activePixels);
 /* Device pointers of the frames (for NCCL reductions by the caller); *bytes = width·height·V·4 floats. */
 int yc_frame_device_ptrs(yc_ctx* ctx, void** hdr, void** ldr, size_t* bytes);
 /* Re-run the tonemap over the whole HDR frame (after a cross-GPU sum). */
@@ -470,6 +515,9 @@ int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples);
 /* Tile sharding with AOVs (yc_enable_aovs): see there. */
 int yc_comm_reduce_aovs(yc_ctx* ctx, int root);
 int yc_resolve_aovs_combined(yc_ctx* ctx, float* albedoRGBA, float* normalDepthRGBA);
+/* Tile sharding with adaptive sampling (yc_set_adaptive): see there. */
+int yc_comm_reduce_adaptive(yc_ctx* ctx, int root);
+int yc_resolve_adaptive_combined(yc_ctx* ctx, uint32_t* samples, float* error);
 /* Control values (ray counts, abort votes): in-place sum over all participants. */
 int yc_comm_sum_u64(yc_ctx* ctx, uint64_t* values, uint32_t n);
 /* The reference's binned-SAH BVH (src/core/bvh.hpp:140-184, 273-347) built on the device, level by level: the same
@@ -641,6 +689,15 @@ int yr_enable_aovs(yr_renderer* r, int enable);
  * (yr_render_sync / yr_wait) and YC_ERR_STATE while one runs.  Tile sharding: the combined planes, on the root; other
  * ranks' buffers are left untouched, as with yr_read. */
 int yr_read_aovs(yr_renderer* r, float* albedoRGBA, float* normalDepthRGBA);
+/* Adaptive sampling for the renders that follow (yc_set_adaptive; NULL: off).  YC_ERR_INVALID for bad parameters,
+ * YC_ERR_UNSUPPORTED for YR_SHARD_BUCKETS over more than one participant, YC_ERR_STATE while a render runs.  A render
+ * ends early, as a normal completion (done callback with aborted = 0), after the first wave that leaves no pixel sampling
+ * on any participant; YrRenderData.samplesTaken is then the schedule's samples up to that wave.  The wave and tile
+ * callbacks and the frame target fire for every wave that ran. */
+int yr_set_adaptive(yr_renderer* r, const YcAdaptive* params);
+/* The samples / error planes of the last render (width*height*V texels each, either pointer may be NULL), valid once it
+ * has returned.  Tile sharding: the combined planes, on the root (combined once per render, aborted renders included). */
+int yr_read_adaptive(yr_renderer* r, uint32_t* samples, float* error);
 /* writePPM(out, renderer buffer): the tonemapped frame as a binary PPM (frontend main.cpp writes out.ppm); width x
  * (height·V) with several views. */
 int yr_write_ppm(yr_renderer* r, const char* path);

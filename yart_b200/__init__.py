@@ -318,7 +318,29 @@ class Context:
         self._ck(lib().yc_resolve_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yc_resolve_aovs")
         return albedo, nd
 
+    def set_adaptive(self, threshold=None, min_samples=0, luma_floor=1e-3):
+        """yc_set_adaptive: adaptive sampling for the frames that follow (include/yart_cuda.h has the rule); threshold
+        None switches it off."""
+        p = None if threshold is None else C.byref(capi.YcAdaptive(threshold, min_samples, luma_floor, 0))
+        self._ck(lib().yc_set_adaptive(self._h, p), "yc_set_adaptive")
+
+    def resolve_adaptive(self):
+        """(samples uint32, error float32, active pixels): the planes as (views * h, w) arrays."""
+        h, w = self.frame.height * self.views, self.frame.width
+        samples, error, active = np.empty((h, w), np.uint32), np.empty((h, w), np.float32), C.c_uint64()
+        self._ck(lib().yc_resolve_adaptive(self._h, samples.ctypes.data, error.ctypes.data, C.byref(active)), "yc_resolve_adaptive")
+        return samples, error, active.value
+
     # ---- collectives (yc_comm_*) ----
+    def comm_reduce_adaptive(self, root: int = 0):
+        self._ck(lib().yc_comm_reduce_adaptive(self._h, root), "yc_comm_reduce_adaptive")
+
+    def resolve_adaptive_combined(self):
+        h, w = self.frame.height * self.views, self.frame.width
+        samples, error = np.empty((h, w), np.uint32), np.empty((h, w), np.float32)
+        self._ck(lib().yc_resolve_adaptive_combined(self._h, samples.ctypes.data, error.ctypes.data), "yc_resolve_adaptive_combined")
+        return samples, error
+
     def comm_reduce_aovs(self, root: int = 0):
         self._ck(lib().yc_comm_reduce_aovs(self._h, root), "yc_comm_reduce_aovs")
 
@@ -413,11 +435,12 @@ class Renderer:
                  first_wave_samples=None, max_wave_samples=None, tile_size=64, max_depth=30, background=(0, 0, 0),
                  tonemap=TONEMAP_AGX, estimator=ESTIMATOR_GMON, shard_index=0, shard_count=1, device=0,
                  integrator=capi.INTEGRATOR_MIS, scrambler=capi.SCRAMBLER_FAST_OWEN, sampler=capi.SAMPLER_SOBOL,
-                 traversal=None, sharding=capi.SHARD_TILES, devices=None, dist=None, aovs=False):
+                 traversal=None, sharding=capi.SHARD_TILES, devices=None, dist=None, aovs=False, adaptive=None):
         """camera: a YcCamera, or a sequence of them: one view per camera in every frame (yr_set_cameras), and the
         frames, AOV planes, pinned buffers and frame target get a leading view axis (V, height, width, ...).
         devices=[g0, g1, ...]: one renderer over several GPUs of this process (yr_create_multi).
         aovs=True: collect the first-hit albedo / normal / depth planes (yr_enable_aovs; read_aovs()).
+        adaptive=(threshold, min_samples, luma_floor): let converged pixels stop sampling (yr_set_adaptive; read_adaptive()).
         dist=(rank, world, comm): one process per GPU (yr_create_dist); comm = the 128 bytes of comm_unique_id() from
         rank 0, or a callable collective(buf_ptr, count, dtype, root) → 0 (yr_create_dist_custom)."""
         traversal = default_traversal if traversal is None else traversal
@@ -460,6 +483,8 @@ class Renderer:
             self._frame_views = self._views
         if aovs:
             self.enable_aovs()
+        if adaptive is not None:
+            self.set_adaptive(*adaptive)
 
     def close(self):
         if self._h:
@@ -597,6 +622,20 @@ class Renderer:
         albedo, nd = np.zeros(shape, np.float32), np.zeros(shape, np.float32)
         self._ck(lib().yr_read_aovs(self._h, albedo.ctypes.data, nd.ctypes.data), "yr_read_aovs")
         return dict(albedo=albedo[..., :3].copy(), coverage=albedo[..., 3].copy(), normal=nd[..., :3].copy(), depth=nd[..., 3].copy())
+
+    def set_adaptive(self, threshold=None, min_samples=0, luma_floor=1e-3):
+        """yr_set_adaptive: a pixel stops sampling once the noise estimate of its neighbourhood is below `threshold`
+        (include/yart_cuda.h has the rule) in the renders that follow; threshold None switches it off."""
+        p = None if threshold is None else C.byref(capi.YcAdaptive(threshold, min_samples, luma_floor, 0))
+        self._ck(lib().yr_set_adaptive(self._h, p), "yr_set_adaptive")
+
+    def read_adaptive(self) -> dict:
+        """The last render's adaptive planes: dict(samples=(h, w) uint32, error=(h, w) float32) (tile sharding over
+        ranks: the combined planes on rank 0; zeros elsewhere); a leading view axis with a sequence of cameras."""
+        shape = self._shape(self._frame_views)
+        samples, error = np.zeros(shape, np.uint32), np.zeros(shape, np.float32)
+        self._ck(lib().yr_read_adaptive(self._h, samples.ctypes.data, error.ctypes.data), "yr_read_adaptive")
+        return dict(samples=samples, error=error)
 
     def write_ppm(self, path: str):
         self._ck(lib().yr_write_ppm(self._h, path.encode()), "yr_write_ppm")

@@ -60,6 +60,10 @@ class YcStats(C.Structure):
                 ("hitsShaded", u64), ("commMs", C.c_double)]
 
 
+class YcAdaptive(C.Structure):
+    _fields_ = [("threshold", f32), ("minSamples", u32), ("lumaFloor", f32), ("reserved", u32)]
+
+
 class YcRay(C.Structure):
     _fields_ = [("o", f32 * 3), ("tmin", f32), ("d", f32 * 3), ("tmax", f32)]
 
@@ -172,6 +176,10 @@ PROTOTYPES = {
     "yc_resolve_aovs": (C.c_int, [P, P, P]),
     "yc_comm_reduce_aovs": (C.c_int, [P, C.c_int]),
     "yc_resolve_aovs_combined": (C.c_int, [P, P, P]),
+    "yc_set_adaptive": (C.c_int, [P, C.POINTER(YcAdaptive)]),
+    "yc_resolve_adaptive": (C.c_int, [P, P, P, C.POINTER(u64)]),
+    "yc_comm_reduce_adaptive": (C.c_int, [P, C.c_int]),
+    "yc_resolve_adaptive_combined": (C.c_int, [P, P, P]),
     "yc_kat": (C.c_int, [P, C.c_char_p, P, C.c_size_t, P, C.c_size_t]),
     "ys_scene_load": (C.c_int, [C.c_char_p, C.POINTER(P)]),
     "ys_scene_load_bvh": (C.c_int, [C.c_char_p, u32, C.POINTER(P)]),
@@ -213,6 +221,8 @@ PROTOTYPES = {
     "yr_write_ppm": (C.c_int, [P, C.c_char_p]),
     "yr_enable_aovs": (C.c_int, [P, C.c_int]),
     "yr_read_aovs": (C.c_int, [P, P, P]),
+    "yr_set_adaptive": (C.c_int, [P, C.POINTER(YcAdaptive)]),
+    "yr_read_adaptive": (C.c_int, [P, P, P]),
     "yr_context": (P, [P]),
     "yr_last_error": (C.c_char_p, [P]),
 }

@@ -24,6 +24,7 @@
 #include "rt.cuh"
 #include "comm.cuh"
 #include "bvh_build.cuh"
+#include "scan.cuh"
 #include "trace_kernels.cuh"
 
 using namespace yb;
@@ -128,6 +129,28 @@ struct yc_ctx {
   float4 *dAovSum = nullptr, *dAov = nullptr, *dAovComm = nullptr;
   uint32_t* dAovCount = nullptr;
   bool aovCombined = false;  // this context is the root of a completed yc_comm_reduce_aovs of the current frame
+
+  // adaptive sampling (yc_set_adaptive), per texel of the frame: moments {s1, s2, n (bits), e}, samples S and the stop
+  // state (0 sampling, 1 stopped by the last stop test, 2 stopped before); per pixel of the shard: the pixels still
+  // sampling in shard-list order (two lists, the compaction writes the other), the pixels the last stop test stopped, a
+  // rectangle wave's pixels and the compaction's scan words.  Allocated with the frame while adaptive sampling is on.
+  struct PixList {
+    uint32_t* pix = nullptr;
+    uint16_t* view = nullptr;
+  };
+  bool adaptive = false;
+  YcAdaptive adParams{};
+  std::vector<void*> adAllocs;
+  size_t adTexels = 0, adPixels = 0;
+  float4* dAdMom = nullptr;
+  uint32_t *dAdS = nullptr, *dAdState = nullptr, *dAdPlanes = nullptr, *dAdComm = nullptr;  // {S, e}: resolved, combined
+  PixList adActive[2], adJust, adRect;
+  int adCur = 0;                              // adActive[adCur] is the list of pixels still sampling
+  uint32_t adActiveCount = 0, adJustCount = 0;
+  unsigned long long *dAdScan = nullptr, *dAdSums = nullptr;
+  const unsigned long long* dAdCount = nullptr;  // the last compaction's {sampling | stopped << 32}, not read back yet
+  uint64_t adSamples = 0;                     // pixel samples taken in the frame (YcStats.samples)
+  bool adCombined = false;                    // this context is the root of a completed yc_comm_reduce_adaptive
 
   // wavefront storage lives in the lanes; the ray hooks (yc_trace*) use lane 0's counters and spill area
   uint32_t* dCtr = nullptr;
@@ -483,6 +506,149 @@ struct AovResolveK {
   }
 };
 
+// ---- adaptive sampling (yc_set_adaptive; the rule is include/yart_cuda.h's) ----
+// Start of a frame: no moments, e = +inf (a texel never sampled never lets a neighbour stop).
+struct AdaptiveInitK {
+  float4* mom;
+  YB_DEV void operator()(uint32_t idx) const { mom[idx] = make_float4(0.0f, 0.0f, 0.0f, INFINITY); }
+};
+
+// After the chunk's AccumulateK, in chunk order: pixel p adds the luma of its K accepted exposure-scaled samples, and
+// their squares, in sample order.
+struct AdaptiveMomentK {
+  const float4* L;
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  const float* exposureScales;
+  float4* mom;
+  uint32_t pixBase, nPix, K, width, height, estimator;
+  YB_DEV void operator()(uint32_t p) const {
+    const uint32_t view = pixelViews[pixBase + p];
+    const size_t idx = texelIndex(pixelList[pixBase + p], view, width, height);
+    const float exposureScale = exposureScales[view];
+    float4 m = mom[idx];
+    uint32_t n = __float_as_uint(m.z);
+    for (uint32_t k = 0; k < K; k++) {
+      const float4 L4 = L[size_t(k) * nPix + p];
+      const V3 s = V3(L4.x, L4.y, L4.z) * exposureScale;
+      if (!estimatorAccepts(int(estimator), s)) continue;
+      const float y = luma(s);
+      m.x += y;
+      m.y += y * y;
+      n++;
+    }
+    m.z = __uint_as_float(n);
+    mom[idx] = m;
+  }
+};
+
+// After FinalizeK, per pixel of the call: the wave's samples count into S (only now, so that S always describes the
+// finalized frame, also after an aborted call), and e = sqrt(var / n) / max(mean, lumaFloor), +inf below two accepted
+// samples.
+struct AdaptiveErrorK {
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  float4* mom;
+  uint32_t* S;
+  uint32_t width, height, waveSamples;
+  float lumaFloor;
+  YB_DEV void operator()(uint32_t p) const {
+    const size_t idx = texelIndex(pixelList[p], pixelViews[p], width, height);
+    S[idx] += waveSamples;
+    float4 m = mom[idx];
+    const uint32_t n = __float_as_uint(m.z);
+    float e = INFINITY;
+    if (n >= 2) {
+      const float fn = float(n);
+      const float mean = __fdiv_rn(m.x, fn);
+      float var = __fdiv_rn(m.y - m.x * mean, float(n - 1));
+      if (!(var > 0.0f)) var = 0.0f;
+      e = __fdiv_rn(sqrtf(__fdiv_rn(var, fn)), mean > lumaFloor ? mean : lumaFloor);
+    }
+    m.w = e;
+    mom[idx] = m;
+  }
+};
+
+// After AdaptiveErrorK, per pixel of the call: the pixel stops once it has taken minSamples and every e of its 3x3
+// neighbourhood within its view and its reference tile is below the threshold (NaN and +inf never are).
+struct AdaptiveStopK {
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  const float4* mom;
+  const uint32_t* S;
+  uint32_t* state;
+  uint32_t width, height, tileSize, minSamples;
+  float threshold;
+  YB_DEV void operator()(uint32_t p) const {
+    const uint32_t pix = pixelList[p], view = pixelViews[p];
+    const size_t idx = texelIndex(pix, view, width, height);
+    if (S[idx] < minSamples) return;
+    const uint32_t x = pix & 0xffffu, y = pix >> 16;
+    const uint32_t x0 = x / tileSize * tileSize, y0 = y / tileSize * tileSize;
+    const uint32_t x1 = x0 + tileSize < width ? x0 + tileSize : width, y1 = y0 + tileSize < height ? y0 + tileSize : height;
+    for (uint32_t ny = y > y0 ? y - 1 : y; ny <= y + 1 && ny < y1; ny++)
+      for (uint32_t nx = x > x0 ? x - 1 : x; nx <= x + 1 && nx < x1; nx++)
+        if (!(mom[texelIndex(nx | (ny << 16), view, width, height)].w < threshold)) return;
+    state[idx] = 1u;
+  }
+};
+
+// Stable compaction of a pixel list by stop state, in three steps: AdaptiveClassK packs {sampling, just stopped} per
+// entry into one word, the scan (scan.cuh) sums them, AdaptiveScatterK moves each entry to its place in `keep` or
+// `stopped` (when given: it also marks the entry stopped before).
+struct AdaptiveClassK {
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  const uint32_t* state;
+  unsigned long long* scan;
+  uint32_t width, height;
+  YB_DEV void operator()(uint32_t i) const {
+    const uint32_t s = state[texelIndex(pixelList[i], pixelViews[i], width, height)];
+    scan[i] = (s == 0u ? 1ull : 0ull) | (s == 1u ? 1ull << 32 : 0ull);
+  }
+};
+struct AdaptiveScatterK {
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  const unsigned long long* scan;
+  uint32_t* state;
+  uint32_t *keep, *stopped;
+  uint16_t *keepViews, *stoppedViews;
+  uint32_t width, height;
+  YB_DEV void operator()(uint32_t i) const {
+    const uint32_t pix = pixelList[i], view = pixelViews[i];
+    const size_t idx = texelIndex(pix, view, width, height);
+    const uint32_t s = state[idx];
+    const unsigned long long at = scan[i];
+    if (s == 0u) {
+      const uint32_t j = uint32_t(at) - 1u;
+      keep[j] = pix, keepViews[j] = uint16_t(view);
+    } else if (s == 1u && stopped) {
+      const uint32_t j = uint32_t(at >> 32) - 1u;
+      stopped[j] = pix, stoppedViews[j] = uint16_t(view);
+      state[idx] = 2u;
+    }
+  }
+};
+
+// The planes of yc_resolve_adaptive {S, e}: every texel (pixelList null), or only the entries of a pixel list, into
+// planes cleared before (the combination over tile shards: zero outside the participant's tiles).
+struct AdaptiveResolveK {
+  const uint32_t* pixelList;
+  const uint16_t* pixelViews;
+  const float4* mom;
+  const uint32_t* S;
+  uint32_t* samples;
+  float* error;
+  uint32_t width, height;
+  YB_DEV void operator()(uint32_t i) const {
+    const size_t idx = pixelList ? texelIndex(pixelList[i], pixelViews[i], width, height) : i;
+    samples[idx] = S[idx];
+    error[idx] = mom[idx].w;
+  }
+};
+
 // Which BVH layout a traversal launch walks: the wide one when the context built it (YcOptions::traversal, scenes
 // without alpha-tested materials), unless the launch draws alpha-test samples or counts box / triangle tests (the counts
 // of the reference-order walk define the roofline's algorithmic bytes).  Kernels are picked as
@@ -757,6 +923,7 @@ extern "C" void yc_destroy(yc_ctx* ctx) {
   destroyComm(ctx);
   freeFrame(ctx);
   freeAovPlanes(ctx);
+  freeAll(ctx->adAllocs);
   freeAll(ctx->sceneAllocs);
   freeAll(ctx->waveAllocs);
   rt::release(ctx->dCams);
@@ -1056,6 +1223,61 @@ extern "C" int yc_enable_aovs(yc_ctx* ctx, int enable) {
   return YC_OK;
 }
 
+// The adaptive-sampling state of the frame `ctx->frame` describes, allocated for its size and reset: no moments, e = +inf,
+// S = 0, every pixel of the shard sampling.
+static int prepareAdaptive(yc_ctx* ctx) {
+  const size_t texels = frameTexels(ctx), nPix = std::max<size_t>(ctx->pixels.size(), 1);
+  if (ctx->adTexels != texels || ctx->adPixels != nPix) {
+    freeAll(ctx->adAllocs);
+    ctx->dAdComm = nullptr;
+    ctx->adTexels = ctx->adPixels = 0;
+    auto& own = ctx->adAllocs;
+    YC_TRY(devAlloc(own, &ctx->dAdMom, texels));
+    YC_TRY(devAlloc(own, &ctx->dAdS, texels));
+    YC_TRY(devAlloc(own, &ctx->dAdState, texels));
+    YC_TRY(devAlloc(own, &ctx->dAdPlanes, 2 * texels));
+    for (yc_ctx::PixList* l : {&ctx->adActive[0], &ctx->adActive[1], &ctx->adJust, &ctx->adRect}) {
+      YC_TRY(devAlloc(own, &l->pix, nPix));
+      YC_TRY(devAlloc(own, &l->view, nPix));
+    }
+    YC_TRY(devAlloc(own, &ctx->dAdScan, nPix));
+    YC_TRY(devAlloc(own, &ctx->dAdSums, nPix / 1024 + 64));
+    ctx->adTexels = texels, ctx->adPixels = nPix;
+  }
+  rt::launchFor(ctx->st, uint32_t(texels), AdaptiveInitK{ctx->dAdMom});
+  YC_TRY(rt::zero(ctx->st, ctx->dAdS, texels * sizeof(uint32_t)));
+  YC_TRY(rt::zero(ctx->st, ctx->dAdState, texels * sizeof(uint32_t)));
+  ctx->adCur = 0;
+  YC_TRY(rt::d2d(ctx->st, ctx->adActive[0].pix, ctx->dPixels, ctx->pixels.size() * sizeof(uint32_t)));
+  YC_TRY(rt::d2d(ctx->st, ctx->adActive[0].view, ctx->dPixelViews, ctx->pixels.size() * sizeof(uint16_t)));
+  ctx->adActiveCount = uint32_t(ctx->pixels.size()), ctx->adJustCount = 0;
+  ctx->dAdCount = nullptr;
+  ctx->adSamples = 0;
+  ctx->adCombined = false;
+  return YC_OK;
+}
+
+extern "C" int yc_set_adaptive(yc_ctx* ctx, const YcAdaptive* params) {
+  if (!ctx) return YC_ERR_INVALID;
+  if (params && !(std::isfinite(params->threshold) && params->threshold >= 0.0f && std::isfinite(params->lumaFloor) &&
+                  params->lumaFloor > 0.0f))
+    return fail(ctx, YC_ERR_INVALID, "yc_set_adaptive: threshold must be finite and >= 0, lumaFloor finite and > 0");
+  YC_ENTER(ctx);
+  if (ctx->frameRendered) return fail(ctx, YC_ERR_STATE, "yc_set_adaptive inside a frame (after its first wave)");
+  if (!params) {
+    ctx->adaptive = false;
+    return YC_OK;
+  }
+  ctx->adParams = *params;
+  // (already on in this frame: yc_begin_frame has reset the state, and no wave has run since)
+  if (ctx->inFrame && !ctx->adaptive) {
+    if (int rc = prepareAdaptive(ctx)) return rc;
+    YC_TRY(rt::sync(ctx->st));
+  }
+  ctx->adaptive = true;
+  return YC_OK;
+}
+
 extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   if (!ctx || !f) return YC_ERR_INVALID;
   YC_ENTER(ctx);
@@ -1126,6 +1348,8 @@ extern "C" int yc_begin_frame(yc_ctx* ctx, const YcFrameDesc* f) {
   ctx->frameRendered = false;
   if (ctx->aovs)
     if (const int arc = prepareAovPlanes(ctx)) return arc;
+  if (ctx->adaptive)
+    if (const int arc = prepareAdaptive(ctx)) return arc;
   // finalize leaves every bucket it reads zeroed, so the planes only need clearing when an accumulate was not
   // followed by its finalize (an error or abort mid-wave, a partial-rectangle finalize) or when they are new
   if (ctx->bucketsDirty) {
@@ -1344,6 +1568,11 @@ static int renderChunks(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dVie
       rt::launchFor(L.side, f.nPix,
                     AccumulateK{acc, ctx->dBuckets, ctx->bucketCapacity, dViews, ctx->dExposureScales, f.pixBase, f.nPix, f.K, f.sDone,
                                 f.stride, m, ctx->frame.estimator});
+      if (ctx->adaptive) {
+        rt::launchFor(L.side, f.nPix, AdaptiveMomentK{acc.L, dList, dViews, ctx->dExposureScales, ctx->dAdMom, f.pixBase, f.nPix,
+                                                      f.K, ctx->frame.width, ctx->frame.height, ctx->frame.estimator});
+        ctx->launches++;
+      }
       if (ctx->aovs) {
         rt::launchFor(L.side, f.nPix, AovAccumulateK{L.aov[f.buf], dList, dViews, ctx->dAovSum, ctx->dAovCount, ctx->aovTexels, f.pixBase,
                                                      f.nPix, f.K, ctx->frame.width, ctx->frame.height});
@@ -1486,23 +1715,100 @@ static int accumulateWave(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dV
                           : renderChunks<false>(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, m, bucketShard, bucketShardCount);
 }
 
+// The call's list holds every pixel of the shard that takes samples: the shard's list, or with adaptive sampling the
+// list of its pixels still sampling.
+static bool wholeShardList(const yc_ctx* ctx, const uint32_t* dList) {
+  return dList == ctx->dPixels || (ctx->adaptive && dList == ctx->adActive[ctx->adCur].pix);
+}
+
+// Tile sharding, direct delivery: the root's copy a finalizing call of `dList` stores its pixels into, or null.
+static void rootFrames(yc_ctx* ctx, const uint32_t* dList, float4** hdrRoot, float4** ldrRoot) {
+  *hdrRoot = *ldrRoot = nullptr;
+  if (ctx->comm && ctx->comm->direct) {
+    Comm& c = *ctx->comm;
+    // the copy the next yc_comm_reduce_frames publishes (noteWave has marked it stale if this wave is a partial one)
+    if (wholeShardList(ctx, dList) && !c.stale && c.frameTexels == frameTexels(ctx)) *hdrRoot = c.hdrAll[c.epoch & 1u], *ldrRoot = c.ldrAll[c.epoch & 1u];
+  }
+}
+
 // Estimator value of the wave + finishTile's blend and tonemap (tile-renderer.hpp:220-239).
 static void finalizeWave(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dViews, uint32_t nPixCall, uint32_t waveSamples, uint32_t takenBefore) {
   const YcFrameDesc& f = ctx->frame;
   const uint32_t takenAfter = takenBefore + waveSamples;
   const float wCurrent = float(takenBefore) / float(takenAfter), wWave = float(waveSamples) / float(takenAfter);
-  float4 *hdrRoot = nullptr, *ldrRoot = nullptr;
-  if (ctx->comm && ctx->comm->direct) {
-    Comm& c = *ctx->comm;
-    // the copy the next yc_comm_reduce_frames publishes (noteWave has marked it stale if this wave is a partial one)
-    if (dList == ctx->dPixels && !c.stale && c.frameTexels == frameTexels(ctx)) hdrRoot = c.hdrAll[c.epoch & 1u], ldrRoot = c.ldrAll[c.epoch & 1u];
-  }
+  float4 *hdrRoot, *ldrRoot;
+  rootFrames(ctx, dList, &hdrRoot, &ldrRoot);
   rt::launchFor(ctx->st, nPixCall,
                 FinalizeK{dList, dViews, ctx->dBuckets, ctx->bucketCapacity, ctx->dHdr, ctx->dLdr, hdrRoot, ldrRoot, f.width, f.height,
                           waveBuckets(f, waveSamples), f.estimator, waveSamples, f.tonemap, wCurrent, wWave});
   rt::eventRecord(ctx->st, ctx->evFinal);
   ctx->launches++;
-  if (dList == ctx->dPixels) ctx->bucketsDirty = false;  // every plane this shard touches was read and zeroed
+  if (wholeShardList(ctx, dList)) ctx->bucketsDirty = false;  // every plane this shard touches was read and zeroed
+}
+
+// Stable compaction of `n` entries of `in` by stop state (n > 0): the pixels still sampling into `keep`, and — when
+// `stopped` is given — those the last stop test stopped into `stopped`, which are marked as stopped before.  Leaves the
+// two counts in dAdCount, read back by adaptiveCounts.
+static void compactPixels(yc_ctx* ctx, yc_ctx::PixList in, uint32_t n, yc_ctx::PixList keep, yc_ctx::PixList* stopped) {
+  const uint32_t W = ctx->frame.width, H = ctx->frame.height;
+  rt::launchFor(ctx->st, n, AdaptiveClassK{in.pix, in.view, ctx->dAdState, ctx->dAdScan, W, H});
+  inclusiveScan(ctx->st, ctx->dAdScan, ctx->dAdSums, n);
+  rt::launchFor(ctx->st, n, AdaptiveScatterK{in.pix, in.view, ctx->dAdScan, ctx->dAdState, keep.pix, stopped ? stopped->pix : nullptr,
+                                             keep.view, stopped ? stopped->view : nullptr, W, H});
+  ctx->launches += 5;
+  ctx->dAdCount = ctx->dAdScan + (n - 1);
+}
+
+// The counts of the last compaction (waits for it).
+static int adaptiveCounts(yc_ctx* ctx, uint32_t* keep, uint32_t* stopped) {
+  unsigned long long v = 0;
+  YC_TRY(rt::d2h(ctx->st, &v, ctx->dAdCount, sizeof v));
+  ctx->dAdCount = nullptr;
+  *keep = uint32_t(v), *stopped = uint32_t(v >> 32);
+  return YC_OK;
+}
+
+// Pixel list of an adaptive wave call: the shard's pixels still sampling, or those of them inside `px`.
+static int adaptivePixels(yc_ctx* ctx, YcRect px, const uint32_t** dList, const uint16_t** dViews, uint32_t* nPixCall) {
+  if (ctx->dAdCount)
+    if (const int rc = adaptiveCounts(ctx, &ctx->adActiveCount, &ctx->adJustCount)) return rc;
+  if (wholeFrame(ctx, px)) {
+    *dList = ctx->adActive[ctx->adCur].pix, *dViews = ctx->adActive[ctx->adCur].view, *nPixCall = ctx->adActiveCount;
+    return YC_OK;
+  }
+  const uint32_t* sub;
+  const uint16_t* subViews;
+  uint32_t nSub, stopped;
+  if (const int rc = wavePixels(ctx, px, &sub, &subViews, &nSub)) return rc;
+  *dList = ctx->adRect.pix, *dViews = ctx->adRect.view, *nPixCall = 0;
+  if (nSub == 0) return YC_OK;
+  compactPixels(ctx, {const_cast<uint32_t*>(sub), const_cast<uint16_t*>(subViews)}, nSub, ctx->adRect, nullptr);
+  return adaptiveCounts(ctx, nPixCall, &stopped);
+}
+
+// After an adaptive call's finalize: e and the stop test for the call's pixels, then the shard's pixels still sampling
+// into the other list.  Direct frame delivery: a pixel stopped by the previous call was stored into that call's copy of
+// the root's frames only, so it is pushed into this call's copy first.
+static void adaptiveAfterWave(yc_ctx* ctx, const uint32_t* dList, const uint16_t* dViews, uint32_t nPixCall, uint32_t waveSamples) {
+  const YcFrameDesc& f = ctx->frame;
+  float4 *hdrRoot, *ldrRoot;
+  rootFrames(ctx, dList, &hdrRoot, &ldrRoot);
+  if (hdrRoot && ctx->adJustCount) {
+    rt::launchFor(ctx->st, ctx->adJustCount,
+                  PushFramesK{ctx->adJust.pix, ctx->adJust.view, ctx->dHdr, ctx->dLdr, hdrRoot, ldrRoot, f.width, f.height});
+    ctx->launches++;
+  }
+  ctx->adJustCount = 0;
+  if (nPixCall == 0) return;
+  const YcAdaptive& a = ctx->adParams;
+  rt::launchFor(ctx->st, nPixCall, AdaptiveErrorK{dList, dViews, ctx->dAdMom, ctx->dAdS, f.width, f.height, waveSamples, a.lumaFloor});
+  rt::launchFor(ctx->st, nPixCall, AdaptiveStopK{dList, dViews, ctx->dAdMom, ctx->dAdS, ctx->dAdState, f.width, f.height, f.tileSize,
+                                                 a.minSamples, a.threshold});
+  ctx->launches += 2;
+  const int cur = ctx->adCur;
+  compactPixels(ctx, ctx->adActive[cur], ctx->adActiveCount, ctx->adActive[cur ^ 1], &ctx->adJust);
+  ctx->adCur = cur ^ 1;
+  ctx->adActiveCount = 0;  // (read back with the next call)
 }
 
 // Bookkeeping for the direct frame delivery of comm.cuh, from the ARGUMENTS of a finalizing call only — every
@@ -1526,8 +1832,12 @@ static int issueWave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset, uint32_t wav
   const uint32_t* dList;
   const uint16_t* dViews;
   uint32_t nPixCall;
-  if (const int prc = wavePixels(ctx, px, &dList, &dViews, &nPixCall)) return prc;
-  if (nPixCall == 0) return YC_OK;
+  if (const int prc = ctx->adaptive ? adaptivePixels(ctx, px, &dList, &dViews, &nPixCall) : wavePixels(ctx, px, &dList, &dViews, &nPixCall))
+    return prc;
+  if (nPixCall == 0) {
+    if (ctx->adaptive) adaptiveAfterWave(ctx, dList, dViews, 0, 0);
+    return YC_OK;
+  }
   if (!ctx->wavesPending) rt::eventRecord(ctx->st, ctx->ev0);
   const int rc = accumulateWave(ctx, dList, dViews, nPixCall, sampleOffset, waveSamples, 0, 1);
   if (rc != YC_OK) {
@@ -1535,6 +1845,10 @@ static int issueWave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset, uint32_t wav
     return rc;
   }
   finalizeWave(ctx, dList, dViews, nPixCall, waveSamples, takenBefore);
+  if (ctx->adaptive) {
+    adaptiveAfterWave(ctx, dList, dViews, nPixCall, waveSamples);
+    ctx->adSamples += uint64_t(nPixCall) * waveSamples;
+  }
   rt::eventRecord(ctx->st, ctx->ev1);
   ctx->wavesPending = true;
   return YC_OK;
@@ -1569,6 +1883,8 @@ extern "C" int yc_accumulate_wave(yc_ctx* ctx, YcRect px, uint32_t sampleOffset,
   if (bucketShardCount == 0 || bucketShard >= bucketShardCount) return fail(ctx, YC_ERR_INVALID, "bucket shard out of range");
   // a pixel's samples would be split over the participants, and its AOV sums would lose their order
   if (ctx->aovs && bucketShardCount > 1) return fail(ctx, YC_ERR_UNSUPPORTED, "AOVs with bucket sharding");
+  // (the same for the moments of adaptive sampling, whose stop test runs in the finalizing wave calls)
+  if (ctx->adaptive) return fail(ctx, YC_ERR_UNSUPPORTED, "yc_accumulate_wave with adaptive sampling (use yc_render_wave)");
   ctx->frameRendered = true;
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
   const uint32_t* dList;
@@ -1586,6 +1902,7 @@ extern "C" int yc_finalize_wave(yc_ctx* ctx, YcRect px, uint32_t waveSamples, ui
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
   if (!ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_finalize_wave before yc_begin_frame");
+  if (ctx->adaptive) return fail(ctx, YC_ERR_UNSUPPORTED, "yc_finalize_wave with adaptive sampling (use yc_render_wave)");
   if (const int vrc = checkViews(ctx)) return vrc;
   noteWave(ctx, px);
   if (waveSamples == 0 || px.w == 0 || px.h == 0) return YC_OK;
@@ -1626,6 +1943,7 @@ static int readStats(yc_ctx* ctx, YcStats* stats) {
   stats->raysReference = c.raysReference;
   stats->raysExtend = ctx->raysExtend + c.raysExtend;
   stats->raysShadow = c.raysShadow;
+  stats->samples = ctx->adaptive ? ctx->adSamples : 0;
   stats->boxTests = c.boxTests;
   stats->triTests = c.triTests;
   stats->kernelLaunches = ctx->launches;
@@ -1663,6 +1981,27 @@ extern "C" int yc_resolve_aovs(yc_ctx* ctx, float* albedoRGBA, float* normalDept
   if (normalDepthRGBA) YC_TRY(rt::d2h(ctx->st, normalDepthRGBA, ctx->dAov + n, n * sizeof(float4)));
   YC_TRY(rt::sync(ctx->st));
   YC_TRY(rt::lastError());
+  return YC_OK;
+}
+
+extern "C" int yc_resolve_adaptive(yc_ctx* ctx, uint32_t* samples, float* error, uint64_t* activePixels) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->adaptive || !ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_resolve_adaptive: adaptive sampling is off for this frame");
+  if (ctx->dAdCount)
+    if (const int rc = adaptiveCounts(ctx, &ctx->adActiveCount, &ctx->adJustCount)) return rc;
+  const size_t n = ctx->adTexels;
+  if (samples || error) {
+    rt::launchFor(ctx->st, uint32_t(n), AdaptiveResolveK{nullptr, nullptr, ctx->dAdMom, ctx->dAdS, ctx->dAdPlanes,
+                                                         reinterpret_cast<float*>(ctx->dAdPlanes + n), ctx->frame.width,
+                                                         ctx->frame.height});
+    ctx->launches++;
+  }
+  if (samples) YC_TRY(rt::d2h(ctx->st, samples, ctx->dAdPlanes, n * sizeof(uint32_t)));
+  if (error) YC_TRY(rt::d2h(ctx->st, error, ctx->dAdPlanes + n, n * sizeof(float)));
+  YC_TRY(rt::sync(ctx->st));
+  YC_TRY(rt::lastError());
+  if (activePixels) *activePixels = ctx->adActiveCount;
   return YC_OK;
 }
 
@@ -2304,6 +2643,19 @@ extern "C" int yc_comm_allreduce_buckets(yc_ctx* ctx, uint32_t waveSamples) {
 // Tile sharding: every participant resolves its planes (zero outside its tiles) into a buffer of its own and the buffers
 // are summed into the root's as 32-bit integers — each texel is non-zero on one participant only, so the integer sum
 // keeps every bit pattern, -0.0 included.  Out of place: the sums keep accumulating and repeated calls count nothing twice.
+// `resolve` writes the planes into `buf` (`words` 32-bit words) and returns a YC_ code; *combined tells whether this
+// context holds the result.
+template <class F>
+static int reducePlanes(yc_ctx* ctx, int root, void* buf, size_t words, bool* combined, F&& resolve) {
+  const int rc = timedCollective(ctx, [&] {
+    if (const int rrc = resolve()) return rrc;
+    return commSum(ctx, buf, words, kCommI32, root);
+  });
+  if (rc != YC_OK) return rc;
+  *combined = ctx->comm->rank == root;
+  return YC_OK;
+}
+
 extern "C" int yc_comm_reduce_aovs(yc_ctx* ctx, int root) {
   if (!ctx) return YC_ERR_INVALID;
   YC_ENTER(ctx);
@@ -2312,12 +2664,40 @@ extern "C" int yc_comm_reduce_aovs(yc_ctx* ctx, int root) {
   if (root < 0 || root >= ctx->comm->world) return fail(ctx, YC_ERR_INVALID, "bad root");
   const size_t n = ctx->aovTexels;
   if (!ctx->dAovComm) YC_TRY(rt::alloc(reinterpret_cast<void**>(&ctx->dAovComm), 2 * n * sizeof(float4)));
-  const int rc = timedCollective(ctx, [&] {
-    resolveAovs(ctx, ctx->dAovComm, ctx->dAovComm + n);
-    return commSum(ctx, ctx->dAovComm, 2 * n * 4, kCommI32, root);
+  return reducePlanes(ctx, root, ctx->dAovComm, 2 * n * 4, &ctx->aovCombined,
+                      [&] {
+                        resolveAovs(ctx, ctx->dAovComm, ctx->dAovComm + n);
+                        return YC_OK;
+                      });
+}
+
+// The same for the adaptive planes {S, e}: each participant writes its own pixels' values into zeroed planes (a texel
+// never sampled reads e = +inf on its own participant only).
+extern "C" int yc_comm_reduce_adaptive(yc_ctx* ctx, int root) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->comm) return fail(ctx, YC_ERR_STATE, "yc_comm_reduce_adaptive without a communicator");
+  if (!ctx->adaptive || !ctx->inFrame) return fail(ctx, YC_ERR_STATE, "yc_comm_reduce_adaptive: adaptive sampling is off for this frame");
+  if (root < 0 || root >= ctx->comm->world) return fail(ctx, YC_ERR_INVALID, "bad root");
+  const size_t n = ctx->adTexels;
+  if (!ctx->dAdComm) YC_TRY(devAlloc(ctx->adAllocs, &ctx->dAdComm, 2 * n));
+  return reducePlanes(ctx, root, ctx->dAdComm, 2 * n, &ctx->adCombined, [&] {
+    YC_TRY(rt::zero(ctx->st, ctx->dAdComm, 2 * n * sizeof(uint32_t)));
+    rt::launchFor(ctx->st, uint32_t(ctx->pixels.size()),
+                  AdaptiveResolveK{ctx->dPixels, ctx->dPixelViews, ctx->dAdMom, ctx->dAdS, ctx->dAdComm,
+                                   reinterpret_cast<float*>(ctx->dAdComm + n), ctx->frame.width, ctx->frame.height});
+    ctx->launches++;
+    return YC_OK;
   });
-  if (rc != YC_OK) return rc;
-  ctx->aovCombined = ctx->comm->rank == root;
+}
+
+extern "C" int yc_resolve_adaptive_combined(yc_ctx* ctx, uint32_t* samples, float* error) {
+  if (!ctx) return YC_ERR_INVALID;
+  YC_ENTER(ctx);
+  if (!ctx->adCombined) return fail(ctx, YC_ERR_STATE, "yc_resolve_adaptive_combined: not the root of a completed yc_comm_reduce_adaptive");
+  const size_t n = ctx->adTexels;
+  if (samples) YC_TRY(rt::d2h(ctx->st, samples, ctx->dAdComm, n * sizeof(uint32_t)));
+  if (error) YC_TRY(rt::d2h(ctx->st, error, ctx->dAdComm + n, n * sizeof(float)));
   return YC_OK;
 }
 

@@ -9,6 +9,7 @@
 // Compiled with g++ -ffp-contract=off (derived constants must round like the reference's).
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <mutex>
 #include <new>
 #include <thread>
@@ -312,6 +313,8 @@ struct yr_renderer {
   YrRenderData last{};
   int lastRc = YC_OK;
   bool aovs = false;                // yr_enable_aovs
+  bool adaptive = false;            // yr_set_adaptive
+  YcAdaptive adParams{};
   std::atomic<bool> running{false}; // a render is in progress (yr_render's worker, or yr_render_sync)
 };
 
@@ -537,6 +540,7 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
     // the whole frame and takes its (bucket, pixel class) units of every wave
     f.shardIndex = buckets ? 0u : r->rank0 + uint32_t(i), f.shardCount = buckets ? 1u : r->world;
     if ((e = yc_begin_frame(sh.ctx, &f)) != YC_OK) return e;
+    if ((e = yc_set_adaptive(sh.ctx, r->adaptive ? &r->adParams : nullptr)) != YC_OK) return e;
     return yc_enable_aovs(sh.ctx, r->aovs ? 1 : 0);
   });
   if (rc != YC_OK) return rfail(r, rc, r->err);
@@ -561,16 +565,20 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
       return buckets ? yc_accumulate_wave(c, full, taken, ws, r->rank0 + uint32_t(i), r->world) : yc_render_wave(c, full, taken, ws, taken);
     });
     if (rc != YC_OK && rc != YC_ERR_ABORTED) return rfail(r, rc, r->err);
-    // rays of the wave over all participants, and whether anyone was told to stop: agreed on collectively, so
-    // that either every participant enters the wave's data collective or none does
-    uint64_t agree[2] = {0, uint64_t(rc == YC_ERR_ABORTED || r->stop != 0)};
+    // rays of the wave over all participants, whether anyone was told to stop, and the pixels still sampling (adaptive
+    // sampling): agreed on collectively, so that either every participant enters the wave's data collective or none does
+    uint64_t agree[3] = {0, uint64_t(rc == YC_ERR_ABORTED || r->stop != 0), 0};
     for (Shard& sh : r->shards) {
       YcStats st{};
       yc_resolve(sh.ctx, nullptr, nullptr, &st);
       agree[0] += st.raysReference;
+      uint64_t active = 0;
+      if (r->adaptive && !agree[1] && (rc = yc_resolve_adaptive(sh.ctx, nullptr, nullptr, &active)) != YC_OK)
+        return rfail(r, rc, yc_last_error(sh.ctx));
+      agree[2] += active;
     }
     if (r->comm && r->shards.size() == 1) {  // one process per GPU: sum over the ranks
-      if ((rc = yc_comm_sum_u64(r->shards[0].ctx, agree, 2)) != YC_OK) return rfail(r, rc, yc_last_error(r->shards[0].ctx));
+      if ((rc = yc_comm_sum_u64(r->shards[0].ctx, agree, 3)) != YC_OK) return rfail(r, rc, yc_last_error(r->shards[0].ctx));
     }
     if (agree[1]) {
       aborted = true;
@@ -618,6 +626,7 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
       r->cb(&data, &wd, r->cbUser);
     }
     raysBefore = agree[0];
+    if (r->adaptive && agree[2] == 0) break;  // every pixel has stopped: the render is complete
     const uint64_t next = (wave > 0 || waveSamples > 1) ? std::min<uint64_t>(waveSamples * 2, maxWave) : 1;
     waveSamples = std::min<uint64_t>(next, remaining);
     wave++;
@@ -626,6 +635,10 @@ static int renderBlocking(yr_renderer* r, YrRenderData* out) {
     // tile sharding (bucket sharding refuses AOVs): the shards' planes into the root's, once per render — after an abort
     // too, since the abort vote has brought every participant here
     rc = onShards(r, [&](size_t i) { return yc_comm_reduce_aovs(r->shards[i].ctx, 0); });
+    if (rc != YC_OK) return rfail(r, rc, r->err);
+  }
+  if (r->adaptive && r->comm) {  // the same for the adaptive planes (bucket sharding refuses adaptive sampling)
+    rc = onShards(r, [&](size_t i) { return yc_comm_reduce_adaptive(r->shards[i].ctx, 0); });
     if (rc != YC_OK) return rfail(r, rc, r->err);
   }
   {
@@ -720,6 +733,33 @@ extern "C" int yr_read_aovs(yr_renderer* r, float* albedoRGBA, float* normalDept
     if (rootHere(r)) rc = yc_resolve_aovs_combined(c0, albedoRGBA, normalDepthRGBA);
   } else {
     rc = yc_resolve_aovs(c0, albedoRGBA, normalDepthRGBA);
+  }
+  return rc != YC_OK ? rfail(r, rc, yc_last_error(c0)) : YC_OK;
+}
+
+extern "C" int yr_set_adaptive(yr_renderer* r, const YcAdaptive* params) {
+  if (!r) return YC_ERR_INVALID;
+  if (r->running) return rfail(r, YC_ERR_STATE, "yr_set_adaptive while a render runs");
+  if (params && !(std::isfinite(params->threshold) && params->threshold >= 0.0f && std::isfinite(params->lumaFloor) &&
+                  params->lumaFloor > 0.0f))
+    return rfail(r, YC_ERR_INVALID, "yr_set_adaptive: threshold must be finite and >= 0, lumaFloor finite and > 0");
+  if (params && r->comm && r->s.sharding == YR_SHARD_BUCKETS)
+    return rfail(r, YC_ERR_UNSUPPORTED, "adaptive sampling with bucket sharding: a pixel's samples are split over the participants");
+  r->adaptive = params != nullptr;  // applied to the contexts by the next render, after its yc_begin_frame
+  if (params) r->adParams = *params;
+  return YC_OK;
+}
+
+extern "C" int yr_read_adaptive(yr_renderer* r, uint32_t* samples, float* error) {
+  if (!r) return YC_ERR_INVALID;
+  if (r->running) return rfail(r, YC_ERR_STATE, "yr_read_adaptive while a render runs");
+  if (!r->adaptive) return rfail(r, YC_ERR_STATE, "yr_read_adaptive: adaptive sampling is off (yr_set_adaptive)");
+  yc_ctx* c0 = r->shards[0].ctx;
+  int rc = YC_OK;
+  if (r->comm && r->s.sharding == YR_SHARD_TILES) {
+    if (rootHere(r)) rc = yc_resolve_adaptive_combined(c0, samples, error);
+  } else {
+    rc = yc_resolve_adaptive(c0, samples, error, nullptr);
   }
   return rc != YC_OK ? rfail(r, rc, yc_last_error(c0)) : YC_OK;
 }
